@@ -2,7 +2,7 @@
 """Benchmark of the MPPI hot path (BASELINE.json metric: MPPI sample-steps/s and p50 control-step
 latency at K samples x H horizon).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Headline workload (config.workload): differential-drive MPPI, K = 1M samples PER GPU, H = 50,
 Philox noise generated in-kernel, `sum` cost / frozen window (the parallel modes of the reference
@@ -19,6 +19,11 @@ Prints ONE JSON line (rank 0).  `value` is device-timed (CUDA events on the laun
 resident); `e2e` goes through the drop-in class `MPPIAlgorithms._calc_input_control` with a host
 state in and a host control out every tick.  `--impl reference` times the CPU restatement of the
 reference tick (oracle/, the one place bench.py may execute it) on the host cores.
+
+`--dump-outputs DIR` writes what the device-timed tick handed back after its last timed step -- the nominal
+control sequence `u_seq.npy` (H, 2) and the returned control `u0.npy` (2,), float32, the pair `mppi_step`
+returns -- so two builds run with the same arguments (same seeds, same tick indices) can be compared output for
+output.
 """
 import argparse
 import contextlib
@@ -239,10 +244,10 @@ def run_reference_arm(args):
     if rank != 0:
         return
     # the SAME configuration as the B200 arm's N=1 workload: K = 1M samples x H = 50 per step, sum / frozen, Philox noise;
-    # one step is ~0.5 s on 16 cores, so the step count is capped to keep the run within a few minutes
+    # one step is ~0.5 s on 16 cores
     K_s = K_PER_GPU
     cpu_port_run(1, K_s, T_H, 10.0)
-    n_ref = max(1, min(args.steps, 30))
+    n_ref = args.steps
     times, nthr = cpu_port_run(n_ref, K_s, T_H, 10.0)
     ms = 1e3 * float(np.mean(times))
     val = K_s * T_H / float(np.mean(times))
@@ -350,6 +355,13 @@ def run_b200_arm(args):
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = eng.timings()["launches"] - launches0
+    if args.dump_outputs and rank == 0:
+        # read before the e2e loop below steps the same handle again; the tick leaves the shifted nominal on the device and
+        # mppi_step returns it with its row 0 as u0
+        u_seq = eng.get_nominal().astype(np.float32)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "u_seq.npy"), u_seq)
+        np.save(os.path.join(args.dump_outputs, "u0.npy"), u_seq[0].copy())
     step_ms = np.array([a.elapsed_time(b) for a, b in ev])
     local_ms = float(step_ms.sum())
     if world > 1:
@@ -788,7 +800,13 @@ def main():
     ap.add_argument("--steps", type=int, default=400)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write u_seq.npy and u0.npy of the last timed step to DIR (b200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(3, args.warmup)
     # stdout carries exactly ONE JSON line: native libraries (NCCL prints its version banner there) and anything else
     # that writes to fd 1 during the run go to stderr; the line itself is written to the saved descriptor

@@ -4,8 +4,7 @@ can be pinned against them and golden vectors can be generated.
 
 /root/reference exists only in the build container, never on the GPU box, so nothing
 that runs under `-m gpu`, `smoke()` or `bench.py` may import this module.  It is used
-by `tests/golden/make_golden.py` (fixture generator, run here) and by the
-`requires_reference` CPU tests (skipped when the tree is absent).
+only by `tests/golden/make_golden.py` (the fixture generator); the tests read what it stored.
 
 The reference imports matplotlib at module top
 (controllers/mppi_differential_drive.py:6,8; models/vehicle.py:2-5) but only uses it

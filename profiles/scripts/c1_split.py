@@ -1,7 +1,8 @@
 """Where the literal C1 tick (K = 1000, T = 30, cost_mode last, waypoint_mode strict) spends its time: the handle's own event
 timings (rollout = strict passes incl. their host round trips, update = K2 kernel) next to the host-to-host latency."""
 import sys, time
-sys.path[:0] = ['/root/repo', '/root/repo/dnn-mppi-mpc_b200', '/root/repo/tests']
+import os
+sys.path[:0] = [os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import numpy as np
 from bench import diffdrive_kwargs
 from mppi_b200.mppi_differential_drive import MPPIAlgorithms

@@ -2,7 +2,7 @@
 one box, fused NVLink exchange, device-timed per tick (CUDA events on the launching stream), MAX over ranks.
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P profiles/scripts/k_sweep_multi.py"""
 import os, sys
-sys.path[:0] = ['/root/repo', '/root/repo/dnn-mppi-mpc_b200', '/root/repo/tests']
+sys.path[:0] = [os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import numpy as np, torch, torch.distributed as dist
 from bench import diffdrive_kwargs
 from mppi_b200.mppi_differential_drive import MPPIAlgorithms

@@ -1,7 +1,7 @@
 """K=1M, H=50 diff-drive (sum/frozen, Philox): how many samples' costs differ from the FP64 C oracle by more than
 rtol 1e-5 (= nearest-waypoint near-ties decided differently in FP32), for the library MPPI_B200_LIB points at.
 Test infrastructure use of oracle/ (same check as tests/test_gpu_parity.py::test_large_K_full_size_property)."""
-import sys; sys.path[:0] = ['/root/repo', '/root/repo/dnn-mppi-mpc_b200', '/root/repo/tests']
+import os, sys; sys.path[:0] = [os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import numpy as np, torch
 from golden_util import Golden
 from gpu_util import engine_from_spec

@@ -1,4 +1,4 @@
-import sys; sys.path[:0]=['/root/repo','/root/repo/dnn-mppi-mpc_b200','/root/repo/tests']
+import os, sys; sys.path[:0]=[os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import numpy as np, torch
 from golden_util import Golden
 from gpu_util import engine_from_spec

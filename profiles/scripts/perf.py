@@ -1,4 +1,4 @@
-import sys, time; sys.path[:0]=['/root/repo','/root/repo/dnn-mppi-mpc_b200','/root/repo/tests']
+import os, sys, time; sys.path[:0]=[os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import numpy as np, torch
 from bench import diffdrive_kwargs
 from mppi_b200.mppi_differential_drive import MPPIAlgorithms

@@ -1,4 +1,4 @@
-import sys, time; sys.path[:0]=['/root/repo','/root/repo/dnn-mppi-mpc_b200','/root/repo/tests']
+import os, sys, time; sys.path[:0]=[os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import os, numpy as np, torch
 NH = int(os.environ.get("NH", "2")); NIN = int(os.environ.get("NIN", "3"))    # hidden tanh layers (2 | 3), inputs (3 | 5)
 from golden_util import Golden

@@ -1,6 +1,6 @@
 """Where the ~8 us between the back-to-back tick time and bench.py's per-step event time come from: per-step CUDA events with
 (a) nothing, (b) the 256 MiB L2-flush memset, (c) a small unrelated kernel between the ticks."""
-import sys; sys.path[:0]=['/root/repo','/root/repo/dnn-mppi-mpc_b200','/root/repo/tests']
+import os, sys; sys.path[:0]=[os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "..", d) for d in (".", "dnn-mppi-mpc_b200", "tests")]
 import numpy as np, torch
 from bench import diffdrive_kwargs
 from mppi_b200.mppi_differential_drive import MPPIAlgorithms

@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for p in (ROOT, os.path.join(ROOT, "dnn-mppi-mpc_b200"), os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -11,14 +9,3 @@ for p in (ROOT, os.path.join(ROOT, "dnn-mppi-mpc_b200"), os.path.join(ROOT, "tes
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "requires_reference: needs /root/reference (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    from oracle import ref_loader
-    if ref_loader.reference_available():
-        return
-    skip = pytest.mark.skip(reason="reference tree not present on this machine")
-    for it in items:
-        if "requires_reference" in it.keywords:
-            it.add_marker(skip)

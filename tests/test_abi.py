@@ -4,7 +4,6 @@ import ctypes as C
 import os
 import re
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -53,14 +52,24 @@ def test_errors_are_status_codes_not_exceptions_across_the_abi():
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from mppi_b200 import MppiError
-    from mppi_b200.mppi_differential_drive import MPPIAlgorithms
-    with pytest.raises(MppiError):
-        MPPIAlgorithms(0.1, np.zeros((30, 3)), 5.0, 3.14, 100, 10, 1e-4, 1.0, 0.2, np.diag([0.1, 0.01]),
-                       np.ones(3), np.ones(3))
+    """Without a CUDA device the drop-in class refuses to construct.  Checked in a child process that sees no device, so
+    the check also runs on a machine that has one."""
+    import subprocess
+    import sys
+    code = ("import sys\n"
+            "sys.path.insert(0, %r)\n"
+            "import numpy as np\n"
+            "from mppi_b200 import MppiError\n"
+            "from mppi_b200.mppi_differential_drive import MPPIAlgorithms\n"
+            "try:\n"
+            "    MPPIAlgorithms(0.1, np.zeros((30, 3)), 5.0, 3.14, 100, 10, 1e-4, 1.0, 0.2, np.diag([0.1, 0.01]),\n"
+            "                   np.ones(3), np.ones(3))\n"
+            "except MppiError:\n"
+            "    sys.exit(0)\n"
+            "sys.exit('constructed without a CUDA device')\n") % os.path.join(ROOT, "dnn-mppi-mpc_b200")
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
 
 
 def test_product_never_imports_the_oracle():

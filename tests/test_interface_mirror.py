@@ -1,7 +1,6 @@
 """The drop-in boundary (SURVEY.md 8b): every host class keeps the reference class's constructor parameters (names,
 order, defaults) and per-tick method name.  The expected signatures below were read off the reference sources
-(file:line cited per entry); in the build container, where /root/reference exists, the same comparison also runs
-against the unmodified reference classes themselves."""
+(file:line cited per entry)."""
 import inspect
 
 import pytest
@@ -34,12 +33,12 @@ EXPECTED = [
       "number_of_samples_K": 100, "param_exploration": 0.01, "param_lambda": 50.0, "param_alpha": 1.0,
       "collision_safety_margin_rat": 1.5}),
 ]
-REFERENCE_CLASSES = {
-    "controllers/mppi_differential_drive.py:44-60": ("controllers.mppi_differential_drive", "MPPIAlgorithms"),
-    "controllers/mppi_differential_drive_obs.py:44-62": ("controllers.mppi_differential_drive_obs", "MPPIAlgorithms"),
-    "test/mppi_differential_drive_obs.py:44-62": ("test.mppi_differential_drive_obs", "MPPIAlgorithms"),
-    "controllers/mppi_race_car_obstacle.py:11-30": ("controllers.mppi_race_car_obstacle", "MPPIRacecarController"),
-}
+# the first positional parameter that has a default in the reference: it and every later one may be omitted by a caller
+# (in the race-car class that includes the array-valued ref_path, sigma, weights and obstacle_circles, :11-30)
+FIRST_DEFAULTED = {"mppi_b200.mppi_differential_drive": "visualize_optimal_traj",
+                   "mppi_b200.mppi_differential_drive_obs": "visualize_optimal_traj",
+                   "mppi_b200.mppi_differential_drive_goal": "visualize_optimal_traj",
+                   "mppi_b200.mppi_race_car_obstacle": "delta_t"}
 
 
 def _positional(cls):
@@ -56,29 +55,10 @@ def test_drop_in_signature_matches_the_reference_source(mod, cls, tick, ref, nam
     assert got_names == names, ref
     for k, v in defaults.items():
         assert got_defaults[k] == v, (ref, k)
+    assert [n for n in got_names if n in got_defaults] == names[names.index(FIRST_DEFAULTED[mod]):], ref
     assert callable(getattr(c, tick))
     # everything this repo adds is keyword-only, so positional call sites of the reference keep working
     params = inspect.signature(c.__init__).parameters.values()
     extra = {p.name for p in params if p.kind is p.KEYWORD_ONLY}
     forwards = any(p.kind is p.VAR_KEYWORD for p in params)           # subclasses forward **kw to the base class
     assert {"seed", "device"} <= extra or forwards
-
-
-@pytest.mark.requires_reference
-@pytest.mark.parametrize("mod,cls,tick,ref,names,defaults", EXPECTED, ids=[e[0].split(".")[-1] for e in EXPECTED])
-def test_drop_in_signature_matches_the_reference_class(mod, cls, tick, ref, names, defaults):
-    import importlib
-    from oracle import ref_loader
-    ref_loader.load_reference_extras()
-    rmod, rcls = REFERENCE_CLASSES[ref]
-    r = getattr(importlib.import_module(rmod), rcls)
-    c = getattr(importlib.import_module(mod), cls)
-    r_names, r_defaults = _positional(r)
-    c_names, c_defaults = _positional(c)
-    assert c_names == r_names
-    for k, v in r_defaults.items():
-        if isinstance(v, (int, float, bool)):
-            assert c_defaults[k] == v, k
-        else:
-            assert k in c_defaults, k                    # array-valued defaults (sigma, weights, obstacles): present
-    assert hasattr(r, tick) and hasattr(c, tick)
