@@ -105,6 +105,7 @@ struct mppi_handle_s {
     size_t sort_temp_bytes = 0;
     unsigned long long *d_trace = nullptr;     // per-CTA time stamps of the last tick (mppi_set_trace)
     int trace_n = 0;
+    int trace_grid = 0;                        // CTAs per robot of the last traced launch
     // timing / bookkeeping
     bool timing = false;
     cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
@@ -150,10 +151,24 @@ static int fail(mppi_handle_t h, int code, const char *msg) {
     return code;
 }
 
-// Fused exchange: the kernel raises out[7] (device + mapped host record) when a peer never published its triple; that
-// tick was NOT applied (nominal and waypoint index untouched).  Report it once and clear it, so later ticks are judged
-// on their own.  Call after a stream synchronize.
+// finalize_tick raises out[MPPI_OUT_FAULT] of a robot whose costs were not finite, and the fused exchange raises out[7]
+// (device + mapped host record) when a peer never published its triple; that tick was NOT applied (nominal and waypoint
+// index untouched).  Report it once and clear it, so later ticks are judged on their own.  Call after a stream synchronize.
 static int check_tick_faults(mppi_handle_t h) {
+    const int R = h->cfg.n_robots;
+    if (R > 1) {                                         // a fleet has no mapped record: read every robot's word back
+        std::vector<float> fault((size_t)R);
+        const size_t pitch = sizeof(float) * MPPI_OUT_STRIDE;
+        CK(h, cudaMemcpy2DAsync(fault.data(), sizeof(float), h->d_out + MPPI_OUT_FAULT, pitch, sizeof(float), R,
+                                cudaMemcpyDeviceToHost, h->stream));
+        CK(h, cudaStreamSynchronize(h->stream));
+        const int r = (int)(std::find_if(fault.begin(), fault.end(), [](float v) { return v != 0.f; }) - fault.begin());
+        if (r == R) return MPPI_OK;
+        CK(h, cudaMemset2DAsync(h->d_out + MPPI_OUT_FAULT, pitch, 0, sizeof(float), R, h->stream));
+        h->err = "robot " + std::to_string(r) + ": non-finite sample costs (NaN/inf observed state); the tick was not applied "
+                 "to that robot (its u0 row reads NaN, its nominal and waypoint index are unchanged)";
+        return MPPI_E_NUMERIC;
+    }
     if (h->h_out[MPPI_OUT_FAULT] != 0.f) {               // finalize_tick refused non-finite costs
         h->h_out[MPPI_OUT_FAULT] = 0.f;
         cudaMemsetAsync(h->d_out + MPPI_OUT_FAULT, 0, sizeof(float), h->stream);
@@ -341,6 +356,9 @@ int mppi_create(const mppi_config_t *cfg, mppi_handle_t *out) {
             h->grid_x_tpar = gt;
             gx = std::max(gx, gt);
         }
+        if (std::getenv("MPPI_VERBOSE"))          // the path Philox ticks take, and its grid
+            std::fprintf(stderr, "mppi_create: rollout path %s, %d CTAs per robot\n", h->tpar ? "tpar" : h->stash ? "stash" : "regenerate",
+                         h->tpar ? h->grid_x_tpar : h->stash ? h->grid_x_stash : h->grid_x);
     }
 
     CKC(gmalloc(h, &h->d_U, sizeof(float) * R * T * 2));
@@ -728,6 +746,7 @@ static int strict_costs(mppi_handle_t h, const double *x0, const float *d_eps, f
 static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
     const int stash = (!inj && !(a.flags & F_FROM_S)) ? (h->tpar ? 2 : h->stash ? 1 : 0) : 0;
     dim3 grid(stash == 2 ? h->grid_x_tpar : stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
+    if (a.trace) h->trace_grid = (int)grid.x;
     const int model = (h->cfg.model == MPPI_MODEL_DIFFDRIVE_MLP) ? MPPI_MODEL_DIFFDRIVE : h->cfg.model;
     if (h->world > 1 && h->p2p && (a.flags & F_UPDATE)) {
         TickArgs b = a;                      // exchange fused into the tick kernel: ONE launch, no NCCL call
@@ -832,6 +851,7 @@ int mppi_rollout_costs(mppi_handle_t h, const double *x0, const float *d_eps, ui
         TickArgs a = h->args;
         a.flags = F_IDX_ONLY;
         dim3 grid(1, 1);
+        if (a.trace) h->trace_grid = 1;
         CK(h, mppi_launch_tick(a, MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE, MPPI_COSTKIND_PATH, h->sum, false, false, grid, h->stream));
         h->tm.launches++;
     } else if (h->strict) {
@@ -845,6 +865,7 @@ int mppi_rollout_costs(mppi_handle_t h, const double *x0, const float *d_eps, ui
         TickArgs a = h->args;
         a.eps = d_eps; a.S = d_S; a.flags = F_WRITE_S;
         dim3 grid(h->grid_x, 1);
+        if (a.trace) h->trace_grid = (int)grid.x;
         CK(h, mppi_launch_tick(a, h->cfg.model, h->cfg.collision, h->cfg.cost_kind, h->sum, d_eps != nullptr, false, grid, h->stream));
         h->tm.launches++;
     }
@@ -961,6 +982,7 @@ int mppi_run_closed_loop(mppi_handle_t h, const double *x0, int32_t n_ticks, uin
         gfree(h, h->d_plant_log); h->d_plant_log = nullptr;
         if (h->loop_graph) { cudaGraphExecDestroy(h->loop_graph); h->loop_graph = nullptr; }     // it holds the old pointer
         CK(h, gmalloc(h, &h->d_plant_log, sizeof(float) * log_floats));
+        CK(h, cudaMemset(h->d_plant_log, 0, sizeof(float) * log_floats));
         h->plant_log_cap = n_ticks;
     }
     if (!h->d_x0) CK(h, gmalloc(h, &h->d_x0, sizeof(float) * 4 * R));
@@ -1028,7 +1050,7 @@ int mppi_run_closed_loop(mppi_handle_t h, const double *x0, int32_t n_ticks, uin
     for (size_t i = 0; i < (size_t)(n_ticks + 1) * R; ++i)
         for (int j = 0; j < nx; ++j) states_out[i * nx + j] = log[4 * i + j];
     if (controls_out) std::memcpy(controls_out, log.data() + (size_t)4 * (n_ticks + 1) * R, sizeof(float) * 2 * n_ticks * R);
-    return R == 1 ? check_tick_faults(h) : MPPI_OK;
+    return check_tick_faults(h);
 }
 
 int mppi_step_batched(mppi_handle_t h, const float *d_x0, uint64_t seed, uint64_t tick, float *d_u0_out) {
@@ -1045,6 +1067,7 @@ int mppi_step_batched(mppi_handle_t h, const float *d_x0, uint64_t seed, uint64_
     a.x0_dev = h->d_x0; a.eps = nullptr; a.S = nullptr; a.flags = F_UPDATE; a.u0_out = d_u0_out;
     a.out_host = nullptr;
     dim3 grid(h->stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
+    if (a.trace) h->trace_grid = (int)grid.x;
     CK(h, mppi_launch_tick(a, h->cfg.model, h->cfg.collision, h->cfg.cost_kind, h->sum, false, h->stash ? 1 : 0, grid, h->stream));
     h->tm.launches++;
     return MPPI_OK;
@@ -1132,7 +1155,8 @@ int mppi_get_trace(mppi_handle_t h, uint64_t *out, int32_t capacity, int32_t *n_
     const int n = std::min(capacity, h->trace_n);
     CK(h, cudaMemcpyAsync(out, h->d_trace, sizeof(uint64_t) * n, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    *n_ctas_out = h->tpar ? h->grid_x_tpar : h->stash ? h->grid_x_stash : h->grid_x;
+    if (h->trace_grid == 0) return fail(h, MPPI_E_STATE, "no tick has been traced since mppi_set_trace(h, 1)");
+    *n_ctas_out = h->trace_grid;
     return MPPI_OK;
 }
 

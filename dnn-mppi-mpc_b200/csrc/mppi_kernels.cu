@@ -9,6 +9,8 @@
 #include "mppi_launch.h"
 
 #include <algorithm>
+#include <mutex>
+#include <vector>
 
 namespace {
 
@@ -201,6 +203,14 @@ __device__ void merge_partials(const TickArgs &a, const float *parts, int P, Mer
     __syncthreads();
 }
 
+// This tick's rows of `robot` in the closed-loop log: the plant state after the step, and the control applied.
+__device__ __forceinline__ void plant_log_rows(const TickArgs &a, int robot, float *&lg, float *&lu) {
+    const int R = gridDim.y;
+    const int pt = a.loop_state ? (int)(__ldcg(a.loop_state) - __ldcg(a.loop_state + 1)) : a.plant_tick;
+    lg = a.plant_log + 4 * ((size_t)(pt + 1) * R + robot);
+    lu = a.plant_log + 4 * (size_t)(a.plant_n + 1) * R + 2 * ((size_t)pt * R + robot);
+}
+
 // A13-A15 + Q8 from the merged triple in ms.col: normalise, filter, update, shift, publish.
 __device__ void finalize_tick(const TickArgs &a, int robot, int idx_new, MergeSmem &ms) {
     const int tid = threadIdx.x, T = a.T;
@@ -210,9 +220,21 @@ __device__ void finalize_tick(const TickArgs &a, int robot, int idx_new, MergeSm
     float *out = a.out + (size_t)robot * MPPI_OUT_STRIDE;
     // eta = sum of exp(-(S - min S)/tau) >= 1 whenever the costs are finite.  NaN / inf costs (a NaN observed state, a
     // learned residual that diverged, a missed hand-off in the learned-dynamics kernel) must not poison the nominal for
-    // good: the tick is NOT applied and the fault is reported to the host (MPPI_E_NUMERIC).
+    // good: the tick is NOT applied and the fault is reported to the host (MPPI_E_NUMERIC).  In a fleet only this robot's
+    // tick is refused: its u0 row and this tick's plant-log rows read NaN (not the previous tick's control), its nominal,
+    // waypoint index and plant state stay as they were; every other robot owns its CTAs and is unaffected.
     if (!(eta > 0.f && eta < CUDART_INF_F)) {
-        if (tid == 0) { out[MPPI_OUT_FAULT] = 1.f; if (robot == 0 && a.out_host) a.out_host[MPPI_OUT_FAULT] = 1.f; }
+        if (tid == 0) {
+            out[MPPI_OUT_FAULT] = 1.f;
+            if (robot == 0 && a.out_host) a.out_host[MPPI_OUT_FAULT] = 1.f;
+            if (a.u0_out) { a.u0_out[2 * robot] = CUDART_NAN_F; a.u0_out[2 * robot + 1] = CUDART_NAN_F; }
+            if (a.plant_state) {
+                float *lg, *lu;
+                plant_log_rows(a, robot, lg, lu);
+                lg[0] = lg[1] = lg[2] = lg[3] = CUDART_NAN_F;
+                lu[0] = lu[1] = CUDART_NAN_F;
+            }
+        }
         return;
     }
     for (int c = tid; c < 2 * T; c += MPPI_BLOCK) ms.weps[c] = ms.col[4 + c] * inv_eta;
@@ -251,8 +273,6 @@ __device__ void finalize_tick(const TickArgs &a, int robot, int idx_new, MergeSm
         if (a.plant_state) {
             // A17: plant step between ticks.  0: DifferentialDrive.update_state (mppi_differential_drive.py:33-40),
             // unclamped u0; 1: Vehicle.update (models/vehicle.py:95-110), clamp then Euler bicycle.  One plant per robot.
-            const int R = gridDim.y;
-            const int pt = a.loop_state ? (int)(__ldcg(a.loop_state) - __ldcg(a.loop_state + 1)) : a.plant_tick;
             float *ps = a.plant_state + 4 * robot;
             float px = ps[0], py = ps[1], pyaw = ps[2], pv = ps[3];
             float sn, cs;
@@ -264,9 +284,9 @@ __device__ void finalize_tick(const TickArgs &a, int robot, int idx_new, MergeSm
                 px += pv * cs * a.dt; py += pv * sn * a.dt; pyaw += pv * a.dt_over_L * tanf(steer); pv += accel * a.dt;
             }
             ps[0] = px; ps[1] = py; ps[2] = pyaw; ps[3] = pv;
-            float *lg = a.plant_log + 4 * ((size_t)(pt + 1) * R + robot);
+            float *lg, *lu;
+            plant_log_rows(a, robot, lg, lu);
             lg[0] = px; lg[1] = py; lg[2] = pyaw; lg[3] = pv;
-            float *lu = a.plant_log + 4 * (size_t)(a.plant_n + 1) * R + 2 * ((size_t)pt * R + robot);
             lu[0] = u0x; lu[1] = u0y;
         }
         if (!(a.flags & F_KEEP_IDX)) a.idx[robot] = idx_new;
@@ -928,11 +948,31 @@ size_t mppi_tick_dyn_smem(int T, int stash) {
     return stash ? std::max(sizeof(float2) * (size_t)T * MPPI_CHUNK, small) : small;
 }
 
+// Opt-in of a tick kernel to `dyn` bytes of dynamic shared memory on the current device.  The attribute belongs to the
+// function, so every handle of an instantiation shares it: it is only ever RAISED, under one process-wide record of the
+// largest opt-in per (kernel, device).  Setting it to each new handle's own size would cut it below what a live handle with a
+// longer horizon launches with, and that handle's next tick would fail with cudaErrorInvalidValue.
+static cudaError_t raise_dyn_smem_limit(const void *kern, int dev, size_t dyn) {
+    struct OptIn { const void *kern; int dev; size_t dyn; };
+    static std::mutex mu;
+    static std::vector<OptIn> done;
+    std::lock_guard<std::mutex> lock(mu);
+    OptIn *rec = nullptr;
+    for (OptIn &o : done)
+        if (o.kern == kern && o.dev == dev) { rec = &o; break; }
+    if (rec && rec->dyn >= dyn) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+    if (e != cudaSuccess) return e;
+    if (rec) rec->dyn = dyn;
+    else done.push_back({kern, dev, dyn});
+    return cudaSuccess;
+}
+
 cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_kind, bool sum, bool inj, int stash, dim3 grid, cudaStream_t st) {
     const size_t dyn = mppi_tick_dyn_smem(a.T, stash);
     return with_tick_kernel(model, coll, cost_kind, sum, inj, a.window == 20, stash, [&](auto kern) {
         if (dyn > 32 * 1024) {          // static shared memory (12 KB) counts against the 48 KB default limit too
-            // opt in to > 48 KB of dynamic shared memory once per (instantiation, device), not on every tick
+            // lock-free fast path: a limit this thread has seen at >= dyn is still >= dyn (it only rises)
             static thread_local const void *done_kern[64];
             static thread_local size_t done_dyn[64];
             static thread_local int done_dev[64], n_done = 0;
@@ -942,7 +982,7 @@ cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_ki
             for (int i = 0; i < n_done; ++i)
                 if (done_kern[i] == (const void *)kern && done_dev[i] == dev && done_dyn[i] >= dyn) { found = true; break; }
             if (!found) {
-                cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+                cudaError_t e = raise_dyn_smem_limit((const void *)kern, dev, dyn);
                 if (e != cudaSuccess) return e;
                 if (n_done < 64) { done_kern[n_done] = (const void *)kern; done_dyn[n_done] = dyn; done_dev[n_done] = dev; ++n_done; }
             }
@@ -958,7 +998,9 @@ int mppi_tick_occupancy(int model, int coll, int cost_kind, bool sum, bool inj, 
     const size_t dyn = mppi_tick_dyn_smem(T, stash);
     cudaError_t e = with_tick_kernel(model, coll, cost_kind, sum, inj, window == 20, stash, [&](auto kern) {
         if (dyn > 32 * 1024) {          // static shared memory (12 KB) counts against the 48 KB default limit too
-            cudaError_t e2 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+            int dev = 0;
+            cudaGetDevice(&dev);
+            cudaError_t e2 = raise_dyn_smem_limit((const void *)kern, dev, dyn);
             if (e2 != cudaSuccess) return e2;
         }
         return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, MPPI_BLOCK, dyn);

@@ -242,7 +242,10 @@ int mppi_run_closed_loop(mppi_handle_t h, const double *x0, int32_t n_ticks, uin
 
 /* Batched multi-robot tick: n_robots independent controllers in one launch (no reference
  * equivalent; R copies of the loop at mppi_differential_drive.py:111-141).
- *   d_x0  device (R, nx) float32;  d_u0_out device (R, 2) float32 (may be NULL) */
+ *   d_x0  device (R, nx) float32;  d_u0_out device (R, 2) float32 (may be NULL)
+ * A robot whose sample costs are not finite (NaN state) is not updated: its u0 row reads NaN, its nominal and waypoint
+ * index stay as they were, the other robots are unaffected, and the next mppi_synchronize returns MPPI_E_NUMERIC naming
+ * the first such robot (mppi_run_closed_loop likewise, with that robot's log rows NaN from the faulted tick on). */
 int mppi_step_batched(mppi_handle_t h, const float *d_x0, uint64_t seed, uint64_t tick, float *d_u0_out);
 
 /* Sample sharding across GPUs: each rank owns K of K_global samples; one exchange of
@@ -271,7 +274,8 @@ int mppi_comm_p2p_trace(mppi_handle_t h, uint64_t stamps_out[4]);
 
 /* Diagnostics, no reference counterpart: per-CTA %globaltimer stamps (ns) of the LAST single-robot tick -- out[2b] CTA b
  * entered the kernel, out[2b+1] its rollouts ended; after the n CTAs: out[2n] partials merged, out[2n+1] nominal updated
- * (last CTA).  Shows where a tick's time outside the rollouts goes (profiles/). */
+ * (last CTA).  Shows where a tick's time outside the rollouts goes (profiles/).  *n_ctas_out is the grid width (CTAs per
+ * robot) of the last traced launch, which depends on the rollout path that tick took (regenerate, stash, time-parallel). */
 int mppi_set_trace(mppi_handle_t h, int32_t enabled);
 int mppi_get_trace(mppi_handle_t h, uint64_t *out, int32_t capacity, int32_t *n_ctas_out);
 
