@@ -103,6 +103,11 @@ struct mppi_handle_s {
     int *d_sorted_idx = nullptr, *d_iota = nullptr;
     void *d_sort_temp = nullptr;
     size_t sort_temp_bytes = 0;
+    // per-robot scenes (fleets): one SceneRec per robot, installed by mppi_set_robot_goals / mppi_set_robot_obstacles; the
+    // components in use are args.scene_mask.  scene_stash: the rollout path of the scene instantiation (1 noise stash, 0
+    // regenerate), chosen at the first install; -1 before.
+    SceneRec *d_scene = nullptr;
+    int scene_stash = -1;
     unsigned long long *d_trace = nullptr;     // per-CTA time stamps of the last tick (mppi_set_trace)
     int trace_n = 0;
     int trace_grid = 0;                        // CTAs per robot of the last traced launch
@@ -432,7 +437,7 @@ int mppi_destroy(mppi_handle_t h) {
     gfree(h, h->d_xchg); gfree(h, h->d_trace); gfree(h, h->d_loop);
     if (h->loop_graph) cudaGraphExecDestroy(h->loop_graph);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
-    gfree(h, h->d_paths); gfree(h, h->d_path_len);
+    gfree(h, h->d_paths); gfree(h, h->d_path_len); gfree(h, h->d_scene);
     gfree(h, h->d_Sc); gfree(h, h->d_Ssorted); gfree(h, h->d_sorted_idx); gfree(h, h->d_iota); gfree(h, h->d_sort_temp);
     if (h->mlp) mlp_destroy(h->mlp);
     gfree(h, h->d_path); gfree(h, h->d_U); gfree(h, h->d_M); gfree(h, h->d_S); gfree(h, h->d_part);
@@ -555,6 +560,7 @@ int mppi_set_obstacles(mppi_handle_t h, const double *xyr, int32_t m) {
     if (!h || m < 0 || m > MPPI_MAX_OBSTACLES || (m > 0 && !xyr)) return MPPI_E_BADARG;
     if (h->cfg.cost_kind == MPPI_COSTKIND_TARGET_SOFT) return fail(h, MPPI_E_STATE, "TARGET_SOFT takes mppi_set_moving_obstacles");
     refresh_obstacle_args(h, xyr, m);
+    h->args.scene_mask &= ~MPPI_SCENE_OBS;                 // back to one shared obstacle set
     return MPPI_OK;
 }
 
@@ -562,6 +568,7 @@ int mppi_set_goal(mppi_handle_t h, const double *goal, int32_t n) {
     if (!h || !goal || n < 2 || n > 3) return MPPI_E_BADARG;
     if (h->cfg.cost_kind == MPPI_COSTKIND_PATH) return fail(h, MPPI_E_STATE, "handle was not created with a goal / target cost kind");
     for (int i = 0; i < n; ++i) { h->cfg.goal[i] = goal[i]; h->args.goal[i] = (float)goal[i]; }
+    h->args.scene_mask &= ~MPPI_SCENE_GOAL;                // back to one shared goal
     return MPPI_OK;
 }
 
@@ -574,7 +581,84 @@ int mppi_set_moving_obstacles(mppi_handle_t h, const double *pos, const double *
         a.obs_x[i] = (float)pos[2 * i]; a.obs_y[i] = (float)pos[2 * i + 1];
         a.obs_vx[i] = (float)vel[2 * i]; a.obs_vy[i] = (float)vel[2 * i + 1];
     }
+    a.scene_mask &= ~MPPI_SCENE_OBS;                       // back to one shared obstacle set
     return MPPI_OK;
+}
+
+// ---- per-robot scenes (fleets) ---------------------------------------------------------------------------------------------
+// Checks common to both installs; allocates the table and picks the scene instantiation's rollout path on first use: the
+// handle's noise-stash path (time-parallel handles too: the scene instantiations have no time-parallel variant) when that
+// kernel can be resident, else its regenerate-noise variant.  The grid widths stay the ones mppi_create computed.
+static int scene_modes_supported(mppi_handle_t h) {
+    if (h->strict || h->mlp) return fail(h, MPPI_E_UNSUPPORTED, "per-robot goals / obstacles: frozen waypoint mode, analytic dynamics");
+    if (h->world > 1) return fail(h, MPPI_E_UNSUPPORTED, "per-robot goals / obstacles: one GPU (no sample sharding)");
+    return MPPI_OK;
+}
+
+static int prepare_scene(mppi_handle_t h) {
+    CK(h, cudaSetDevice(h->cfg.device));
+    if (h->scene_stash < 0) {
+        const mppi_config_t &c = h->cfg;
+        const bool want_stash = h->stash || h->tpar;
+        const int occ_st = want_stash ? mppi_tick_occupancy(c.model, c.collision, c.cost_kind, h->sum, false, c.window, c.T, 1, true) : 0;
+        const int occ_rg = occ_st >= 1 ? 0 : mppi_tick_occupancy(c.model, c.collision, c.cost_kind, h->sum, false, c.window, c.T, 0, true);
+        if (occ_st < 1 && occ_rg < 1)
+            return fail(h, MPPI_E_UNSUPPORTED, "per-robot goals / obstacles are built for diff-drive + circles and bicycle + footprint "
+                                               "on a path, and for the GOAL (no obstacles or circles) and TARGET_SOFT cost kinds");
+        h->scene_stash = occ_st >= 1 ? 1 : 0;
+        if (std::getenv("MPPI_VERBOSE"))
+            std::fprintf(stderr, "mppi_set_robot_*: scene ticks take the %s path, %d CTAs per robot (occ %d)%s\n",
+                         h->scene_stash ? "stash" : "regenerate", h->scene_stash ? h->grid_x_stash : h->grid_x,
+                         h->scene_stash ? occ_st : occ_rg,
+                         h->tpar ? "; this handle's shared-scene ticks are time-parallel, its scene ticks are not" : "");
+    }
+    if (!h->d_scene) {
+        CK(h, gmalloc(h, &h->d_scene, sizeof(SceneRec) * h->cfg.n_robots));
+        CK(h, cudaMemsetAsync(h->d_scene, 0, sizeof(SceneRec) * h->cfg.n_robots, h->stream));
+    }
+    return MPPI_OK;
+}
+
+int mppi_set_robot_obstacles(mppi_handle_t h, const float *d_obs, const int32_t *d_count, int32_t m, int32_t ncol) {
+    if (!h || m < 0 || m > MPPI_MAX_OBSTACLES || (ncol != 3 && ncol != 4) || (m > 0 && !d_obs)) return MPPI_E_BADARG;
+    if (int rc = scene_modes_supported(h)) return rc;
+    const mppi_config_t &c = h->cfg;
+    if (ncol == 4 && c.cost_kind != MPPI_COSTKIND_TARGET_SOFT)
+        return fail(h, MPPI_E_STATE, "moving obstacles [x, y, vx, vy] belong to MPPI_COSTKIND_TARGET_SOFT handles");
+    if (ncol == 3 && (c.cost_kind == MPPI_COSTKIND_TARGET_SOFT || c.collision == MPPI_COLLISION_NONE))
+        return fail(h, MPPI_E_STATE, "static circles [x, y, r] need a handle created with circle or footprint collision");
+    if (int rc = prepare_scene(h)) return rc;
+    const double hl = 0.5 * c.vehicle_l * c.margin, hw = 0.5 * c.vehicle_w * c.margin;       // as refresh_obstacle_args
+    CK(h, mppi_launch_scene_obstacles(d_obs, d_count, c.n_robots, m, ncol, c.collision == MPPI_COLLISION_CIRCLE,
+                                      c.robot_radius * c.margin, std::sqrt(hl * hl + hw * hw), h->d_scene, h->stream));
+    h->tm.launches++;
+    h->args.scene = h->d_scene;
+    h->args.scene_mask |= MPPI_SCENE_OBS;
+    return MPPI_OK;
+}
+
+int mppi_set_robot_goals(mppi_handle_t h, const float *d_goal, int32_t n) {
+    if (!h || !d_goal || n < 2 || n > 3) return MPPI_E_BADARG;
+    if (int rc = scene_modes_supported(h)) return rc;
+    const int kind = h->cfg.cost_kind;
+    if (kind == MPPI_COSTKIND_PATH) return fail(h, MPPI_E_STATE, "handle was not created with a goal / target cost kind");
+    if (n != (kind == MPPI_COSTKIND_GOAL ? 2 : 3))
+        return fail(h, MPPI_E_BADARG, "per-robot goals: n = 2 (GOAL: goal point) or 3 (TARGET_SOFT: target pose)");
+    if (int rc = prepare_scene(h)) return rc;
+    CK(h, mppi_launch_scene_goals(d_goal, h->cfg.n_robots, n, h->d_scene, h->stream));
+    h->tm.launches++;
+    h->args.scene = h->d_scene;
+    h->args.scene_mask |= MPPI_SCENE_GOAL;
+    return MPPI_OK;
+}
+
+// The per-robot scene is threaded through the fleet tick (mppi_step_batched, mppi_run_closed_loop) only.
+static int scene_refused(mppi_handle_t h, const char *what) {
+    if (!h->args.scene_mask) return MPPI_OK;
+    h->err = std::string(what) + ": per-robot goals / obstacles are installed; they are run by mppi_step_batched and "
+                                 "mppi_run_closed_loop (mppi_set_goal / mppi_set_obstacles / mppi_set_moving_obstacles "
+                                 "return the handle to the shared scene)";
+    return MPPI_E_STATE;
 }
 
 int mppi_set_nominal(mppi_handle_t h, const float *u) {
@@ -744,7 +828,8 @@ static int strict_costs(mppi_handle_t h, const double *x0, const float *d_eps, f
 }
 
 static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
-    const int stash = (!inj && !(a.flags & F_FROM_S)) ? (h->tpar ? 2 : h->stash ? 1 : 0) : 0;
+    const bool scene = a.scene_mask != 0;                // only the fleet entry points get here with a scene installed
+    const int stash = scene ? h->scene_stash : (!inj && !(a.flags & F_FROM_S)) ? (h->tpar ? 2 : h->stash ? 1 : 0) : 0;
     dim3 grid(stash == 2 ? h->grid_x_tpar : stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
     if (a.trace) h->trace_grid = (int)grid.x;
     const int model = (h->cfg.model == MPPI_MODEL_DIFFDRIVE_MLP) ? MPPI_MODEL_DIFFDRIVE : h->cfg.model;
@@ -769,7 +854,7 @@ static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
         h->tm.launches += 2;
         return MPPI_OK;
     }
-    CK(h, mppi_launch_tick(a, model, h->cfg.collision, h->cfg.cost_kind, h->sum, inj, stash, grid, h->stream));
+    CK(h, mppi_launch_tick(a, model, h->cfg.collision, h->cfg.cost_kind, h->sum, inj, stash, grid, h->stream, scene));
     h->tm.launches++;
     return MPPI_OK;
 }
@@ -779,6 +864,7 @@ static int step_common(mppi_handle_t h, const double *x0, const float *d_eps, ui
     if (!h || !x0) return MPPI_E_BADARG;
     if (!h->have_path) return fail(h, MPPI_E_STATE, "mppi_set_ref_path has not been called");
     if (h->cfg.n_robots != 1) return fail(h, MPPI_E_BADARG, "use mppi_step_batched for n_robots > 1");
+    if (int rc = scene_refused(h, "mppi_step")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     set_x0(h, x0);
     set_seed(h, seed, tick);
@@ -842,6 +928,7 @@ int mppi_rollout_costs(mppi_handle_t h, const double *x0, const float *d_eps, ui
     if (!h || !x0 || !d_S) return MPPI_E_BADARG;
     if (!h->have_path) return fail(h, MPPI_E_STATE, "mppi_set_ref_path has not been called");
     if (h->cfg.n_robots != 1) return MPPI_E_BADARG;
+    if (int rc = scene_refused(h, "mppi_rollout_costs")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     set_x0(h, x0);
     set_seed(h, seed, tick);
@@ -878,6 +965,7 @@ int mppi_reduce_update(mppi_handle_t h, const float *d_S, const float *d_eps, ui
     if (!h || !d_S) return MPPI_E_BADARG;
     if (!h->have_path) return fail(h, MPPI_E_STATE, "mppi_set_ref_path has not been called");
     if (h->cfg.n_robots != 1) return MPPI_E_BADARG;
+    if (int rc = scene_refused(h, "mppi_reduce_update")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     set_seed(h, seed, tick);
     TickArgs a = h->args;
@@ -912,6 +1000,7 @@ int mppi_get_trajectories(mppi_handle_t h, const double *x0, const float *d_eps,
                           float *optimal_out, float *d_sampled_out) {
     if (!h || !x0) return MPPI_E_BADARG;
     if (h->cfg.n_robots != 1 || h->mlp) return fail(h, MPPI_E_UNSUPPORTED, "trajectories: single-robot analytic models only");
+    if (int rc = scene_refused(h, "mppi_get_trajectories")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     set_x0(h, x0);
     set_seed(h, seed, tick);
@@ -949,6 +1038,7 @@ int mppi_get_top_trajectories(mppi_handle_t h, const double *x0, const float *d_
     if (!h || !x0 || n_top < 1 || n_top > h->cfg.K || !d_traj_out || index_shift < 0 || index_shift > 1) return MPPI_E_BADARG;
     if (h->cfg.n_robots != 1 || h->mlp) return fail(h, MPPI_E_UNSUPPORTED, "trajectories: single-robot analytic models only");
     if (!h->keep_costs || !h->d_Sc) return fail(h, MPPI_E_STATE, "call mppi_set_keep_costs(h, 1) before the tick");
+    if (int rc = scene_refused(h, "mppi_get_top_trajectories")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     set_x0(h, x0);
     set_seed(h, seed, tick);
@@ -1002,7 +1092,8 @@ int mppi_run_closed_loop(mppi_handle_t h, const double *x0, int32_t n_ticks, uin
     // The n ticks as ONE CUDA graph of n identical kernel nodes: every launch carries the same arguments (the running tick
     // and the log row come from d_loop, advanced by each launch's last CTA), so the instantiated graph is reused by every
     // later call with the same (n_ticks, plant, seed, sample-cost flag, obstacle set); MPPI_CLOSED_LOOP_GRAPH=0 falls back
-    // to n stream launches (A/B measurements).
+    // to n stream launches (A/B measurements).  Per-robot goals / obstacles are read from the handle's table, whose pointer
+    // never changes: re-installing them between calls does not re-instantiate the graph.
     set_seed(h, seed, 0);
     TickArgs a = h->args;
     a.x0_dev = h->d_x0; a.eps = nullptr; a.S = nullptr; a.flags = F_UPDATE;
@@ -1066,9 +1157,11 @@ int mppi_step_batched(mppi_handle_t h, const float *d_x0, uint64_t seed, uint64_
                             h->cfg.n_robots, cudaMemcpyDeviceToDevice, h->stream));
     a.x0_dev = h->d_x0; a.eps = nullptr; a.S = nullptr; a.flags = F_UPDATE; a.u0_out = d_u0_out;
     a.out_host = nullptr;
-    dim3 grid(h->stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
+    const bool scene = a.scene_mask != 0;
+    const int stash = scene ? h->scene_stash : h->stash ? 1 : 0;
+    dim3 grid(stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
     if (a.trace) h->trace_grid = (int)grid.x;
-    CK(h, mppi_launch_tick(a, h->cfg.model, h->cfg.collision, h->cfg.cost_kind, h->sum, false, h->stash ? 1 : 0, grid, h->stream));
+    CK(h, mppi_launch_tick(a, h->cfg.model, h->cfg.collision, h->cfg.cost_kind, h->sum, false, stash, grid, h->stream, scene));
     h->tm.launches++;
     return MPPI_OK;
 }
@@ -1086,6 +1179,7 @@ int mppi_comm_get_unique_id(void *out128) {
 int mppi_comm_init(mppi_handle_t h, const void *uid, int32_t rank, int32_t world) {
     if (!h || !uid || world < 1 || rank < 0 || rank >= world) return MPPI_E_BADARG;
     if (h->cfg.n_robots != 1 || h->strict) return fail(h, MPPI_E_UNSUPPORTED, "sample sharding needs frozen mode, one robot");
+    if (int rc = scene_refused(h, "mppi_comm_init")) return rc;
     if (!g_nccl.load()) return fail(h, MPPI_E_NCCL, "cannot load libnccl.so.2");
     CK(h, cudaSetDevice(h->cfg.device));
     ncclUniqueId id;
@@ -1102,6 +1196,7 @@ int mppi_comm_init(mppi_handle_t h, const void *uid, int32_t rank, int32_t world
 int mppi_comm_p2p_export(mppi_handle_t h, int32_t world, void *out64) {
     if (!h || !out64 || world < 2 || world > MPPI_MAX_PEERS) return MPPI_E_BADARG;
     if (h->cfg.n_robots != 1 || h->strict) return fail(h, MPPI_E_UNSUPPORTED, "sample sharding needs frozen mode, one robot");
+    if (int rc = scene_refused(h, "mppi_comm_p2p_export")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     if (!h->d_xchg) {
         CK(h, gmalloc(h, &h->d_xchg, sizeof(unsigned long long) * MPPI_XCHG_TOTAL));
@@ -1118,6 +1213,7 @@ int mppi_comm_p2p_export(mppi_handle_t h, int32_t world, void *out64) {
 int mppi_comm_p2p_open(mppi_handle_t h, const void *handles, int32_t rank, int32_t world) {
     if (!h || !handles || world < 2 || world > MPPI_MAX_PEERS || rank < 0 || rank >= world) return MPPI_E_BADARG;
     if (!h->d_xchg) return fail(h, MPPI_E_STATE, "call mppi_comm_p2p_export first");
+    if (int rc = scene_refused(h, "mppi_comm_p2p_open")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     for (int p = 0; p < world; ++p) {
         if (p == rank) { h->peer_buf[p] = h->d_xchg; continue; }
@@ -1178,6 +1274,7 @@ int mppi_debug_check_guards(mppi_handle_t h) {
 int mppi_comm_p2p_barrier(mppi_handle_t h) {
     if (!h) return MPPI_E_BADARG;
     if (!h->p2p || h->world < 2) return fail(h, MPPI_E_STATE, "no fused exchange on this handle");
+    if (int rc = scene_refused(h, "mppi_comm_p2p_barrier")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     TickArgs b = h->args;
     for (int p = 0; p < h->world; ++p) b.peer_buf[p] = h->peer_buf[p];
@@ -1190,6 +1287,7 @@ int mppi_comm_p2p_barrier(mppi_handle_t h) {
 int mppi_comm_p2p_trace(mppi_handle_t h, uint64_t stamps_out[4]) {
     if (!h || !stamps_out) return MPPI_E_BADARG;
     if (!h->p2p || !h->d_xchg) return fail(h, MPPI_E_STATE, "no fused exchange on this handle");
+    if (int rc = scene_refused(h, "mppi_comm_p2p_trace")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaMemcpyAsync(stamps_out, h->d_xchg + MPPI_XCHG_WORDS, sizeof(uint64_t) * 4, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <math_constants.h>
+#include <type_traits>
 #include "../../include/mppi_b200.h"
 
 // -DMPPI_DEBUG_CHECKS=1: device-side bounds / protocol assertions at every shared-memory and global hand-off (the build the
@@ -62,6 +63,19 @@ enum : int {
     F_P2P = 128,         // multi-GPU: exchange the per-GPU triples over peer memory inside this kernel
     F_COST_SUM = 0x10000 // MLP kernel: cost_mode == sum (the tick kernel takes it as a template argument)
 };
+
+// One robot's scene in a fleet (mppi_set_robot_goals / mppi_set_robot_obstacles): the handle keeps one record per robot
+// ([R], device), and a scene tick kernel loads its robot's record into shared memory in the prologue.  The fields carry the
+// names TickArgs gives the shared scene, so collided / goal_cost / target_soft_cost read either one through a template.
+struct SceneRec {
+    float goal[4];                        // GOAL: (x, y); TARGET_SOFT: desired pose (x, y, yaw)
+    int n_obs, pad_[3];                   // obstacles this robot uses (rows 0 .. n_obs - 1)
+    float obs_x[MPPI_MAX_OBSTACLES], obs_y[MPPI_MAX_OBSTACLES];
+    float obs_r2[MPPI_MAX_OBSTACLES], obs_far2[MPPI_MAX_OBSTACLES];     // as refresh_obstacle_args computes them (FP64)
+    float obs_vx[MPPI_MAX_OBSTACLES], obs_vy[MPPI_MAX_OBSTACLES];       // TARGET_SOFT: moving obstacles
+};
+#define MPPI_SCENE_GOAL 1                 // TickArgs::scene_mask: the goal comes from the per-robot table
+#define MPPI_SCENE_OBS 2                  // ... the obstacles come from the per-robot table
 
 // Everything a tick needs, passed by value (kernel parameter = constant bank).
 struct TickArgs {
@@ -122,6 +136,10 @@ struct TickArgs {
     unsigned p2p_timeout_ms;          // a peer that has not published within this time fails the tick (MPPI_E_NCCL)
     unsigned long long *trace;        // diagnostics (mppi_set_trace): %globaltimer of CTA b's start [2b] and end of its rollouts
                                       // [2b+1], then the last CTA's merge done [2B] and nominal updated [2B+1]; or null
+    // per-robot scenes (read by the scene instantiations of the tick kernel only): [R] records; the components named in
+    // scene_mask come from the robot's record, the others from the shared fields above
+    const SceneRec *scene;
+    int scene_mask;
 };
 
 // ------------------------------------------------------------------------------------------
@@ -567,26 +585,62 @@ __device__ __forceinline__ float wrap_2pi(float yaw) {
     return r;
 }
 
-// A10: collision tests.  Returns true if the state collides with any obstacle.
+// A10: collision tests.  Returns true if the state collides with any obstacle.  The obstacles come from `sc`: the shared
+// set in TickArgs (sc is `a`), or a robot's SceneRec in shared memory (scene instantiations).
+// A per-robot obstacle set (SceneRec in shared memory): the same tests, walked one obstacle per trip -- its operands are
+// shared-memory loads, and unrolled trips would hold several obstacles' worth of them in registers.
 template <int MODEL, int COLL>
-__device__ __forceinline__ bool collided(const TickArgs &a, float x, float y, float cs, float sn) {
+__device__ __forceinline__ bool collided_scene(const TickArgs &a, const SceneRec &sc, float x, float y, float cs, float sn) {
+    bool hit = false;
+    if constexpr (COLL == MPPI_COLLISION_CIRCLE) {
+#pragma unroll 1
+        for (int m = 0; m < sc.n_obs; ++m) {
+            const float dx = x - sc.obs_x[m], dy = y - sc.obs_y[m];
+            hit |= (dx * dx + dy * dy < sc.obs_r2[m]);
+        }
+    } else if constexpr (COLL == MPPI_COLLISION_FOOTPRINT) {
+#pragma unroll 1
+        for (int m = 0; m < sc.n_obs; ++m) {
+            const float cx = x - sc.obs_x[m], cy = y - sc.obs_y[m];
+            if (cx * cx + cy * cy >= sc.obs_far2[m]) continue;
+            const float r2 = sc.obs_r2[m];
+            const float ac = a.fp_hl * cs, as = a.fp_hl * sn, bc = a.fp_hw * cs, bs = a.fp_hw * sn;
+            float px, py;
+            px = cx - ac;      py = cy - as;      hit |= (px * px + py * py < r2);
+            px = cx - ac - bs; py = cy - as + bc; hit |= (px * px + py * py < r2);
+            px = cx - bs;      py = cy + bc;      hit |= (px * px + py * py < r2);
+            px = cx + ac - bs; py = cy + as + bc; hit |= (px * px + py * py < r2);
+            px = cx + ac;      py = cy + as;      hit |= (px * px + py * py < r2);
+            px = cx + ac + bs; py = cy + as - bc; hit |= (px * px + py * py < r2);
+            px = cx + bs;      py = cy - bc;      hit |= (px * px + py * py < r2);
+            px = cx - ac + bs; py = cy - as - bc; hit |= (px * px + py * py < r2);
+        }
+    }
+    return hit;
+}
+
+// A10: collision tests.  Returns true if the state collides with any obstacle.  The obstacles come from `sc`: the shared
+// set in TickArgs (sc is `a`, constant-bank operands), or a robot's SceneRec in shared memory (scene instantiations).
+template <int MODEL, int COLL, class SC>
+__device__ __forceinline__ bool collided(const TickArgs &a, const SC &sc, float x, float y, float cs, float sn) {
+    if constexpr (!std::is_same<SC, TickArgs>::value) return collided_scene<MODEL, COLL>(a, sc, x, y, cs, sn);
     bool hit = false;
     if constexpr (COLL == MPPI_COLLISION_NONE) {
         return false;
     } else if constexpr (COLL == MPPI_COLLISION_CIRCLE) {        // mppi_differential_drive_obs.py:301-313
-        for (int m = 0; m < a.n_obs; ++m) {
-            const float dx = x - a.obs_x[m], dy = y - a.obs_y[m];
-            hit |= (dx * dx + dy * dy < a.obs_r2[m]);
+        for (int m = 0; m < sc.n_obs; ++m) {
+            const float dx = x - sc.obs_x[m], dy = y - sc.obs_y[m];
+            hit |= (dx * dx + dy * dy < sc.obs_r2[m]);
         }
         return hit;
     } else {
     // footprint: 8 perimeter points of the (l*margin) x (w*margin) box rotated by the raw yaw
     // (mppi_race_car_obstacle.py:255-274)
-    for (int m = 0; m < a.n_obs; ++m) {
-        const float ox = a.obs_x[m], oy = a.obs_y[m];
+    for (int m = 0; m < sc.n_obs; ++m) {
+        const float ox = sc.obs_x[m], oy = sc.obs_y[m];
         const float cx = x - ox, cy = y - oy;
-        if (cx * cx + cy * cy >= a.obs_far2[m]) continue;      // conservative reject
-        const float r2 = a.obs_r2[m];
+        if (cx * cx + cy * cy >= sc.obs_far2[m]) continue;      // conservative reject
+        const float r2 = sc.obs_r2[m];
         const float ac = a.fp_hl * cs, as = a.fp_hl * sn, bc = a.fp_hw * cs, bs = a.fp_hw * sn;
         float px, py;
         px = cx - ac;      py = cy - as;      hit |= (px * px + py * py < r2);   // (-hl, 0)
@@ -619,8 +673,9 @@ __device__ __forceinline__ float tracking_cost(const float4 ref, const float z[4
 // Goal-point cost of test/mppi_differential_drive_obs.py:202-232: w0 * |xy - goal|^2 + w1 * wrap(atan2(dy, dx) - yaw)^2
 // with (dx, dy) = xy - goal (the bearing FROM the goal, as the reference writes it) and wrap(a) =
 // atan2(sin a, cos a) in (-pi, pi], evaluated as the FMA remainder a - 2pi*rint(a / 2pi) (only its square is used).
-__device__ __forceinline__ float goal_cost(const TickArgs &a, const float z[4], const float w[4]) {
-    const float dx = z[0] - a.goal[0], dy = z[1] - a.goal[1];
+template <class SC>
+__device__ __forceinline__ float goal_cost(const SC &sc, const float z[4], const float w[4]) {
+    const float dx = z[0] - sc.goal[0], dy = z[1] - sc.goal[1];
     const float d2 = fmaf(dy, dy, dx * dx);
     const float diff = atan2f(dy, dx) - z[2];
     const float k = rintf(diff * 0.15915494309189535f);
@@ -632,16 +687,17 @@ __device__ __forceinline__ float goal_cost(const TickArgs &a, const float z[4], 
 // Running cost of test/test_mppi_diff_obs.py:44-66 for the state reached by horizon step t (time t*dt) under the
 // clamped control (v0, v1): (z - target)^T Q (z - target) + v^T R v + W * sum_m exp(sd - d_m) [d_m < sd] with
 // d_m the distance to obstacle m at pos_m + vel_m * t*dt (:14-20).  `full` = false: the quadratic pose error only.
-__device__ __forceinline__ float target_soft_cost(const TickArgs &a, const float z[4], float v0, float v1, int t,
+template <class SC>
+__device__ __forceinline__ float target_soft_cost(const TickArgs &a, const SC &sc, const float z[4], float v0, float v1, int t,
                                                   const float w[4], bool full) {
-    const float ex = z[0] - a.goal[0], ey = z[1] - a.goal[1], eth = z[2] - a.goal[2];
+    const float ex = z[0] - sc.goal[0], ey = z[1] - sc.goal[1], eth = z[2] - sc.goal[2];
     float c = w[0] * ex * ex + w[1] * ey * ey + w[2] * eth * eth;
     if (full) {
         c += a.ctrl_w[0] * v0 * v0 + a.ctrl_w[1] * v1 * v1;
         const float tt = (float)t * a.dt;
         float soft = 0.f;
-        for (int m = 0; m < a.n_obs; ++m) {
-            const float dx = z[0] - fmaf(a.obs_vx[m], tt, a.obs_x[m]), dy = z[1] - fmaf(a.obs_vy[m], tt, a.obs_y[m]);
+        for (int m = 0; m < sc.n_obs; ++m) {
+            const float dx = z[0] - fmaf(sc.obs_vx[m], tt, sc.obs_x[m]), dy = z[1] - fmaf(sc.obs_vy[m], tt, sc.obs_y[m]);
             const float d = sqrtf(fmaf(dy, dy, dx * dx));
             if (d < a.soft_sd) soft += expf(a.soft_sd - d);
         }
@@ -652,13 +708,13 @@ __device__ __forceinline__ float target_soft_cost(const TickArgs &a, const float
 
 // A9 for every cost kind: the cost of state z reached by horizon step t with weights w.  For the path kinds the
 // waypoint (ref, yaw_eff) found here is kept so the terminal cost of the same state can reuse it.
-template <int MODEL, int WIN>
-__device__ __forceinline__ float eval_state_cost(const TickArgs &a, const TickSmem &sm, const float z[4], float v0, float v1,
-                                                 int t, const float w[4], float4 &ref, float &yaw_eff) {
+template <int MODEL, int WIN, class SC>
+__device__ __forceinline__ float eval_state_cost(const TickArgs &a, const SC &sc, const TickSmem &sm, const float z[4], float v0,
+                                                 float v1, int t, const float w[4], float4 &ref, float &yaw_eff) {
     if constexpr (WIN == MPPI_WIN_GOAL) {
-        return goal_cost(a, z, w);
+        return goal_cost(sc, z, w);
     } else if constexpr (WIN == MPPI_WIN_TARGET) {
-        return target_soft_cost(a, z, v0, v1, t, w, true);
+        return target_soft_cost(a, sc, z, v0, v1, t, w, true);
     } else {
         const int j = nearest_wp<WIN>(sm, z[0], z[1]);
         ref = window_ref(sm, j);
@@ -667,10 +723,10 @@ __device__ __forceinline__ float eval_state_cost(const TickArgs &a, const TickSm
     }
 }
 // terminal cost of the SAME state the last stage cost was evaluated at (A9, :126)
-template <int MODEL, int WIN>
-__device__ __forceinline__ float eval_terminal_cost(const TickArgs &a, const float z[4], const float4 ref, float yaw_eff) {
-    if constexpr (WIN == MPPI_WIN_GOAL) return goal_cost(a, z, a.tw);
-    else if constexpr (WIN == MPPI_WIN_TARGET) return target_soft_cost(a, z, 0.f, 0.f, 0, a.tw, false);
+template <int MODEL, int WIN, class SC>
+__device__ __forceinline__ float eval_terminal_cost(const TickArgs &a, const SC &sc, const float z[4], const float4 ref, float yaw_eff) {
+    if constexpr (WIN == MPPI_WIN_GOAL) return goal_cost(sc, z, a.tw);
+    else if constexpr (WIN == MPPI_WIN_TARGET) return target_soft_cost(a, sc, z, 0.f, 0.f, 0, a.tw, false);
     else return tracking_cost<MODEL>(ref, z, yaw_eff, a.tw);
 }
 
@@ -716,8 +772,8 @@ __device__ __forceinline__ float clampf(float v, float lim) { return fminf(fmaxf
 // The loop is also software-pipelined by hand: the noise of the NEXT timestep pair (Philox + Box-Muller:
 // integer/ALU + MUFU work) is generated in the same straight-line block as the two dynamics/cost
 // steps of the CURRENT pair (FMA-pipe work), so the ALU, MUFU and FMA pipes are busy at the same time.
-template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int SPT>
-__device__ __forceinline__ void rollout_samples(const TickArgs &a, const TickSmem &sm, const uint32_t (&kg)[SPT], const int (&klocal)[SPT],
+template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int SPT, class SC>
+__device__ __forceinline__ void rollout_samples(const TickArgs &a, const SC &sc, const TickSmem &sm, const uint32_t (&kg)[SPT], const int (&klocal)[SPT],
                                                 uint32_t robot, const bool (&exploit)[SPT], float2 *stash, float (&smooth)[SPT], int (&ncoll)[SPT],
                                                 uint32_t tick_add = 0u) {
     const int T = a.T;
@@ -753,10 +809,10 @@ __device__ __forceinline__ void rollout_samples(const TickArgs &a, const TickSme
         dyn_step<MODEL>(a, z[s], v0[s], v1[s], cs[s], sn[s]);
         sincos_cw(z[s][2], sn[s], cs[s]);
         if (SUM) {
-            const float c = eval_state_cost<MODEL, WIN>(a, sm, z[s], v0[s], v1[s], t, a.sw, ref[s], yaw_eff[s]);
+            const float c = eval_state_cost<MODEL, WIN>(a, sc, sm, z[s], v0[s], v1[s], t, a.sw, ref[s], yaw_eff[s]);
             const float2 q = sm.Q[t];                                                // zero when gamma == 0
             acc[s] += c + (q.x * v0[s] + q.y * v1[s]);
-            hit[s] = collided<MODEL, COLL>(a, z[s][0], z[s][1], cs[s], sn[s]);
+            hit[s] = collided<MODEL, COLL>(a, sc, z[s][0], z[s][1], cs[s], sn[s]);
             nc[s] += hit[s] ? 1 : 0;
         }
     };
@@ -790,13 +846,13 @@ __device__ __forceinline__ void rollout_samples(const TickArgs &a, const TickSme
             step(s, T - 1, e[s][0], e[s][1]);
         }
         if (SUM) {                          // terminal cost: same state, same waypoint as the last stage cost (A9)
-            acc[s] += eval_terminal_cost<MODEL, WIN>(a, z[s], ref[s], yaw_eff[s]);
+            acc[s] += eval_terminal_cost<MODEL, WIN>(a, sc, z[s], ref[s], yaw_eff[s]);
             nc[s] += hit[s] ? 1 : 0;
         } else {                            // Q1: only the last stage cost survives, plus terminal
             const float2 q = sm.Q[T - 1];
-            acc[s] = eval_state_cost<MODEL, WIN>(a, sm, z[s], v0[s], v1[s], T - 1, a.sw, ref[s], yaw_eff[s]) + (q.x * v0[s] + q.y * v1[s]);
-            acc[s] += eval_terminal_cost<MODEL, WIN>(a, z[s], ref[s], yaw_eff[s]);
-            nc[s] = collided<MODEL, COLL>(a, z[s][0], z[s][1], cs[s], sn[s]) ? 2 : 0;
+            acc[s] = eval_state_cost<MODEL, WIN>(a, sc, sm, z[s], v0[s], v1[s], T - 1, a.sw, ref[s], yaw_eff[s]) + (q.x * v0[s] + q.y * v1[s]);
+            acc[s] += eval_terminal_cost<MODEL, WIN>(a, sc, z[s], ref[s], yaw_eff[s]);
+            nc[s] = collided<MODEL, COLL>(a, sc, z[s][0], z[s][1], cs[s], sn[s]) ? 2 : 0;
         }
         smooth[s] = acc[s];
         ncoll[s] = nc[s];
@@ -818,7 +874,8 @@ __device__ __forceinline__ void rollout_samples(const TickArgs &a, const TickSme
 //   S  one thread per sample: the T costs added in horizon order -- the same sum, in the same order, as the serial loop.
 // Two such CTAs are resident per SM (T * 64 * 24 B of shared memory each), so one CTA's serial phase D overlaps the other's
 // wide phases.  Same device functions as rollout_samples, so a sample's result does not depend on which rollout ran it.
-// All MPPI_BLOCK threads must call; threads tid < n return their sample, the others (inf, INT_MAX).
+// All MPPI_BLOCK threads must call; threads tid < n return their sample, the others (inf, INT_MAX).  Shared scene only: the
+// per-robot-scene instantiations have no time-parallel variant.
 // ------------------------------------------------------------------------------------------
 #define MPPI_TPAR_SLOTS 64
 #ifndef MPPI_TPAR_PROBE
@@ -940,16 +997,16 @@ __device__ __forceinline__ void rollout_tpar(const TickArgs &a, const TickSmem &
                 const float v1 = clampf(exploit ? __fadd_rn(u.y, e.y) : e.y, a.umax1);
                 float4 ref = make_float4(0.f, 0.f, 0.f, 0.f);
                 float yaw_eff = 0.f;
-                const float c = eval_state_cost<MODEL, WIN>(a, sm, z, v0, v1, t, a.sw, ref, yaw_eff);
+                const float c = eval_state_cost<MODEL, WIN>(a, a, sm, z, v0, v1, t, a.sw, ref, yaw_eff);
                 const float2 q = sm.Q[t];
                 const float cc = c + (q.x * v0 + q.y * v1);
                 bool hit = false;
                 if constexpr (COLL != MPPI_COLLISION_NONE) {
                     float cs, sn;
                     sincos_cw(z[2], sn, cs);
-                    hit = collided<MODEL, COLL>(a, z[0], z[1], cs, sn);
+                    hit = collided<MODEL, COLL>(a, a, z[0], z[1], cs, sn);
                 }
-                const float term = (t == T - 1) ? eval_terminal_cost<MODEL, WIN>(a, z, ref, yaw_eff) : 0.f;
+                const float term = (t == T - 1) ? eval_terminal_cost<MODEL, WIN>(a, a, z, ref, yaw_eff) : 0.f;
                 zbuf[t * MPPI_TPAR_SLOTS + slot] = make_float4(cc, term, hit ? 1.f : 0.f, 0.f);
             }
         }

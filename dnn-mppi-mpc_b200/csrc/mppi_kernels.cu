@@ -313,7 +313,19 @@ struct RunSmem {
 //                  regenerate-the-noise path (injected noise, K2 alone, horizons too long to stash).
 extern __shared__ __align__(16) unsigned char mppi_dyn_smem[];
 
-template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int STASH>      // STASH: 0 regenerate, 1 noise stash, 2 stash + time-parallel rollout
+// The scene a tick scores against: the shared one in TickArgs, or (SCENE) this CTA's copy of its robot's record.
+template <bool SCENE>
+__device__ __forceinline__ auto &scene_src(const TickArgs &a) {
+    if constexpr (SCENE) {
+        __shared__ SceneRec rec;
+        return rec;
+    } else {
+        return a;
+    }
+}
+
+// STASH: 0 regenerate, 1 noise stash, 2 stash + time-parallel rollout.  SCENE: per-robot goal / obstacles (fleets).
+template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int STASH, bool SCENE>
 __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick_add) {
     __shared__ TickSmem sm;
     __shared__ RunSmem run;
@@ -327,6 +339,27 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
     if (a.trace && tid == 0 && robot == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); a.trace[2 * b] = t; }
     // ---- prologue: observed state, step-1 index update (A8 with update=True), window, nominal
     if (tid < 4) sm.x0[tid] = a.x0_dev ? a.x0_dev[robot * 4 + tid] : a.x0[tid];
+    auto &sc = scene_src<SCENE>(a);
+    if constexpr (SCENE) {
+        // this robot's scene, each component from its per-robot record or from the shared fields; the obstacle count is
+        // per CTA, so the obstacle loops stay warp-uniform
+        static_assert(STASH != 2, "scene ticks take the noise-stash or regenerate path");
+        const SceneRec &row = a.scene[robot];
+        const bool pg = a.scene_mask & MPPI_SCENE_GOAL, po = a.scene_mask & MPPI_SCENE_OBS;
+        if (tid < 4) sc.goal[tid] = pg ? row.goal[tid] : a.goal[tid];
+        if (tid == 0) sc.n_obs = po ? row.n_obs : a.n_obs;
+        if (tid < MPPI_MAX_OBSTACLES) {
+            sc.obs_x[tid] = po ? row.obs_x[tid] : a.obs_x[tid];
+            sc.obs_y[tid] = po ? row.obs_y[tid] : a.obs_y[tid];
+            if constexpr (WIN == MPPI_WIN_TARGET) {
+                sc.obs_vx[tid] = po ? row.obs_vx[tid] : a.obs_vx[tid];
+                sc.obs_vy[tid] = po ? row.obs_vy[tid] : a.obs_vy[tid];
+            } else {
+                sc.obs_r2[tid] = po ? row.obs_r2[tid] : a.obs_r2[tid];
+                sc.obs_far2[tid] = po ? row.obs_far2[tid] : a.obs_far2[tid];
+            }
+        }
+    }
     __syncthreads();
     // the robot's reference path: shared, or its own row of the per-robot table (mppi_set_ref_paths_spline)
     const float4 *rpath = a.path_len ? a.path + (size_t)robot * a.path_stride : a.path;
@@ -429,7 +462,7 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
                 for (int s = 0; s < SPT; ++s)
                     if (active[s]) { smooth[s] = Srow[k[s]]; ncoll[s] = a.NC ? a.NC[k[s]] : 0; }
             } else {
-                rollout_samples<MODEL, COLL, SUM, INJ, WIN, SPT>(a, sm, kg, ksafe, (uint32_t)robot, exploit,
+                rollout_samples<MODEL, COLL, SUM, INJ, WIN, SPT>(a, sc, sm, kg, ksafe, (uint32_t)robot, exploit,
                                                                  STASH ? stash + tid : nullptr, smooth, ncoll, tick_add);
 #pragma unroll
                 for (int s = 0; s < SPT; ++s) {
@@ -706,12 +739,14 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
     if (a.trace && tid == 0 && robot == 0) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); a.trace[2 * B + 1] = t; }
 }
 
-template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int STASH>
-__global__ void __launch_bounds__(MPPI_BLOCK, STASH ? MPPI_STASH_BLOCKS : MPPI_MIN_BLOCKS) mppi_tick_kernel(const __grid_constant__ TickArgs a) {
+// (scene instantiations are register-budgeted for MPPI_STASH_BLOCKS resident CTAs on both rollout paths: their obstacle and
+// goal operands are shared-memory loads, not constant-bank operands)
+template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int STASH, bool SCENE = false>
+__global__ void __launch_bounds__(MPPI_BLOCK, (STASH || SCENE) ? MPPI_STASH_BLOCKS : MPPI_MIN_BLOCKS) mppi_tick_kernel(const __grid_constant__ TickArgs a) {
     // graph-captured closed loop: the tick this launch computes is read from device memory (every CTA reads it before any
     // CTA of the same launch can advance it: the advance happens after ALL CTAs have taken a ticket, below)
     const uint32_t tick_add = a.loop_state ? __ldcg(a.loop_state) : 0u;
-    tick_body<MODEL, COLL, SUM, INJ, WIN, STASH>(a, tick_add);
+    tick_body<MODEL, COLL, SUM, INJ, WIN, STASH, SCENE>(a, tick_add);
     if (a.loop_state) {
         __syncthreads();
         if (threadIdx.x == 0) {
@@ -871,7 +906,7 @@ __global__ void __launch_bounds__(MPPI_BLOCK) mppi_strict_kernel(const __grid_co
                 const float u0 = a.U[2 * t], u1 = a.U[2 * t + 1];
                 c += (u0 * a.gq[0] + u1 * a.gq[2]) * v0 + (u0 * a.gq[1] + u1 * a.gq[3]) * v1;
             }
-            const bool hit = collided<MODEL, COLL>(a, z[0], z[1], cs, sn);
+            const bool hit = collided<MODEL, COLL>(a, a, z[0], z[1], cs, sn);
             if (stage && !SUM) { acc = c; nc = hit ? 1 : 0; }      // Q1: assignment
             else { acc += c; nc += hit ? 1 : 0; }
         }
@@ -918,8 +953,41 @@ static cudaError_t with_tick_kernel_mc(bool sum, bool inj, bool win20, int stash
 #undef MPPI_PICK
 }
 
+// Per-robot-scene instantiations: only what fleets launch (Philox noise, noise stash or regenerate, cost mode last / sum)
+// for diff-drive + circles and bicycle + footprint on a path (static and dynamic window), and the path-free kinds.
+template <int MODEL, int COLL, int WIN, typename F>
+static cudaError_t with_scene_kernel_w(bool sum, int stash, F &&f) {
+#define MPPI_PICK(S, ST) return f(mppi_tick_kernel<MODEL, COLL, S, false, WIN, ST, true>)
+    if (sum) { if (stash) MPPI_PICK(true, 1); MPPI_PICK(true, 0); }
+    if (stash) MPPI_PICK(false, 1);
+    MPPI_PICK(false, 0);
+#undef MPPI_PICK
+}
+
 template <typename F>
-static cudaError_t with_tick_kernel(int model, int coll, int cost_kind, bool sum, bool inj, bool win20, int stash, F &&f) {
+static cudaError_t with_scene_kernel(int model, int coll, int cost_kind, bool sum, bool inj, bool win20, int stash, F &&f) {
+    if (inj || stash == 2 || model == MPPI_MODEL_DIFFDRIVE_MLP) return cudaErrorInvalidValue;
+    if (cost_kind == MPPI_COSTKIND_GOAL) {
+        if (coll == MPPI_COLLISION_NONE) return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE, MPPI_WIN_GOAL>(sum, stash, f);
+        if (coll == MPPI_COLLISION_CIRCLE) return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE, MPPI_WIN_GOAL>(sum, stash, f);
+        return cudaErrorInvalidValue;
+    }
+    if (cost_kind == MPPI_COSTKIND_TARGET_SOFT)
+        return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE, MPPI_WIN_TARGET>(sum, stash, f);
+    if (model == MPPI_MODEL_DIFFDRIVE && coll == MPPI_COLLISION_CIRCLE) {
+        if (win20) return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE, 20>(sum, stash, f);
+        return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE, 0>(sum, stash, f);
+    }
+    if (model == MPPI_MODEL_BICYCLE && coll == MPPI_COLLISION_FOOTPRINT) {
+        if (win20) return with_scene_kernel_w<MPPI_MODEL_BICYCLE, MPPI_COLLISION_FOOTPRINT, 20>(sum, stash, f);
+        return with_scene_kernel_w<MPPI_MODEL_BICYCLE, MPPI_COLLISION_FOOTPRINT, 0>(sum, stash, f);
+    }
+    return cudaErrorInvalidValue;
+}
+
+template <typename F>
+static cudaError_t with_tick_kernel(int model, int coll, int cost_kind, bool sum, bool inj, bool win20, int stash, bool scene, F &&f) {
+    if (scene) return with_scene_kernel(model, coll, cost_kind, sum, inj, win20, stash, f);
     if (cost_kind == MPPI_COSTKIND_GOAL) {              // test/mppi_differential_drive_obs.py: unicycle, circle obstacles
         if (model != MPPI_MODEL_DIFFDRIVE) return cudaErrorInvalidValue;
         if (coll == MPPI_COLLISION_NONE) return with_tick_kernel_nopath<MPPI_COLLISION_NONE, MPPI_WIN_GOAL>(sum, inj, stash, f);
@@ -968,9 +1036,10 @@ static cudaError_t raise_dyn_smem_limit(const void *kern, int dev, size_t dyn) {
     return cudaSuccess;
 }
 
-cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_kind, bool sum, bool inj, int stash, dim3 grid, cudaStream_t st) {
+cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_kind, bool sum, bool inj, int stash, dim3 grid,
+                             cudaStream_t st, bool scene) {
     const size_t dyn = mppi_tick_dyn_smem(a.T, stash);
-    return with_tick_kernel(model, coll, cost_kind, sum, inj, a.window == 20, stash, [&](auto kern) {
+    return with_tick_kernel(model, coll, cost_kind, sum, inj, a.window == 20, stash, scene, [&](auto kern) {
         if (dyn > 32 * 1024) {          // static shared memory (12 KB) counts against the 48 KB default limit too
             // lock-free fast path: a limit this thread has seen at >= dyn is still >= dyn (it only rises)
             static thread_local const void *done_kern[64];
@@ -993,10 +1062,10 @@ cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_ki
 }
 
 // Resident CTAs per SM of the instantiation the given modes select (0 if it cannot launch).
-int mppi_tick_occupancy(int model, int coll, int cost_kind, bool sum, bool inj, int window, int T, int stash) {
+int mppi_tick_occupancy(int model, int coll, int cost_kind, bool sum, bool inj, int window, int T, int stash, bool scene) {
     int nb = 0;
     const size_t dyn = mppi_tick_dyn_smem(T, stash);
-    cudaError_t e = with_tick_kernel(model, coll, cost_kind, sum, inj, window == 20, stash, [&](auto kern) {
+    cudaError_t e = with_tick_kernel(model, coll, cost_kind, sum, inj, window == 20, stash, scene, [&](auto kern) {
         if (dyn > 32 * 1024) {          // static shared memory (12 KB) counts against the 48 KB default limit too
             int dev = 0;
             cudaGetDevice(&dev);
@@ -1057,5 +1126,53 @@ cudaError_t mppi_launch_traj(const TickArgs &a, int model, const float *rec, flo
 
 cudaError_t mppi_launch_noise(const TickArgs &a, float *d_out, int robot, cudaStream_t st) {
     mppi_noise_kernel<<<(a.K + 255) / 256, 256, 0, st>>>(a, d_out, robot);
+    return cudaGetLastError();
+}
+
+// ---- per-robot scenes (fleets): the caller's device rows converted into the handle's SceneRec table, in stream order ----
+namespace {
+// thread (r, j): obstacle slot j of robot r; the FP64 arithmetic is spelled out (no FMA contraction) so r2 / far2 carry the
+// bits refresh_obstacle_args gives the same obstacle on the host
+__global__ void mppi_scene_obstacles_kernel(const float *__restrict__ obs, const int *__restrict__ count, int R, int m, int ncol,
+                                            bool circle, double rr_base, double diag, SceneRec *__restrict__ scene) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= R * MPPI_MAX_OBSTACLES) return;
+    const int r = i / MPPI_MAX_OBSTACLES, j = i - r * MPPI_MAX_OBSTACLES;
+    SceneRec &s = scene[r];
+    if (j == 0) s.n_obs = count ? max(0, min(count[r], m)) : m;
+    float x = 0.f, y = 0.f, r2 = 0.f, far2 = 0.f, vx = 0.f, vy = 0.f;
+    if (j < m) {
+        const float *row = obs + ((size_t)r * m + j) * ncol;
+        x = row[0]; y = row[1];
+        if (ncol == 4) {
+            vx = row[2]; vy = row[3];
+        } else {
+            const double rad = (double)row[2];
+            const double rr = circle ? __dadd_rn(rr_base, rad) : rad;
+            r2 = (float)__dmul_rn(rr, rr);
+            const double far = __dadd_rn(__dmul_rn(__dadd_rn(diag, rad), 1.001), 1e-3);
+            far2 = (float)__dmul_rn(far, far);
+        }
+    }
+    s.obs_x[j] = x; s.obs_y[j] = y; s.obs_r2[j] = r2; s.obs_far2[j] = far2; s.obs_vx[j] = vx; s.obs_vy[j] = vy;
+}
+
+__global__ void mppi_scene_goals_kernel(const float *__restrict__ goal, int R, int n, SceneRec *__restrict__ scene) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= R * 4) return;
+    const int r = i >> 2, c = i & 3;
+    scene[r].goal[c] = c < n ? goal[(size_t)r * n + c] : 0.f;
+}
+}  // namespace
+
+cudaError_t mppi_launch_scene_obstacles(const float *d_obs, const int *d_count, int R, int m, int ncol, bool circle,
+                                        double rr_base, double diag, SceneRec *d_scene, cudaStream_t st) {
+    const int n = R * MPPI_MAX_OBSTACLES;
+    mppi_scene_obstacles_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_obs, d_count, R, m, ncol, circle, rr_base, diag, d_scene);
+    return cudaGetLastError();
+}
+
+cudaError_t mppi_launch_scene_goals(const float *d_goal, int R, int n, SceneRec *d_scene, cudaStream_t st) {
+    mppi_scene_goals_kernel<<<(R * 4 + 255) / 256, 256, 0, st>>>(d_goal, R, n, d_scene);
     return cudaGetLastError();
 }

@@ -59,6 +59,8 @@ SYMBOLS = {
     "mppi_set_obstacles": (C.c_int, [_H, _PD, C.c_int32]),
     "mppi_set_goal": (C.c_int, [_H, _PD, C.c_int32]),
     "mppi_set_moving_obstacles": (C.c_int, [_H, _PD, _PD, C.c_int32]),
+    "mppi_set_robot_obstacles": (C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32]),
+    "mppi_set_robot_goals": (C.c_int, [_H, C.c_void_p, C.c_int32]),
     "mppi_set_nominal": (C.c_int, [_H, _PF]),
     "mppi_get_nominal": (C.c_int, [_H, _PF]),
     "mppi_set_waypoint_idx": (C.c_int, [_H, _PI]),

@@ -74,6 +74,11 @@ class MPPIEngine:
         self._useq = (C.c_float * (2 * self.T))()
         self._useq_np = np.frombuffer(self._useq, dtype=np.float32).reshape(self.T, 2)
         self._u0_np = np.frombuffer(self._u0, dtype=np.float32)
+        # the shared scene as last set (use_shared_scene re-installs it after per-robot goals / obstacles)
+        self._cost_kind, self._collision = cost_kind, collision
+        self._shared_goal = np.asarray(c.goal[:2 if cost_kind == "goal" else 3], dtype=np.float64)
+        self._shared_obs = np.zeros((0, 3))
+        self._shared_moving = (np.zeros((0, 2)), np.zeros((0, 2)))
         if obstacles is not None and len(obstacles):
             self.set_obstacles(obstacles)
 
@@ -116,10 +121,12 @@ class MPPIEngine:
     def set_obstacles(self, obstacles):
         o = np.ascontiguousarray(obstacles, dtype=np.float64).reshape(-1, 3)
         self._ck(self.lib.mppi_set_obstacles(self._h, o.ctypes.data_as(_lib._PD), o.shape[0]), "mppi_set_obstacles")
+        self._shared_obs = o.copy()
 
     def set_goal(self, goal):
         g = np.ascontiguousarray(goal, dtype=np.float64).reshape(-1)
         self._ck(self.lib.mppi_set_goal(self._h, g.ctypes.data_as(_lib._PD), g.shape[0]), "mppi_set_goal")
+        self._shared_goal = g.copy()
 
     def set_moving_obstacles(self, pos_xy, vel_xy):
         p = np.ascontiguousarray(pos_xy, dtype=np.float64).reshape(-1, 2)
@@ -128,6 +135,64 @@ class MPPIEngine:
             raise ValueError("positions and velocities must both be (M,2)")
         self._ck(self.lib.mppi_set_moving_obstacles(self._h, p.ctypes.data_as(_lib._PD), v.ctypes.data_as(_lib._PD), p.shape[0]),
                  "mppi_set_moving_obstacles")
+        self._shared_moving = (p.copy(), v.copy())
+
+    def use_shared_scene(self):
+        """Drops per-robot goals / obstacles: every robot scores against the shared goal and obstacle set last given to the
+        constructor or to set_goal / set_obstacles / set_moving_obstacles."""
+        if self._cost_kind != "path":
+            self.set_goal(self._shared_goal)
+        if self._cost_kind == "target_soft":
+            self.set_moving_obstacles(*self._shared_moving)
+        elif self._collision != "none":
+            self.set_obstacles(self._shared_obs)
+
+    def _device_rows(self, a, dtype, shape, what):
+        """(tensor, uploaded) for a per-robot argument: a CUDA tensor is used as it is (read by a kernel on the engine's
+        stream), a host array is uploaded and the upload is waited for."""
+        import torch
+        if isinstance(a, torch.Tensor) and a.is_cuda:
+            if a.dtype != dtype or not a.is_contiguous() or tuple(a.shape) != shape or a.device.index != self.device:
+                raise ValueError("%s must be a contiguous %s CUDA tensor of shape %s on cuda:%d" % (what, dtype, shape, self.device))
+            return a, False
+        t = torch.as_tensor(np.ascontiguousarray(a), dtype=dtype, device="cuda:%d" % self.device).contiguous()
+        if tuple(t.shape) != shape:
+            raise ValueError("%s must have shape %s" % (what, shape))
+        torch.cuda.current_stream(self.device).synchronize()      # the upload is complete before the engine's stream reads it
+        return t, True
+
+    def _after_upload(self, uploaded):
+        if uploaded:                                             # the staged copy must outlive the install kernel
+            import torch
+            torch.cuda.synchronize(self.device)
+
+    def set_robot_obstacles(self, obs, counts=None):
+        """One obstacle set PER ROBOT: obs (R, m, 3) static circles [x, y, r] (circle / footprint collision) or (R, m, 4)
+        moving soft obstacles [x, y, vx, vy] (target_soft), m <= 16; counts (R,) int32: robot r uses its first counts[r]
+        rows (default: all m).  A CUDA tensor is read by a kernel enqueued on the engine's stream, without a host
+        synchronisation: whatever writes it must be ordered before that stream's work (BatchedMPPI runs the engine on torch's
+        current stream, so torch work issued before the call is; a bare engine runs on its own stream unless set_stream
+        is called).  A numpy array is uploaded, which synchronises the device."""
+        import torch
+        shape = tuple(obs.shape)
+        if len(shape) != 3 or shape[0] != self.R or shape[2] not in (3, 4):
+            raise ValueError("obstacles must be (R, m, 3) or (R, m, 4)")
+        d_obs, up1 = self._device_rows(obs, torch.float32, shape, "obstacles")
+        d_cnt, up2 = (None, False) if counts is None else self._device_rows(counts, torch.int32, (self.R,), "counts")
+        self._ck(self.lib.mppi_set_robot_obstacles(self._h, _dptr(d_obs), _dptr(d_cnt), shape[1], shape[2]),
+                 "mppi_set_robot_obstacles")
+        self._after_upload(up1 or up2)
+
+    def set_robot_goals(self, goals):
+        """One goal PER ROBOT: (R, 2) goal points (goal cost kind) or (R, 3) target poses (target_soft).  CUDA tensors and
+        numpy arrays are consumed as by set_robot_obstacles."""
+        import torch
+        shape = tuple(goals.shape)
+        if len(shape) != 2 or shape[0] != self.R:
+            raise ValueError("goals must be (R, 2) or (R, 3)")
+        d_goal, up = self._device_rows(goals, torch.float32, shape, "goals")
+        self._ck(self.lib.mppi_set_robot_goals(self._h, _dptr(d_goal), shape[1]), "mppi_set_robot_goals")
+        self._after_upload(up)
 
     def set_nominal(self, u):
         u = np.ascontiguousarray(u, dtype=np.float32).reshape(self.R * self.T * 2)

@@ -158,6 +158,24 @@ int mppi_set_goal(mppi_handle_t h, const double *goal, int32_t n);
 /* TARGET_SOFT: circular soft obstacles moving at constant velocity, position at horizon step t (time t*dt) =
  * pos + vel * (t*dt)  (`get_obstacle_positions`, test/test_mppi_diff_obs.py:14-20).  pos_xy, vel_xy: (M,2) doubles */
 int mppi_set_moving_obstacles(mppi_handle_t h, const double *pos_xy, const double *vel_xy, int32_t m);
+/* Fleets with their OWN SCENE PER ROBOT (batched handles).  Each call enqueues one small kernel on the handle's stream that
+ * converts the caller's rows into a handle-owned per-robot table (r2 / far2 in FP64, as mppi_set_obstacles computes them);
+ * the caller may overwrite its buffers with work ordered after the call on that stream, and no host synchronisation takes
+ * place.  Goals and obstacles are independent components: the matching shared setter (mppi_set_goal, mppi_set_obstacles,
+ * mppi_set_moving_obstacles) returns that component to the shared value.  mppi_step_batched and mppi_run_closed_loop run
+ * the per-robot scene (the closed-loop graph holds the table's address only, so a re-install between calls takes effect
+ * without re-instantiating it); while a component is installed every other tick entry point (mppi_step, mppi_step_async,
+ * mppi_rollout_costs, mppi_reduce_update, the trajectory viewers, mppi_comm_*) returns MPPI_E_STATE.
+ * MPPI_E_STATE: a component the handle's kind does not have; MPPI_E_UNSUPPORTED: strict waypoint mode, learned dynamics,
+ * sample sharding, or a model / collision / cost kind without a per-robot-scene kernel (built: diff-drive + circles and
+ * bicycle + footprint on a path, GOAL without obstacles or with circles, TARGET_SOFT).
+ *   d_obs    device (n_robots, m, ncol) float32, 0 <= m <= MPPI_MAX_OBSTACLES;
+ *            ncol = 3: static circles [x, y, r] (CIRCLE / FOOTPRINT collision, like mppi_set_obstacles);
+ *            ncol = 4: moving soft obstacles [x, y, vx, vy] (TARGET_SOFT, like mppi_set_moving_obstacles)
+ *   d_count  device n_robots int32 (robot r uses its first d_count[r] rows, clamped into [0, m]) or NULL (all m) */
+int mppi_set_robot_obstacles(mppi_handle_t h, const float *d_obs, const int32_t *d_count, int32_t m, int32_t ncol);
+/* One goal PER ROBOT: d_goal device (n_robots, n) float32, n = 2 (GOAL: goal_point) or 3 (TARGET_SOFT: target pose). */
+int mppi_set_robot_goals(mppi_handle_t h, const float *d_goal, int32_t n);
 /* `self.u_prev` (T,2) per robot (mppi_differential_drive.py:82) -- host float arrays of n_robots*T*2 */
 int mppi_set_nominal(mppi_handle_t h, const float *u);
 int mppi_get_nominal(mppi_handle_t h, float *u);
