@@ -19,18 +19,10 @@
 #else
 #define MPPI_DCHECK(c) ((void)0)
 #endif
-#ifndef MPPI_BLOCK
-#define MPPI_BLOCK 256
-#endif
+#define MPPI_BLOCK 256                 // threads of a tick CTA, one sample each: a CTA walks its range in chunks of MPPI_BLOCK samples
 #define MPPI_WARPS (MPPI_BLOCK / 32)
-#ifndef MPPI_SPT
-#define MPPI_SPT 1                     // samples per thread of the tick kernel: independent rollouts interleaved in one
-#endif                                 // instruction stream (ILP); a CTA walks its range in chunks of MPPI_CHUNK samples
-#define MPPI_CHUNK (MPPI_BLOCK * MPPI_SPT)
-#ifndef MPPI_MIN_BLOCKS
-#define MPPI_MIN_BLOCKS (MPPI_BLOCK >= 512 ? 1 : 768 / MPPI_BLOCK)   // resident CTAs per SM the regenerate-noise tick kernels are register-budgeted for
-#endif
-#define MPPI_STASH_BLOCKS (MPPI_BLOCK >= 512 ? 1 : 512 / MPPI_BLOCK)  // ... and the stash kernels (512 samples' noise fill shared memory)
+#define MPPI_MIN_BLOCKS (768 / MPPI_BLOCK)    // resident CTAs per SM the regenerate-noise tick kernels are register-budgeted for
+#define MPPI_STASH_BLOCKS (512 / MPPI_BLOCK)  // ... and the stash kernels (512 samples' noise fill shared memory)
 #define MPPI_PENALTY 1.0e10f           // mppi_race_car_obstacle.py:157
 #define MPPI_SENTINEL 1.0e18f          // padded window entries: distance^2 = 1e36, never the minimum
 #define MPPI_OUT_HDR 12                // u0 (post-shift, Q8), idx, rho, ncoll, eta, ess, p2p flag, first row of the PRE-shift nominal,
@@ -191,9 +183,6 @@ __device__ __forceinline__ void philox_eps_pair(const TickArgs &a, uint32_t k, u
     e[3] = __fmaf_rn(a.chol[1], z2, __fmul_rn(a.chol[2], z3));
 }
 
-#ifndef MPPI_KEYIDX_SMEM
-#define MPPI_KEYIDX_SMEM 1      // index addends of the first-minimum key from shared memory (hoisted LDS.128) instead of 20
-#endif                          // immediates re-materialised by MOVs in every loop iteration: 365 -> 349 instructions, +1.7 %
 // ------------------------------------------------------------------------------------------
 // shared-memory view of one robot's tick constants
 // ------------------------------------------------------------------------------------------
@@ -206,15 +195,15 @@ struct TickSmem {
     float x0[4];
     int win_start, n_win16;                // absolute index of window entry 0; padded length / 16
     float4 cb[MPPI_MAX_WINDOW / 16];       // dynamic window: bounding circle (cx, cy, r) of every 16-entry chunk
-    // static 20-entry window, expanded form (MPPI_WIN20_EXPANDED): coordinates relative to the window centre and their
-    // squared norms, d_j - |p'|^2 = ec_j - 2 p'.(ex_j, ey_j)
+    // static 20-entry window, expanded form: coordinates relative to the window centre and their squared norms,
+    // d_j - |p'|^2 = ec_j - 2 p'.(ex_j, ey_j)
     __align__(16) float ex[20];
     __align__(16) float ey[20];
     __align__(16) float ec[20];
     float c2x, c2y;                        // twice the centre
-#if MPPI_KEYIDX_SMEM
-    __align__(16) float kidx[20];          // 0..19: the index addends of the first-minimum key, read as LDS.128
-#endif
+    // 0..19: the index addends of the first-minimum key, read as LDS.128 (hoisted) instead of 20 immediates
+    // re-materialised by MOVs in every loop iteration: 365 -> 349 instructions, +1.7 %
+    __align__(16) float kidx[20];
 };
 
 // Fills the expanded-form arrays of the static window from the (already written) negated coordinates; entries past the
@@ -230,9 +219,7 @@ __device__ __forceinline__ void fill_window_expanded(TickSmem &sm, int nw, int t
         sm.ec[j] = valid ? __fmaf_rn(wy, wy, __fmul_rn(wx, wx)) : 1e30f;
     }
     if (tid == 0) { sm.c2x = 2.f * cx; sm.c2y = 2.f * cy; }
-#if MPPI_KEYIDX_SMEM
     for (int j = tid; j < 20; j += nthreads) sm.kidx[j] = (float)j;
-#endif
 }
 
 // Bounding circle of the window entries path[first .. first + n_valid) (one 16-entry chunk of the dynamic window).
@@ -275,29 +262,6 @@ __device__ __forceinline__ float2 f2_fma(float2 a, float2 b, float2 c) {
     return *reinterpret_cast<float2 *>(&rd);
 }
 
-// First-min argmin over one chunk of CH window entries (CH % 4 == 0), branch-free and almost
-// entirely on the FMA pipe:  d_j = (x-px_j)^2 + (y-py_j)^2 as FFMA2 pairs;  m = min_j d_j (FMNMX3);
-// key_j = (d_j - m) * 2^100 + j, which is exactly j where d_j == m and >= 2^76 elsewhere, so
-// min_j key_j is the FIRST index attaining the minimum (the d.index(min(d)) / np.argmin rule).
-// The window arrays hold NEGATED coordinates so the differences are plain packed adds.
-#ifndef MPPI_WP_CHUNK_ILP
-#define MPPI_WP_CHUNK_ILP 1
-#endif
-#ifndef MPPI_WP_FULL
-#define MPPI_WP_FULL 0          // 1: dynamic window without pruning (A/B: slower at every K, 70 -> 78 us at K = 1024)
-#endif
-#ifndef MPPI_WIN20_EXPANDED
-#define MPPI_WIN20_EXPANDED 1   // static window distances as ec_j - 2 p'.w'_j: 2 packed FMAs per waypoint pair instead of 4 ops (0: direct form)
-#endif
-#ifndef MPPI_ARGMIN_KEY_SEL
-#define MPPI_ARGMIN_KEY_SEL 0   // 1: first-min index by FSETP/SEL chains on the ALU pipe (A/B variant, see profiles/)
-#endif
-#ifndef MPPI_MIN_TREE
-#define MPPI_MIN_TREE 1         // tree-shaped FMNMX3 reductions in the static-window argmin (0: chains of 10; +2.9 % on B200)
-#endif
-#ifndef MPPI_ARGMIN_PACK
-#define MPPI_ARGMIN_PACK 2      // 2: all FP32 work packed (FFMA2); 1: differences scalar, rest packed; 0: all scalar
-#endif
 // Minimum of N register values as a tree of 3-input minima.  Compile-time recursion: every index is a constant after inlining, so
 // the values stay in registers (a run-time `while (n > 1)` over the array, however unrollable it looks, sent the 16-entry chunks
 // of the dynamic window through local memory: 91 registers + a stack frame instead of 126, race-car ticks 2.5x slower).
@@ -316,6 +280,11 @@ __device__ __forceinline__ float min_tree3(const float (&t)[N]) {
         return min_tree3<M>(u);
     }
 }
+// First-min argmin over one chunk of CH window entries (CH % 4 == 0), branch-free and almost
+// entirely on the FMA pipe:  d_j = (x-px_j)^2 + (y-py_j)^2 as FFMA2 pairs;  m = min_j d_j (FMNMX3);
+// key_j = (d_j - m) * 2^100 + j, which is exactly j where d_j == m and >= 2^76 elsewhere, so
+// min_j key_j is the FIRST index attaining the minimum (the d.index(min(d)) / np.argmin rule).
+// The window arrays hold NEGATED coordinates so the differences are plain packed adds.
 template <int CH>
 __device__ __forceinline__ void chunk_argmin(const float4 *nwx4, const float4 *nwy4, float x, float y,
                                              float &m_out, float &key_out) {
@@ -324,25 +293,11 @@ __device__ __forceinline__ void chunk_argmin(const float4 *nwx4, const float4 *n
 #pragma unroll
     for (int q = 0; q < CH / 4; ++q) {
         const float4 X = nwx4[q], Y = nwy4[q];
-#if MPPI_ARGMIN_PACK == 2
         const float2 dxa = f2_add(xx, make_float2(X.x, X.y)), dya = f2_add(yy, make_float2(Y.x, Y.y));
         const float2 dxb = f2_add(xx, make_float2(X.z, X.w)), dyb = f2_add(yy, make_float2(Y.z, Y.w));
         d[2 * q] = f2_fma(dya, dya, f2_mul(dxa, dxa));
         d[2 * q + 1] = f2_fma(dyb, dyb, f2_mul(dxb, dxb));
-#elif MPPI_ARGMIN_PACK == 1
-        const float2 dxa = make_float2(x + X.x, x + X.y), dya = make_float2(y + Y.x, y + Y.y);
-        const float2 dxb = make_float2(x + X.z, x + X.w), dyb = make_float2(y + Y.z, y + Y.w);
-        d[2 * q] = f2_fma(dya, dya, f2_mul(dxa, dxa));
-        d[2 * q + 1] = f2_fma(dyb, dyb, f2_mul(dxb, dxb));
-#else
-        float dx, dy;
-        dx = x + X.x; dy = y + Y.x; d[2 * q].x = fmaf(dy, dy, dx * dx);
-        dx = x + X.y; dy = y + Y.y; d[2 * q].y = fmaf(dy, dy, dx * dx);
-        dx = x + X.z; dy = y + Y.z; d[2 * q + 1].x = fmaf(dy, dy, dx * dx);
-        dx = x + X.w; dy = y + Y.w; d[2 * q + 1].y = fmaf(dy, dy, dx * dx);
-#endif
     }
-#if MPPI_MIN_TREE
     // minimum of the CH distances as a tree of 3-input minima (depth ~3) instead of a chain of CH/2 dependent ones
     float m;
     {
@@ -351,42 +306,7 @@ __device__ __forceinline__ void chunk_argmin(const float4 *nwx4, const float4 *n
         for (int i = 0; i < CH / 2; ++i) t[i] = fminf(d[i].x, d[i].y);
         m = min_tree3<CH / 2>(t);
     }
-#else
-    float m = fminf(d[0].x, d[0].y);
-#pragma unroll
-    for (int i = 1; i < CH / 2; ++i) m = fminf(fminf(m, d[i].x), d[i].y);
-#endif
-#if MPPI_ARGMIN_KEY_SEL
-    // index of the first minimum on the ALU pipe: descending select chains (the lowest index is written last), four
-    // independent chains of CH/4 entries; FSETP + SEL per entry instead of FADD2 + FFMA2 per pair on the FMA pipe
-    {
-        float k0 = (float)CH, k1 = (float)CH, k2 = (float)CH, k3 = (float)CH;
-#pragma unroll
-        for (int i = CH / 8 - 1; i >= 0; --i) {
-            const int a0 = i, a1 = i + CH / 8, a2 = i + 2 * (CH / 8), a3 = i + 3 * (CH / 8);     // float2 slots of the 4 chains
-            k0 = d[a0].y == m ? (float)(2 * a0 + 1) : k0; k0 = d[a0].x == m ? (float)(2 * a0) : k0;
-            k1 = d[a1].y == m ? (float)(2 * a1 + 1) : k1; k1 = d[a1].x == m ? (float)(2 * a1) : k1;
-            k2 = d[a2].y == m ? (float)(2 * a2 + 1) : k2; k2 = d[a2].x == m ? (float)(2 * a2) : k2;
-            k3 = d[a3].y == m ? (float)(2 * a3 + 1) : k3; k3 = d[a3].x == m ? (float)(2 * a3) : k3;
-        }
-        if (CH % 8) {                                   // CH = 20: slots 8, 9 are left over by the 4 x 2 split
-#pragma unroll
-            for (int a = CH / 2 - 1; a >= 4 * (CH / 8); --a) {
-                k3 = d[a].y == m ? (float)(2 * a + 1) : k3; k3 = d[a].x == m ? (float)(2 * a) : k3;
-            }
-            // chain 3 now covers slots 6, 7 (written earlier) and 8, 9 (written later): redo 6, 7 so the lower index wins
-#pragma unroll
-            for (int a = 4 * (CH / 8) - 1; a >= 3 * (CH / 8); --a) {
-                k3 = d[a].y == m ? (float)(2 * a + 1) : k3; k3 = d[a].x == m ? (float)(2 * a) : k3;
-            }
-        }
-        m_out = m;
-        key_out = fminf(fminf(k0, k1), fminf(k2, k3));
-        return;
-    }
-#endif
     const float2 nm = make_float2(-m, -m), huge = make_float2(1.2676506e30f, 1.2676506e30f);
-#if MPPI_MIN_TREE
     float kt[CH / 2];
 #pragma unroll
     for (int i = 0; i < CH / 2; ++i) {
@@ -395,20 +315,6 @@ __device__ __forceinline__ void chunk_argmin(const float4 *nwx4, const float4 *n
     }
     m_out = m;
     key_out = min_tree3<CH / 2>(kt);
-#else
-    float key = CUDART_INF_F;
-#pragma unroll
-    for (int i = 0; i < CH / 2; ++i) {
-#if MPPI_ARGMIN_PACK >= 1
-        const float2 k2 = f2_fma(f2_add(d[i], nm), huge, make_float2((float)(2 * i), (float)(2 * i + 1)));
-#else
-        const float2 k2 = make_float2(fmaf(d[i].x - m, 1.2676506e30f, (float)(2 * i)), fmaf(d[i].y - m, 1.2676506e30f, (float)(2 * i + 1)));
-#endif
-        key = fminf(fminf(key, k2.x), k2.y);
-    }
-    m_out = m;
-    key_out = key;
-#endif
 }
 
 // A8: first-min argmin of squared xy distance over the window
@@ -418,7 +324,6 @@ __device__ __forceinline__ int nearest_wp(const TickSmem &sm, float x, float y) 
     const float4 *nwx4 = reinterpret_cast<const float4 *>(sm.wx);
     const float4 *nwy4 = reinterpret_cast<const float4 *>(sm.wy);
     if (WIN == 20) {
-#if MPPI_WIN20_EXPANDED
         // squared distances up to the common term |p'|^2, in coordinates relative to the window centre (|w'| <= ~1 m, so
         // the cancellation costs no more than the FP32 rounding of the absolute path coordinates does in the direct form)
         const float ax = fmaf(-2.f, x, sm.c2x), ay = fmaf(-2.f, y, sm.c2y);
@@ -432,7 +337,6 @@ __device__ __forceinline__ int nearest_wp(const TickSmem &sm, float x, float y) 
             d[2 * q] = f2_fma(make_float2(Y.x, Y.y), ayy, f2_fma(make_float2(X.x, X.y), axx, make_float2(C.x, C.y)));
             d[2 * q + 1] = f2_fma(make_float2(Y.z, Y.w), ayy, f2_fma(make_float2(X.z, X.w), axx, make_float2(C.z, C.w)));
         }
-#if MPPI_MIN_TREE
         // the two 20-input minima as TREES of 3-input FMNMX3 (depth 3) instead of chains of 10 dependent ones: the
         // horizon recurrence leaves a sample no other work to hide ~80 cycles of chain latency per step behind
         const float m = fminf(fminf(fminf(fminf(d[0].x, d[0].y), d[1].x), fminf(fminf(d[1].y, d[2].x), d[2].y)),
@@ -453,66 +357,12 @@ __device__ __forceinline__ int nearest_wp(const TickSmem &sm, float x, float y) 
                                       fminf(fminf(fminf(fminf(kk[6].x, kk[6].y), kk[7].x), fminf(fminf(kk[7].y, kk[8].x), kk[8].y)),
                                             fminf(kk[9].x, kk[9].y))));
         return __float2int_rn(key);
-#else
-        float m = fminf(d[0].x, d[0].y);
-#pragma unroll
-        for (int i = 1; i < 10; ++i) m = fminf(fminf(m, d[i].x), d[i].y);
-        const float2 nm = make_float2(-m, -m), huge = make_float2(1.2676506e30f, 1.2676506e30f);
-        float key = CUDART_INF_F;
-#if MPPI_KEYIDX_SMEM
-        const float4 *ki4 = reinterpret_cast<const float4 *>(sm.kidx);
-#pragma unroll
-        for (int i = 0; i < 10; i += 2) {
-            const float4 ki = ki4[i >> 1];
-            const float2 ka = f2_fma(f2_add(d[i], nm), huge, make_float2(ki.x, ki.y));
-            const float2 kb = f2_fma(f2_add(d[i + 1], nm), huge, make_float2(ki.z, ki.w));
-            key = fminf(fminf(key, ka.x), ka.y);
-            key = fminf(fminf(key, kb.x), kb.y);
-        }
-#else
-#pragma unroll
-        for (int i = 0; i < 10; ++i) {
-            const float2 k2 = f2_fma(f2_add(d[i], nm), huge, make_float2((float)(2 * i), (float)(2 * i + 1)));
-            key = fminf(fminf(key, k2.x), k2.y);
-        }
-#endif
-        return __float2int_rn(key);
-#endif
-#else
-        float m, key;
-        chunk_argmin<20>(nwx4, nwy4, x, y, m, key);
-        return __float2int_rn(key);
-#endif
     }
     // dynamic window: chunks of 16 entries (the window is padded with sentinels to a multiple of 16)
     float bm = CUDART_INF_F, sbm = CUDART_INF_F;      // best squared distance so far and its square root
     int bj = 0;
     const int nch = sm.n_win16;
     int c = 0;
-#if MPPI_WP_FULL
-    // A/B variant: every chunk evaluated, no pruning, four independent chunk chains per trip (block-uniform trip count)
-    for (; c + 3 < nch; c += 4) {
-        float m0, k0, m1, k1, m2, k2, m3, k3;
-        chunk_argmin<16>(nwx4 + 4 * c, nwy4 + 4 * c, x, y, m0, k0);
-        chunk_argmin<16>(nwx4 + 4 * c + 4, nwy4 + 4 * c + 4, x, y, m1, k1);
-        chunk_argmin<16>(nwx4 + 4 * c + 8, nwy4 + 4 * c + 8, x, y, m2, k2);
-        chunk_argmin<16>(nwx4 + 4 * c + 12, nwy4 + 4 * c + 12, x, y, m3, k3);
-        const bool s01 = m1 < m0, s23 = m3 < m2;
-        const float ma = s01 ? m1 : m0, mb = s23 ? m3 : m2;
-        const float ka = s01 ? k1 + 16.f : k0, kb = s23 ? k3 + 48.f : k2 + 32.f;
-        const bool sb = mb < ma;
-        const float m = sb ? mb : ma;
-        const int j = 16 * c + __float2int_rn(sb ? kb : ka);
-        if (m < bm) { bm = m; bj = j; }
-    }
-    for (; c < nch; ++c) {
-        float m, key;
-        chunk_argmin<16>(nwx4 + 4 * c, nwy4 + 4 * c, x, y, m, key);
-        if (m < bm) { bm = m; bj = 16 * c + __float2int_rn(key); }
-    }
-    (void)sbm;
-    return bj;
-#endif
     // |z - p| >= |z - centre| - r for every point p of a chunk: if that exceeds the best distance (with a 1e-4 relative
     // margin, three orders above FP32 rounding) no point of the chunk can be the minimum or tie with it
     auto far = [&](int ch) {
@@ -520,7 +370,6 @@ __device__ __forceinline__ int nearest_wp(const TickSmem &sm, float x, float y) 
         const float ex = x - cb.x, ey = y - cb.y, R = sbm + cb.z;
         return fmaf(ey, ey, ex * ex) > R * R * 1.0002f;
     };
-#if MPPI_WP_CHUNK_ILP
     // two chunks per trip: their (independent) distance / min / key chains overlap, which is what a latency-bound
     // small-K tick needs; the earlier chunk still wins ties
     for (; c + 1 < nch; c += 2) {
@@ -533,7 +382,6 @@ __device__ __forceinline__ int nearest_wp(const TickSmem &sm, float x, float y) 
         const int j = second ? 16 * c + 16 + __float2int_rn(k1) : 16 * c + __float2int_rn(k0);
         if (m < bm) { bm = m; bj = j; sbm = sqrtf(m); }
     }
-#endif
     for (; c < nch; ++c) {
         if (far(c)) continue;
         float m, key;
@@ -763,13 +611,12 @@ __device__ __forceinline__ void dyn_step_tan(const TickArgs &a, float z[4], floa
 
 __device__ __forceinline__ float clampf(float v, float lim) { return fminf(fmaxf(v, -lim), lim); }
 
-// The rollouts of SPT samples of one thread (frozen window), advanced in LOCKSTEP: every stage is written as a loop over the
-// thread's samples inside one basic block, so the instruction scheduler interleaves SPT independent dependency chains
-// (the horizon recurrence makes a single chain latency-bound: ~220 cycles of dependent latency per step).  Sample s of
-// the thread is chunk slot `slot0 + s * MPPI_BLOCK`.  Returns per sample the smooth cost and the number of collided
-// evaluations separately so 1e10 * n never swallows the tracking cost (SURVEY.md section 7).
+// The rollout of the thread's sample (frozen window; the tick kernel passes SPT = 1: see tick_body for why its values are
+// one-element arrays walked by unrolled loops).  `stash`, if not null, is the sample's column of the chunk's noise stash.
+// Returns the smooth cost and the number of collided evaluations separately so 1e10 * n never swallows the tracking cost
+// (SURVEY.md section 7).
 //
-// The loop is also software-pipelined by hand: the noise of the NEXT timestep pair (Philox + Box-Muller:
+// The loop is software-pipelined by hand: the noise of the NEXT timestep pair (Philox + Box-Muller:
 // integer/ALU + MUFU work) is generated in the same straight-line block as the two dynamics/cost
 // steps of the CURRENT pair (FMA-pipe work), so the ALU, MUFU and FMA pipes are busy at the same time.
 template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int SPT, class SC>
@@ -802,7 +649,7 @@ __device__ __forceinline__ void rollout_samples(const TickArgs &a, const SC &sc,
     };
     auto step = [&](int s, int t, float e0, float e1) {
         MPPI_DCHECK(t >= 0 && t < T);
-        if (stash) stash[t * MPPI_CHUNK + s * MPPI_BLOCK] = make_float2(e0, e1);
+        if (stash) stash[t * MPPI_BLOCK + s * MPPI_BLOCK] = make_float2(e0, e1);
         const float2 u = sm.U[t];
         v0[s] = clampf(exploit[s] ? __fadd_rn(u.x, e0) : e0, a.umax0);                   // A4, A5
         v1[s] = clampf(exploit[s] ? __fadd_rn(u.y, e1) : e1, a.umax1);

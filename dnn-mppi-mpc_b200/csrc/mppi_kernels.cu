@@ -50,14 +50,11 @@ struct MergeSmem {
 // thread owns one float2 COLUMN PAIR of the partial layout and streams every G-th partial with 8 independent
 // coalesced 8-byte loads in flight; the G group sums meet in shared memory.  `sc` is scratch lent by the caller:
 // MPPI_MERGE_SCRATCH floats (the first MPPI_MERGE_TILE hold scale factors, the rest the group sums).
-#ifndef MPPI_MERGE_TWO_LEVEL
-#define MPPI_MERGE_TWO_LEVEL 1          // 0: one B-way merge by the last CTA (A/B)
-#endif
 #define MPPI_MERGE_TWO_LEVEL_MIN 64     // smaller grids keep the single merge (one L2 round trip either way)
 #define MPPI_MERGE_TILE 1000
 #define MPPI_MERGE_GROUPS 4
 #define MPPI_MERGE_SCRATCH (MPPI_MERGE_TILE + MPPI_MERGE_GROUPS * MPPI_NF_MAX)      // 2040 floats <= the 8 KB warpN region
-static_assert(4 * MPPI_BLOCK <= MPPI_MERGE_SCRATCH || MPPI_BLOCK > 256, "merge fast path: group sums must fit the scratch");
+static_assert(4 * MPPI_BLOCK <= MPPI_MERGE_SCRATCH, "merge fast path: group sums must fit the scratch");
 __device__ void merge_partials(const TickArgs &a, const float *parts, int P, MergeSmem &ms, float *sc, int stride = 0) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int NF = MPPI_NF(a.T);
@@ -298,7 +295,7 @@ struct RunSmem {
     float s;
     float eta, e2;
     float N[2 * MPPI_MAX_T];   // running sum of w * eps, relative to (n, s)
-    float w[MPPI_CHUNK];       // stash mode: this chunk's weights
+    float w[MPPI_BLOCK];       // stash mode: this chunk's weights
     float warp_eta[MPPI_WARPS], warp_e2[MPPI_WARPS];
     float red_s[MPPI_WARPS];
     int red_n[MPPI_WARPS];
@@ -307,7 +304,7 @@ struct RunSmem {
 };
 
 // Dynamic shared memory of the tick kernel:
-//   STASH = true : float2 eps[T][MPPI_CHUNK] -- the noise of the chunk being rolled out, written in
+//   STASH = true : float2 eps[T][MPPI_BLOCK] -- the noise of the chunk being rolled out, written in
 //                  pass 1 and consumed by the weighted column sums, so Philox + Box-Muller run once.
 //   STASH = false: float warpN[MPPI_WARPS][2*MPPI_MAX_T] -- per-warp partial sums of the
 //                  regenerate-the-noise path (injected noise, K2 alone, horizons too long to stash).
@@ -397,7 +394,7 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
         int nw = n_path - s_new; nw = nw < a.window ? nw : a.window;
         MPPI_DCHECK(WIN < 0 || (s_new >= 0 && s_new < n_path && nw >= 1));
         // static-window kernels read exactly 20 entries, dynamic ones whole chunks of 16
-        const int fill = (WIN < 0) ? 0 : (WIN == 20) ? 20 : MPPI_WP_FULL ? ((nw + 63) & ~63) : ((nw + 15) & ~15);
+        const int fill = (WIN < 0) ? 0 : (WIN == 20) ? 20 : ((nw + 15) & ~15);
         for (int j = tid; j < fill; j += MPPI_BLOCK) {
             if (j < nw) {
                 const float4 p = rpath[s_new + j];
@@ -407,9 +404,7 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
             }
         }
         if (tid == 0) { sm.win_start = s_new; sm.n_win16 = fill >> 4; }
-#if MPPI_WIN20_EXPANDED
         if (WIN == 20) { __syncthreads(); fill_window_expanded(sm, nw, tid, MPPI_BLOCK); }
-#endif
         if (WIN == 0) {
             __syncthreads();                            // the window is staged: bound every 16-entry chunk from shared memory
             for (int c = tid; c < (fill >> 4); c += MPPI_BLOCK) sm.cb[c] = chunk_bound(sm.wx, sm.wy, 16 * c, min(16, nw - 16 * c));
@@ -425,16 +420,18 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
     }
     __syncthreads();
 
-    // ---- this block's contiguous sample range (balanced over the grid), walked in chunks of MPPI_CHUNK samples:
-    // thread tid owns chunk slots tid, tid + MPPI_BLOCK, ... (MPPI_SPT of them, rolled out in lockstep)
-    constexpr int SPT = MPPI_SPT;
+    // ---- this block's contiguous sample range (balanced over the grid), walked in chunks of MPPI_BLOCK samples:
+    // thread tid owns chunk slot tid.  Its sample's values are one-element arrays walked by unrolled loops (SPT = 1, the
+    // shape of rollout_samples): the compiler keeps them in memory until the loops are unrolled, and plain scalars, promoted
+    // to registers earlier, compile 104 of the 134 tick kernels to differently scheduled machine code
+    constexpr int SPT = 1;
     const int k_begin = (int)((long long)K * b / B);
     const int k_end = (a.flags & F_IDX_ONLY) ? k_begin : (int)((long long)K * (b + 1) / B);
-    MPPI_DCHECK(k_begin >= 0 && k_end <= K && (!STASH || (size_t)T * MPPI_CHUNK * sizeof(float2) <= 232448));
+    MPPI_DCHECK(k_begin >= 0 && k_end <= K && (!STASH || (size_t)T * MPPI_BLOCK * sizeof(float2) <= 232448));
     float *Srow = a.S ? a.S + (size_t)robot * K : nullptr;
     // (time-parallel rollout: chunks of MPPI_TPAR_SLOTS samples on chunk slots 0 .. MPPI_TPAR_SLOTS - 1, the other slots idle)
-    static_assert(STASH != 2 || (SPT == 1 && SUM && !INJ), "time-parallel rollout: one sample per thread, sum mode, Philox noise");
-    constexpr int CHUNK_STRIDE = STASH == 2 ? MPPI_TPAR_SLOTS : MPPI_CHUNK;
+    static_assert(STASH != 2 || (SUM && !INJ), "time-parallel rollout: sum mode, Philox noise");
+    constexpr int CHUNK_STRIDE = STASH == 2 ? MPPI_TPAR_SLOTS : MPPI_BLOCK;
     for (int base = k_begin; base < k_end; base += CHUNK_STRIDE) {
         int k[SPT], ksafe[SPT], ncoll[SPT];
         bool active[SPT], exploit[SPT];
@@ -475,7 +472,7 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
         if (STASH == 1 && !active[0]) {             // tail chunk: a thread that rolled nothing out must not leave garbage (0 * NaN)
             for (int t = 0; t < T; ++t)
 #pragma unroll
-                for (int s = 0; s < SPT; ++s) stash[t * MPPI_CHUNK + s * MPPI_BLOCK + tid] = make_float2(0.f, 0.f);
+                for (int s = 0; s < SPT; ++s) stash[t * MPPI_BLOCK + s * MPPI_BLOCK + tid] = make_float2(0.f, 0.f);
         }
 
         // chunk minimum -> new running minimum
@@ -507,7 +504,7 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
 #pragma unroll
             for (int s = 0; s < SPT; ++s) run.w[tid + s * MPPI_BLOCK] = w[s];
             __syncthreads();
-            constexpr int SCOLS = STASH == 2 ? MPPI_TPAR_SLOTS : MPPI_CHUNK;       // columns of a stash row
+            constexpr int SCOLS = STASH == 2 ? MPPI_TPAR_SLOTS : MPPI_BLOCK;       // columns of a stash row
             float wr[SCOLS / 32];
 #pragma unroll
             for (int i = 0; i < SCOLS / 32; ++i) wr[i] = run.w[lane + 32 * i];
@@ -607,12 +604,12 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
             if (tid == 0) { mine[0] = __int_as_float(run.n); mine[1] = run.s; mine[2] = run.eta; mine[3] = run.e2; }
         }
     }
-    // TWO-LEVEL merge (MPPI_MERGE_TWO_LEVEL, grids of >= MPPI_MERGE_TWO_LEVEL_MIN CTAs): consecutive CTAs form groups of
+    // TWO-LEVEL merge (grids of >= MPPI_MERGE_TWO_LEVEL_MIN CTAs): consecutive CTAs form groups of
     // MPPI_MERGE_GROUP_CTAS; the last CTA of a group to finish merges that group's partials into one group partial -- while the other
     // groups are still rolling out -- and the last GROUP merges the ~B/16 group partials and finalizes.  What stays on the tick's
     // critical path is one 16-way and one B/16-way merge (one L2 round trip each) instead of one B-way merge by a single CTA
     // (8.6 us of a 412 us tick at B = 296).  Same log-sum-exp rule at both levels; the grouping is fixed, so results stay deterministic.
-    const bool two_level = MPPI_MERGE_TWO_LEVEL && (a.flags & F_UPDATE) && B >= MPPI_MERGE_TWO_LEVEL_MIN && a.part2 != nullptr;
+    const bool two_level = (a.flags & F_UPDATE) && B >= MPPI_MERGE_TWO_LEVEL_MIN && a.part2 != nullptr;
     int n_merge = B;                                     // partials the finalizing CTA merges, and where they are
     const float *merge_src = parts;
     if (B > 1) {
@@ -1013,7 +1010,7 @@ size_t mppi_tick_dyn_smem(int T, int stash) {
     // regenerate path: per-warp column sums (8 KB), also large enough for the exchange's gathered triples
     const size_t small = std::max(sizeof(float) * MPPI_WARPS * 2 * MPPI_MAX_T, sizeof(float) * MPPI_MAX_PEERS * MPPI_NF_MAX);
     if (stash == 2) return std::max((sizeof(float2) + sizeof(float4)) * MPPI_TPAR_SLOTS * (size_t)T, small);   // noise + the states of every step
-    return stash ? std::max(sizeof(float2) * (size_t)T * MPPI_CHUNK, small) : small;
+    return stash ? std::max(sizeof(float2) * (size_t)T * MPPI_BLOCK, small) : small;
 }
 
 // Opt-in of a tick kernel to `dyn` bytes of dynamic shared memory on the current device.  The attribute belongs to the

@@ -6,8 +6,8 @@
 // sm_100a mapping (one persistent CTA per SM, clusters of two, each CTA owning 128-sample tiles for the whole horizon):
 //   * the input layer has NO activation (simple_mlp.py:19), so Linear(3,512) and the first hidden
 //     Linear(512,512) are folded on the host into one 3->512 map (W01 = W1 W0, b01 = W1 b0 + b1).  The compute warps evaluate it in
-//     FP32 on the CUDA cores (three-input kernels) or read it back from a split-fp16 tcgen05 MMA (five-input ping-pong kernels,
-//     MPPI_MLP_L1_TC), apply tanh (MUFU), round ONCE to the half-precision operand type and store the A operand straight into
+//     FP32 on the CUDA cores (three-input kernels) or read it back from a split-fp16 tcgen05 MMA (five-input ping-pong kernels),
+//     apply tanh (MUFU), round ONCE to the half-precision operand type and store the A operand straight into
 //     TENSOR MEMORY (tcgen05.st, 256 columns): the activations never touch shared memory, which leaves it to the weight stream;
 //   * the remaining 512x512 layer is the GEMM: D[128x512] = A[128x512] (TMEM) x W2^T, issued by ONE thread as tcgen05.mma kind::f16
 //     with the A operand in TMEM (N=128, K=16), W2 streamed from L2 by TMA (cp.async.bulk.tensor, 128B swizzle) through an mbarrier
@@ -36,7 +36,6 @@
 // Variants that were built, measured and rejected (mma.sync layer 1, register-tiled 16x256b layer 1 / epilogue, early layer 1,
 // K-interleaved last quarters, output-layer records through the constant bank) are described in DESIGN.md 3.4 with the commits that hold them.
 #include <cuda.h>
-#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
@@ -50,29 +49,16 @@
 
 namespace {
 
-// Operand type of the hidden GEMM(s).  fp16 (default): the A operand is a tanh output in [-1, 1] and trained weights are
-// O(1), so half precision's 11-bit significand applies with no range problem -- 8x smaller rounding error than bf16 at the
-// same tensor-core rate (weights beyond +-65504 are refused on the host).  -DMPPI_MLP_F16=0 restores bf16 (A/B measurements).
-#ifndef MPPI_MLP_F16
-#define MPPI_MLP_F16 1
-#endif
-#if MPPI_MLP_F16
+// Operand type of the hidden GEMM(s): fp16.  The A operand is a tanh output in [-1, 1] and trained weights are O(1), so half
+// precision's 11-bit significand applies with no range problem -- 8x smaller rounding error than bf16 at the same tensor-core
+// rate (weights beyond +-65504 are refused on the host).
 typedef __half mlp_op_t;
-#define MLP_TMAP_DTYPE CU_TENSOR_MAP_DATA_TYPE_FLOAT16
-#define MLP_UMMA_FMT 0u
-#else
-typedef __nv_bfloat16 mlp_op_t;
-#define MLP_TMAP_DTYPE CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-#define MLP_UMMA_FMT 1u
-#endif
 
-// Wrong-result TIMING probes (never shipped; profiles/): 1 = epilogue without the output-layer LDS + FMAs, 2 = layer 1 without its
-// LDS + FMAs, 4 = no MUFU (tanh replaced by the identity); bits may be combined
+// -DMPPI_MLP_PROBE=32 (never shipped, profiles/; 32 is its only bit): per-wait stall accounting (clock64 around every barrier wait of
+// the MMA issuer and of compute warp 0, printed by CTA 0)
 #ifndef MPPI_MLP_PROBE
 #define MPPI_MLP_PROBE 0
 #endif
-
-// bit 32: per-wait stall accounting (clock64 around every barrier wait of the MMA issuer and of compute warp 0, printed by CTA 0)
 #if MPPI_MLP_PROBE & 32
 #define MLP_PROBE_DECL() long long pr_c = 0; const long long pr_begin = clock64(); unsigned long long *pr_t = reinterpret_cast<unsigned long long *>(sm.cb) + (warp == 1 ? 0 : 16);   /* static window: cb is unused */ (void)pr_c; \
     if ((threadIdx.x & 31) == 0 && (threadIdx.x >> 5) <= 2) for (int i_ = 0; i_ < 16; ++i_) pr_t[i_] = 0
@@ -90,11 +76,11 @@ typedef __nv_bfloat16 mlp_op_t;
 
 constexpr int HID = 512;
 constexpr int TILE_M = 128;
-constexpr int KCH = 64;                   // K elements per 128-byte swizzle span (bf16)
+constexpr int KCH = 64;                   // K elements per 128-byte swizzle span (fp16)
 
 constexpr int N_MMA = 128;                // N per tcgen05.mma = one accumulator quarter
 constexpr int N_QUARTERS = HID / N_MMA;
-// -DMPPI_MLP_L1_TC=1 (ping-pong kernels): layer 1 ON THE tcgen05 TENSOR CORE.  The folded first layer needs FP32 accuracy, so inputs and
+// Five-input ping-pong kernels: layer 1 ON THE tcgen05 TENSOR CORE.  The folded first layer needs FP32 accuracy, so inputs and
 // weights are split into fp16 pieces, v = hi + lo, x.w ~= x_hi w_hi + x_hi w_lo + x_lo w_hi (three K slots per input + two for the bias: K = 16 | 32).  Its A
 // operand (128 sample rows x K) and B operand (512 hidden units x K) live in shared memory in the same K-major 128B-swizzled layout as
 // the weight boxes (rows padded to 128 B), and each 128-column part is ONE (two for 5 inputs) M128 x N128 x K16 MMA in the SS form.
@@ -103,18 +89,9 @@ constexpr int N_QUARTERS = HID / N_MMA;
 // in order, so the part's commit also proves that quarter 3 is done with A part p), the compute warps read it back (tcgen05.ld), apply
 // tanh, round once to fp16 and store it into A part p.  That replaces a broadcast LDS.128 + 3 (5) FMAs per (row, column) -- the work the
 // compute warps' chain is made of (profiles/r2_mlp_stall_accounting.txt) -- by one tcgen05.ld of 32 columns per thread and part.
-#ifndef MPPI_MLP_L1_TC
-#define MPPI_MLP_L1_TC 1
-#endif
-#ifndef MPPI_MLP_KCH_PER_STAGE
-#define MPPI_MLP_KCH_PER_STAGE 4
-#endif
-#ifndef MPPI_MLP_B_STAGES
-#define MPPI_MLP_B_STAGES 3
-#endif
-constexpr int KCH_PER_STAGE = MPPI_MLP_KCH_PER_STAGE;   // K chunks (TMA boxes) per ring stage: one barrier wait + one commit per 16 MMAs,
+constexpr int KCH_PER_STAGE = 4;          // K chunks (TMA boxes) per ring stage: one barrier wait + one commit per 16 MMAs,
                                           // otherwise the single issuing thread (try_wait ~90 cycles) paces the tensor core
-constexpr int B_STAGES = MPPI_MLP_B_STAGES;
+constexpr int B_STAGES = 3;
 constexpr int B_BOX_BYTES = N_MMA * KCH * 2;       // 16 KB per TMA box
 constexpr int B_TILE_BYTES = KCH_PER_STAGE * B_BOX_BYTES;   // 64 KB per stage
 constexpr int RING_BYTES = 12 * B_BOX_BYTES;        // the 1024-aligned operand region at the start of dynamic shared memory (192 KB)
@@ -122,14 +99,11 @@ constexpr int A2_BYTES = TILE_M * HID * 2;          // NG = 2: second GEMM's A o
 constexpr int B2_STAGES = (RING_BYTES - A2_BYTES) / B_BOX_BYTES;   // NG = 2: one-box stages in what is left (4)
 static_assert(B2_STAGES >= 2, "NG = 2 ring");
 static_assert(B_STAGES * B_TILE_BYTES <= RING_BYTES && (HID / KCH) % KCH_PER_STAGE == 0 && KCH_PER_STAGE % 2 == 0, "NG = 1 ring");
-// -DMPPI_MLP_CG2=1 (ping-pong kernels): the hidden GEMM as PAIR MMAs, tcgen05.mma.cta_group::2 with M = 256 -- the two CTAs of a cluster
+// The other ping-pong kernels: the hidden GEMM as PAIR MMAs, tcgen05.mma.cta_group::2 with M = 256 -- the two CTAs of a cluster
 // (which already walk the weight stream in lockstep) become one MMA unit: rank 0 issues for both, each CTA keeps its own 128 rows of A and
 // D in its tensor memory and only HALF of every W2 box (64 of the 128 rows) in its shared memory.  Per SM that halves the TMA writes and the
 // B-operand reads (2 x 256 KB instead of 2 x 512 KB per tile-step), which share the shared-memory bandwidth with the compute warps'
 // broadcast LDS.128 (profiles/r2_mlp_stall_accounting.txt).  The ring keeps its 192 KB: six 32 KB stages instead of three 64 KB ones.
-#ifndef MPPI_MLP_CG2
-#define MPPI_MLP_CG2 1
-#endif
 constexpr int CG2_BOX_BYTES = B_BOX_BYTES / 2;                    // 64 W2 rows x 64 K halves
 constexpr int RING_SLOTS = 12;                                    // barrier pairs: enough for every ring geometry (asserted in the kernel)
 constexpr int L1_KS_MAX = 32;                       // tcgen05 layer 1: K slots (halves) per row, 16 (3 inputs) or 32 (5 inputs)
@@ -138,20 +112,17 @@ constexpr int L1_KS_MAX = 32;                       // tcgen05 layer 1: K slots 
 constexpr int B1TC_KB_BYTES = HID * 32, A1TC_KB_BYTES = TILE_M * 32;     // one K block of B (16 KB: 4 parts of 4 KB) / of A (4 KB)
 constexpr int B1TC_BYTES = 2 * B1TC_KB_BYTES;       // B operand, 512 hidden units (32 KB)
 constexpr int A1TC_BYTES = 2 * A1TC_KB_BYTES;       // A operand, 128 sample rows (8 KB)
-// which ping-pong kernels use what (shared by the kernel and the launcher): MPPI_MLP_L1_TC = 1 -> the five-input kernels (where it wins:
-// their CUDA-core layer 1 costs two LDS + five FMAs per column), 2 -> all of them; pair MMAs for the others (the tcgen05 layer 1 issues
+// which ping-pong kernels use what (shared by the kernel and the launcher): the tcgen05 layer 1 for the five-input kernels (where it
+// wins: their CUDA-core layer 1 costs two LDS + five FMAs per column); pair MMAs for the others (the tcgen05 layer 1 issues
 // cta_group::1, and one kernel may use only one group size)
-__host__ __device__ constexpr bool mlp_use_l1tc(int nin, bool pp, int ng) { return pp && ng == 1 && (MPPI_MLP_L1_TC == 2 || (MPPI_MLP_L1_TC == 1 && nin == 5)); }
-__host__ __device__ constexpr bool mlp_use_cg2(int nin, bool pp, int ng) { return MPPI_MLP_CG2 && pp && ng == 1 && !mlp_use_l1tc(nin, pp, ng); }
-constexpr int TMEM_A_COL = 0;             // A operand: 512 bf16 per row = 256 packed 32-bit columns
+__host__ __device__ constexpr bool mlp_use_l1tc(int nin, bool pp, int ng) { return pp && ng == 1 && nin == 5; }
+__host__ __device__ constexpr bool mlp_use_cg2(int nin, bool pp, int ng) { return pp && ng == 1 && !mlp_use_l1tc(nin, pp, ng); }
+constexpr int TMEM_A_COL = 0;             // A operand: 512 fp16 per row = 256 packed 32-bit columns
 constexpr int TMEM_D_COL = 256;           // two accumulator buffers of 128 FP32 columns
 constexpr int N_GROUPS = 4;                // compute-warp groups: group g owns accumulator quarter g (128 columns)
 constexpr int N_COMPUTE = 128 * N_GROUPS;  // 16 compute warps: 4 per TMEM lane quarter
 constexpr int MLP_THREADS = 64 + N_COMPUTE;
-#ifndef MPPI_MLP_WARP_ARRIVE
-#define MPPI_MLP_WARP_ARRIVE 1
-#endif
-constexpr int N_ARRIVE = MPPI_MLP_WARP_ARRIVE ? N_COMPUTE / 32 : N_COMPUTE;   // arrivals per compute-warp hand-off (see compute_arrive)
+constexpr int N_ARRIVE = N_COMPUTE / 32;   // arrivals per compute-warp hand-off (see compute_arrive)
 
 
 struct MlpSmem {                          // after the 1024-aligned A / B regions
@@ -196,21 +167,14 @@ __device__ __forceinline__ void mbar_wait(unsigned long long *bar, uint32_t pari
         "WAIT_DONE:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
 
-// Compute warps signal "my part of the operand is written" / "my part of the accumulator is read".  One arrival per WARP (default):
+// Compute warps signal "my part of the operand is written" / "my part of the accumulator is read".  One arrival per WARP:
 // every lane has waited for its tcgen05.st / tcgen05.ld and fenced, __syncwarp orders that before lane 0's releasing arrive -- 16
-// shared-memory barrier operations per hand-off instead of 512.  -DMPPI_MLP_WARP_ARRIVE=0: one arrival per thread (A/B).
-#ifndef MPPI_MLP_WARP_ARRIVE
-#define MPPI_MLP_WARP_ARRIVE 1
-#endif
+// shared-memory barrier operations per hand-off instead of 512.
 __device__ __forceinline__ void mbar_arrive_rank0(unsigned long long *bar);
 template <bool TO_RANK0 = false>                               // pair MMAs: both CTAs report to rank 0's barrier
 __device__ __forceinline__ void compute_arrive(unsigned long long *bar) {
-#if MPPI_MLP_WARP_ARRIVE
     __syncwarp();
     if ((threadIdx.x & 31) == 0) { if constexpr (TO_RANK0) mbar_arrive_rank0(bar); else mbar_arrive(bar); }
-#else
-    if constexpr (TO_RANK0) mbar_arrive_rank0(bar); else mbar_arrive(bar);
-#endif
 }
 
 // non-blocking: has the phase with this parity completed?  (warp-uniform: lane 0's answer)
@@ -266,11 +230,11 @@ __device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t saddr) {
     return d;
 }
 
-// kind::f16 instruction descriptor: F16 x F16 (or BF16 x BF16) -> F32, K-major A and B, M=128, N=128
-constexpr uint32_t UMMA_IDESC = (1u << 4) | (MLP_UMMA_FMT << 7) | (MLP_UMMA_FMT << 10) | ((uint32_t)(N_MMA >> 3) << 17) | ((uint32_t)(TILE_M >> 4) << 24);
+// kind::f16 instruction descriptor: F16 x F16 -> F32 (A and B format fields 0), K-major A and B, M=128, N=128
+constexpr uint32_t UMMA_IDESC = (1u << 4) | ((uint32_t)(N_MMA >> 3) << 17) | ((uint32_t)(TILE_M >> 4) << 24);
 
-// A operand in tensor memory (128 lanes x 8 packed bf16x2 columns per K=16 step), B in shared memory
-__device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t accumulate) {
+// A operand in tensor memory (128 lanes x 8 packed f16x2 columns per K=16 step), B in shared memory
+__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
@@ -278,7 +242,7 @@ __device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, u
         ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(UMMA_IDESC), "r"(accumulate), "r"(0u) : "memory");
 }
 // both operands in shared memory (NG = 2, second GEMM)
-__device__ __forceinline__ void umma_bf16_ss(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
+__device__ __forceinline__ void umma_f16_ss(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
@@ -286,7 +250,7 @@ __device__ __forceinline__ void umma_bf16_ss(uint32_t d_tmem, uint64_t a_desc, u
         ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(UMMA_IDESC), "r"(accumulate), "r"(0u) : "memory");
 }
 // ---- pair MMAs (cta_group::2): rank 0 issues M = 256 MMAs over both CTAs' tensor memory and shared memory ----
-constexpr uint32_t UMMA_IDESC_2SM = (1u << 4) | (MLP_UMMA_FMT << 7) | (MLP_UMMA_FMT << 10) | ((uint32_t)(N_MMA >> 3) << 17) | ((uint32_t)((2 * TILE_M) >> 4) << 24);
+constexpr uint32_t UMMA_IDESC_2SM = (1u << 4) | ((uint32_t)(N_MMA >> 3) << 17) | ((uint32_t)((2 * TILE_M) >> 4) << 24);
 __device__ __forceinline__ void umma_f16_ts_2sm(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
@@ -337,35 +301,20 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
         : "r"(taddr));
 }
 __device__ __forceinline__ float tanh_approx(float x) {
-#if MPPI_MLP_PROBE & 4
-    return x * 0.5f;
-#else
     float y;
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
-#endif
 }
 // two FP32 values -> packed half-precision operand pair (lo in the low half)
 __device__ __forceinline__ uint32_t pack_op2(float lo, float hi) {
     uint32_t p;
-#if MPPI_MLP_F16
     asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(p) : "f"(hi), "f"(lo));
-#else
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(p) : "f"(hi), "f"(lo));
-#endif
     return p;
 }
-// tanh of two FP32 pre-activations -> packed operand pair.  fp16: FP32 MUFU.TANH on the unrounded pre-activation, ONE
-// rounding at the end (tanh.approx.bf16x2 rounds the input first and is two MUFU ops anyway, so this costs the same)
+// tanh of two FP32 pre-activations -> packed operand pair: FP32 MUFU.TANH on the unrounded pre-activation, ONE rounding at
+// the end
 __device__ __forceinline__ uint32_t tanh_op2(float lo, float hi) {
-#if MPPI_MLP_F16
     return pack_op2(tanh_approx(lo), tanh_approx(hi));
-#else
-    uint32_t p, y;
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(p) : "f"(hi), "f"(lo));
-    asm("tanh.approx.bf16x2 %0, %1;" : "=r"(y) : "r"(p));
-    return y;
-#endif
 }
 // v = hi + lo in half precision, packed (hi in the low half)
 __device__ __forceinline__ void split_half(float v, unsigned short &hi, unsigned short &lo) {
@@ -568,9 +517,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
             }
         }
         if (tid == 0) { sm.win_start = s_new; sm.n_win16 = fill >> 4; }
-#if MPPI_WIN20_EXPANDED
         if (a.window == 20) { __syncthreads(); fill_window_expanded(sm, nw, tid, MLP_THREADS); }
-#endif
         if (a.window != 20) {
             __syncthreads();
             for (int c = tid; c < (fill >> 4); c += MLP_THREADS) sm.cb[c] = chunk_bound(sm.wx, sm.wy, 16 * c, min(16, nw - 16 * c));
@@ -667,8 +614,8 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                             if (leader) {
 #pragma unroll
                                 for (int k = 0; k < KCH / 16; ++k) {
-                                    if (g == 0) umma_bf16_ts(d_tmem, a_col0 + k * 8, b_desc0 + (uint64_t)((k * 32) >> 4), (kc | k) ? 1u : 0u);
-                                    else umma_bf16_ss(d_tmem, a_desc0 + (uint64_t)((k * 32) >> 4), b_desc0 + (uint64_t)((k * 32) >> 4), (kc | k) ? 1u : 0u);
+                                    if (g == 0) umma_f16_ts(d_tmem, a_col0 + k * 8, b_desc0 + (uint64_t)((k * 32) >> 4), (kc | k) ? 1u : 0u);
+                                    else umma_f16_ss(d_tmem, a_desc0 + (uint64_t)((k * 32) >> 4), b_desc0 + (uint64_t)((k * 32) >> 4), (kc | k) ? 1u : 0u);
                                 }
                                 umma_commit_mc(&ms.b_empty[stage], (uint16_t)3);
                             }
@@ -699,8 +646,8 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
             if (leader) {
                 const uint64_t a_desc = umma_desc_sw32(smem_u32(smA1));
                 const uint64_t b_desc = umma_desc_sw32(smem_u32(dyn + B1_OFF + (int)l1_parts * (N_MMA * 32)));
-                umma_bf16_ss(tmem + TMEM_D_COL, a_desc, b_desc, 0u);
-                if (NIN == 5) umma_bf16_ss(tmem + TMEM_D_COL, a_desc + (uint64_t)(A1TC_KB_BYTES >> 4), b_desc + (uint64_t)(B1TC_KB_BYTES >> 4), 1u);   // second K block
+                umma_f16_ss(tmem + TMEM_D_COL, a_desc, b_desc, 0u);
+                if (NIN == 5) umma_f16_ss(tmem + TMEM_D_COL, a_desc + (uint64_t)(A1TC_KB_BYTES >> 4), b_desc + (uint64_t)(B1TC_KB_BYTES >> 4), 1u);   // second K block
                 umma_commit(&ms.d1_full);
             }
             __syncwarp();
@@ -742,7 +689,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                     for (int k = 0; k < KPS * (KCH / 16); ++k) {
                         const uint64_t b_desc = b_desc0 + (uint64_t)(((k / (KCH / 16)) * BOX_B + (k % (KCH / 16)) * 32) >> 4);
                         if constexpr (CG2) umma_f16_ts_2sm(d_tmem, a_col0 + k * 8, b_desc, (kb2 | k) ? 1u : 0u);
-                        else umma_bf16_ts(d_tmem, a_col0 + k * 8, b_desc, (kb2 | k) ? 1u : 0u);
+                        else umma_f16_ts(d_tmem, a_col0 + k * 8, b_desc, (kb2 | k) ? 1u : 0u);
                         // ping-pong: quarter 3 is the last reader of A -- release each 128-column part as soon as its MMAs
                         // retire so the other tile's layer 1 can overwrite it
                         if (PP && !L1TC && nq == N_QUARTERS - 1 && (k & 7) == 7) {
@@ -899,13 +846,9 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                         uint32_t pk[4];
 #pragma unroll
                         for (int p = 0; p < 4; ++p) {
-#if MPPI_MLP_PROBE & 2
-                            float pa = st.x + (float)p, pb = st.y + (float)p;
-#else
                             const float4 wa = ms.w01[col + 2 * p], wb = ms.w01[col + 2 * p + 1];
                             float pa = fmaf(wa.x, st.x, fmaf(wa.y, st.y, fmaf(wa.z, st.z, wa.w)));
                             float pb = fmaf(wb.x, st.x, fmaf(wb.y, st.y, fmaf(wb.z, st.z, wb.w)));
-#endif
                             if (NIN == 5) {
                                 const float4 wu = *reinterpret_cast<const float4 *>(&ms.w01u[col + 2 * p]);
                                 pa = fmaf(wu.x, st.w, fmaf(wu.y, su1, pa));
@@ -938,14 +881,9 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                 MLP_TOC(12);
 #pragma unroll
                 for (int i = 0; i < 32; ++i) {
-#if MPPI_MLP_PROBE & 1
-                    const float h = tanh_approx(__uint_as_float(v[i]));
-                    r0 += h;
-#else
                     const float4 w = ms.w3[col + i];
                     const float h = tanh_approx(__uint_as_float(v[i]) + w.x);
                     r0 = fmaf(w.y, h, r0); r1 = fmaf(w.z, h, r1); r2 = fmaf(w.w, h, r2);
-#endif
                 }
                 MLP_TOC(15);
             };
@@ -1076,13 +1014,9 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                         uint32_t pk[4];
 #pragma unroll
                         for (int p = 0; p < 4; ++p) {
-#if MPPI_MLP_PROBE & 2
-                            float pa = st.x + (float)p, pb = st.y + (float)p;
-#else
                             const float4 wa = ms.w01[col + 2 * p], wb = ms.w01[col + 2 * p + 1];
                             float pa = fmaf(wa.x, st.x, fmaf(wa.y, st.y, fmaf(wa.z, st.z, wa.w)));
                             float pb = fmaf(wb.x, st.x, fmaf(wb.y, st.y, fmaf(wb.z, st.z, wb.w)));
-#endif
                             if (NIN == 5) {
                                 const float4 wu = *reinterpret_cast<const float4 *>(&ms.w01u[col + 2 * p]);
                                 pa = fmaf(wu.x, st.w, fmaf(wu.y, su1, pa));
@@ -1108,7 +1042,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                     if (t + 1 < t1) control(t + 1, vn0, vn1);
                     sincos_cw(z[2], sn, cs);
                 }
-                // (2b) three tanh layers: epilogue of GEMM 1 = the A operand of GEMM 2.  D -> +bias -> tanh -> bf16, stored
+                // (2b) three tanh layers: epilogue of GEMM 1 = the A operand of GEMM 2.  D -> +bias -> tanh -> fp16, stored
                 //      to shared memory in the K-major 128B-swizzled layout (row r of K-chunk c at c*16 KB + (r/8)*1 KB +
                 //      (r%8)*128 B, 16-byte units XORed with r%8): conflict-free, a quarter-warp covers all 32 banks
                 if constexpr (NG == 2) {
@@ -1208,7 +1142,7 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32
 
 struct MlpState {
     int K = 0, T = 0, n_sm = 148;
-    mlp_op_t *d_w2 = nullptr;             // n_gemm x [512 out][512 in] fp16 (bf16), K-major B operand (layers stacked along the rows)
+    mlp_op_t *d_w2 = nullptr;             // n_gemm x [512 out][512 in] fp16, K-major B operand (layers stacked along the rows)
     float4 *d_w01 = nullptr, *d_w3 = nullptr;
     float2 *d_w01u = nullptr;             // control columns of the folded first layer (n_in = 5)
     float *d_b3 = nullptr;
@@ -1220,7 +1154,7 @@ struct MlpState {
     unsigned int epoch = 0;
     int n_in = 3, n_gemm = 1;
     CUtensorMap w2_map;
-    CUtensorMap w2_map_half;              // 64-row boxes: each CTA's half of a W2 box under pair MMAs (MPPI_MLP_CG2)
+    CUtensorMap w2_map_half;              // 64-row boxes: each CTA's half of a W2 box under pair MMAs
     bool ready = false;
 };
 
@@ -1324,12 +1258,8 @@ cudaError_t mlp_set_weights(MlpState *m, int n_in, int n_hidden, const float *co
     for (int g = 0; g < n_gemm; ++g)
         for (size_t i = 0; i < (size_t)HID * HID; ++i) {
             const float w = W[2 + g][i];
-#if MPPI_MLP_F16
             if (!(std::fabs(w) <= 65504.f)) return cudaErrorInvalidValue;      // outside half precision's range (or NaN)
             w2[(size_t)g * HID * HID + i] = __float2half_rn(w);
-#else
-            w2[(size_t)g * HID * HID + i] = __float2bfloat16(w);
-#endif
         }
     float b3[4] = {0.f, 0.f, 0.f, 0.f};
     for (int c = 0; c < 3; ++c) b3[c] = (float)((double)b[l_out][c] * (out_scale ? out_scale[c] : 1.0) + (out_mean ? out_mean[c] : 0.0));
@@ -1342,7 +1272,7 @@ cudaError_t mlp_set_weights(MlpState *m, int n_in, int n_hidden, const float *co
     if ((e = cudaMemcpyAsync(m->d_w2, w2.data(), sizeof(mlp_op_t) * w2.size(), cudaMemcpyHostToDevice, st)) != cudaSuccess) return e;
     if (n_gemm == 2 && (e = cudaMemcpyAsync(m->d_bh, b[2], sizeof(float) * HID, cudaMemcpyHostToDevice, st)) != cudaSuccess) return e;
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
-    // TMA descriptor of W2: inner dim = K (512 bf16, contiguous), outer dim = N (512 rows); 64 x 256 boxes, 128B swizzle
+    // TMA descriptor of W2: inner dim = K (512 fp16, contiguous), outer dim = N (512 rows); 64 x 256 boxes, 128B swizzle
     void *fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
     if ((e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres)) != cudaSuccess) return e;
@@ -1351,12 +1281,12 @@ cudaError_t mlp_set_weights(MlpState *m, int n_in, int n_hidden, const float *co
     const cuuint64_t strides[1] = {HID * sizeof(mlp_op_t)};
     const cuuint32_t box[2] = {KCH, N_MMA};
     const cuuint32_t estr[2] = {1, 1};
-    CUresult r = ((PFN_encodeTiled)fn)(&m->w2_map, MLP_TMAP_DTYPE, 2, m->d_w2, dims, strides, box, estr,
+    CUresult r = ((PFN_encodeTiled)fn)(&m->w2_map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, m->d_w2, dims, strides, box, estr,
                                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                                       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
     const cuuint32_t box_half[2] = {KCH, N_MMA / 2};
-    r = ((PFN_encodeTiled)fn)(&m->w2_map_half, MLP_TMAP_DTYPE, 2, m->d_w2, dims, strides, box_half, estr,
+    r = ((PFN_encodeTiled)fn)(&m->w2_map_half, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, m->d_w2, dims, strides, box_half, estr,
                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
