@@ -48,11 +48,12 @@ struct mppi_handle_s {
     TickArgs args{};
     cudaStream_t stream = nullptr;
     bool own_stream = false;
-    int n_sm = 148, occ = 1, nx = 3;
-    int grid_x = 1, grid_x_stash = 1;    // CTAs per robot: regenerate-noise kernels / stash kernels
+    int n_sm = 148, nx = 3;
+    // rollout plan, fixed at mppi_create (launch_tick applies it)
+    int tick_model = MPPI_MODEL_DIFFDRIVE;   // the tick kernels' model: learned dynamics reduce their costs in the diff-drive kernel
+    int grid_x[3] = {1, 1, 1};           // CTAs per robot of each rollout path: regenerate, noise stash, time-parallel
     bool stash = false;                  // Philox ticks keep the chunk's noise in shared memory
-    bool tpar = false;                   // ... and small sample counts run the horizon time-parallel (rollout_tpar), on grid_x_tpar CTAs
-    int grid_x_tpar = 1;
+    bool tpar = false;                   // ... and small sample counts run the horizon time-parallel (rollout_tpar)
     bool sum = false, strict = false;
     bool have_path = false;
     std::vector<double> path_h;          // host copy for the strict-mode step 1 (literal FP64)
@@ -253,6 +254,13 @@ static void build_filter(int T, int kind, std::vector<float> &M) {
     for (size_t i = 0; i < M.size(); ++i) M[i] = (float)m[i];
 }
 
+// The tick-kernel variant of configuration c with tick model `model` on rollout path `stash`.
+static TickKey tick_key(const mppi_config_t &c, int model, bool inj, int stash, bool scene = false) {
+    const int win = c.cost_kind == MPPI_COSTKIND_GOAL ? MPPI_WIN_GOAL : c.cost_kind == MPPI_COSTKIND_TARGET_SOFT ? MPPI_WIN_TARGET
+                  : c.window == 20 ? 20 : 0;
+    return TickKey{model, c.collision, win, c.cost_mode == MPPI_COST_SUM, inj, stash, scene};
+}
+
 static void refresh_obstacle_args(mppi_handle_t h, const double *xyr, int m) {
     TickArgs &a = h->args;
     const mppi_config_t &c = h->cfg;
@@ -286,15 +294,16 @@ int mppi_create(const mppi_config_t *cfg, mppi_handle_t *out) {
     if (cfg->temperature <= 0.0 || cfg->dt <= 0.0) return MPPI_E_BADARG;
     const double det = cfg->sigma[0] * cfg->sigma[3] - cfg->sigma[1] * cfg->sigma[2];
     if (!(cfg->sigma[0] > 0.0) || !(det > 0.0)) return MPPI_E_BADARG;
-    if (cfg->collision == MPPI_COLLISION_FOOTPRINT && cfg->model != MPPI_MODEL_BICYCLE) return MPPI_E_UNSUPPORTED;
+    // learned dynamics: one robot on a reference path, frozen waypoints, no obstacles; the diff-drive tick kernel reduces the
+    // costs the MLP kernel writes
     if (cfg->model == MPPI_MODEL_DIFFDRIVE_MLP &&
-        (cfg->waypoint_mode != MPPI_WP_FROZEN || cfg->n_robots != 1 || cfg->collision != MPPI_COLLISION_NONE))
+        (cfg->waypoint_mode != MPPI_WP_FROZEN || cfg->n_robots != 1 || cfg->collision != MPPI_COLLISION_NONE ||
+         cfg->cost_kind == MPPI_COSTKIND_GOAL || cfg->cost_kind == MPPI_COSTKIND_TARGET_SOFT))
         return MPPI_E_UNSUPPORTED;
+    const int tick_model = cfg->model == MPPI_MODEL_DIFFDRIVE_MLP ? MPPI_MODEL_DIFFDRIVE : cfg->model;
+    if (!mppi_tick_built(tick_key(*cfg, tick_model, false, 0))) return MPPI_E_UNSUPPORTED;
     if (cfg->cost_kind < MPPI_COSTKIND_PATH || cfg->cost_kind > MPPI_COSTKIND_TARGET_SOFT) return MPPI_E_BADARG;
     const bool pathless = cfg->cost_kind != MPPI_COSTKIND_PATH;
-    if (pathless && cfg->model != MPPI_MODEL_DIFFDRIVE) return MPPI_E_UNSUPPORTED;       // both scripts drive a unicycle
-    if (cfg->cost_kind == MPPI_COSTKIND_GOAL && cfg->collision == MPPI_COLLISION_FOOTPRINT) return MPPI_E_UNSUPPORTED;
-    if (cfg->cost_kind == MPPI_COSTKIND_TARGET_SOFT && cfg->collision != MPPI_COLLISION_NONE) return MPPI_E_UNSUPPORTED;
     if (cfg->waypoint_mode == MPPI_WP_STRICT && cfg->n_robots != 1 && !pathless) return MPPI_E_UNSUPPORTED;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0 || cfg->device >= ndev) return MPPI_E_CUDA;
@@ -326,29 +335,23 @@ int mppi_create(const mppi_config_t *cfg, mppi_handle_t *out) {
 
     const int R = c.n_robots, T = c.T, K = c.K;
     // Small sample counts are latency-bound (one thread walks one sample through the whole horizon): spread them over
-    // all SMs in CTAs that own as few as MPPI_MIN_CTA_SAMPLES samples (idle warps of a CTA cost nothing) instead of
-    // filling 256-thread CTAs on a fraction of the SMs.
-    int min_cta = 128;
-    if (const char *env = std::getenv("MPPI_MIN_CTA_SAMPLES")) min_cta = std::max(32, std::min(MPPI_BLOCK, std::atoi(env)));
-    const int chunks = (K + min_cta - 1) / min_cta;
-    const int tick_model = (c.model == MPPI_MODEL_DIFFDRIVE_MLP) ? MPPI_MODEL_DIFFDRIVE : c.model;
-    h->occ = std::max(1, mppi_tick_occupancy(tick_model, c.collision, c.cost_kind, h->sum, false, c.window, T, false));
-    const int occ_stash = mppi_tick_occupancy(tick_model, c.collision, c.cost_kind, h->sum, false, c.window, T, true);
+    // all SMs in CTAs that own as few as 128 samples (idle warps of a CTA cost nothing) instead of filling 256-thread CTAs
+    // on a fraction of the SMs.
+    const int chunks = (K + 127) / 128;
+    h->tick_model = tick_model;
+    const auto grid_for = [&](int occ) { return std::max(1, std::min((h->n_sm * std::max(1, occ) + R - 1) / R, chunks)); };
+    const int occ_stash = mppi_tick_occupancy(tick_key(c, tick_model, false, 1), T);
+    h->grid_x[0] = grid_for(mppi_tick_occupancy(tick_key(c, tick_model, false, 0), T));
+    h->grid_x[1] = grid_for(occ_stash);
     h->stash = occ_stash >= MPPI_STASH_BLOCKS && c.model != MPPI_MODEL_DIFFDRIVE_MLP;
-    int gx = (h->n_sm * h->occ + R - 1) / R;
-    gx = std::max(1, std::min(gx, chunks));
-    h->grid_x = gx;
-    int gxs = (h->n_sm * std::max(1, occ_stash) + R - 1) / R;
-    h->grid_x_stash = std::max(1, std::min(gxs, chunks));
-    gx = std::max(h->grid_x, h->grid_x_stash);
     // Time-parallel rollout (mppi_device.cuh, rollout_tpar): when one robot's samples cannot fill the GPU anyway -- every CTA would own
     // <= MPPI_TPAR_SLOTS of them at two CTAs per SM -- the tick is bound by the latency of one thread's walk through the horizon, and
     // splitting the horizon into noise / recurrence / cost phases over all threads of the CTA cuts that latency (race-car K = 16 384,
     // H = 50: 73 -> 47 us per tick).  Dynamic-window kernels only: with the static 20-entry window the stage cost is too cheap next to
     // the recurrence for the split to pay (diff-drive K = 16 384, H = 30: 22.3 -> 24.6 us, measured).  MPPI_TPAR=0 / 1 overrides.
     {
-        const int occ_tpar = (h->sum && c.cost_kind == MPPI_COSTKIND_PATH && c.window != 20 && c.model != MPPI_MODEL_DIFFDRIVE_MLP)
-                                 ? mppi_tick_occupancy(tick_model, c.collision, c.cost_kind, true, false, c.window, T, 2) : 0;
+        const TickKey kt = tick_key(c, tick_model, false, 2);
+        const int occ_tpar = mppi_tick_built(kt) && c.model != MPPI_MODEL_DIFFDRIVE_MLP ? mppi_tick_occupancy(kt, T) : 0;
         const int gt = std::max(1, std::min(h->n_sm * std::max(1, occ_tpar), (K + 7) / 8));
         const bool fits = occ_tpar >= 1 && (K + gt - 1) / gt <= MPPI_TPAR_SLOTS;
         bool want = R == 1;
@@ -358,13 +361,13 @@ int mppi_create(const mppi_config_t *cfg, mppi_handle_t *out) {
                          occ_tpar, gt, (int)fits, (int)want, (int)h->stash, (int)h->sum, c.window, K, T);
         if (want && fits) {
             h->tpar = true;
-            h->grid_x_tpar = gt;
-            gx = std::max(gx, gt);
+            h->grid_x[2] = gt;
         }
         if (std::getenv("MPPI_VERBOSE"))          // the path Philox ticks take, and its grid
             std::fprintf(stderr, "mppi_create: rollout path %s, %d CTAs per robot\n", h->tpar ? "tpar" : h->stash ? "stash" : "regenerate",
-                         h->tpar ? h->grid_x_tpar : h->stash ? h->grid_x_stash : h->grid_x);
+                         h->grid_x[h->tpar ? 2 : h->stash ? 1 : 0]);
     }
+    const int gx = *std::max_element(h->grid_x, h->grid_x + 3);      // the widest grid sizes the partials
 
     CKC(gmalloc(h, &h->d_U, sizeof(float) * R * T * 2));
     CKC(cudaMemset(h->d_U, 0, sizeof(float) * R * T * 2));
@@ -599,17 +602,15 @@ static int prepare_scene(mppi_handle_t h) {
     CK(h, cudaSetDevice(h->cfg.device));
     if (h->scene_stash < 0) {
         const mppi_config_t &c = h->cfg;
-        const bool want_stash = h->stash || h->tpar;
-        const int occ_st = want_stash ? mppi_tick_occupancy(c.model, c.collision, c.cost_kind, h->sum, false, c.window, c.T, 1, true) : 0;
-        const int occ_rg = occ_st >= 1 ? 0 : mppi_tick_occupancy(c.model, c.collision, c.cost_kind, h->sum, false, c.window, c.T, 0, true);
-        if (occ_st < 1 && occ_rg < 1)
+        if (!mppi_tick_built(tick_key(c, h->tick_model, false, 0, true)))
             return fail(h, MPPI_E_UNSUPPORTED, "per-robot goals / obstacles are built for diff-drive + circles and bicycle + footprint "
                                                "on a path, and for the GOAL (no obstacles or circles) and TARGET_SOFT cost kinds");
+        const int occ_st = h->stash || h->tpar ? mppi_tick_occupancy(tick_key(c, h->tick_model, false, 1, true), c.T) : 0;
         h->scene_stash = occ_st >= 1 ? 1 : 0;
         if (std::getenv("MPPI_VERBOSE"))
             std::fprintf(stderr, "mppi_set_robot_*: scene ticks take the %s path, %d CTAs per robot (occ %d)%s\n",
-                         h->scene_stash ? "stash" : "regenerate", h->scene_stash ? h->grid_x_stash : h->grid_x,
-                         h->scene_stash ? occ_st : occ_rg,
+                         h->scene_stash ? "stash" : "regenerate", h->grid_x[h->scene_stash],
+                         h->scene_stash ? occ_st : mppi_tick_occupancy(tick_key(c, h->tick_model, false, 0, true), c.T),
                          h->tpar ? "; this handle's shared-scene ticks are time-parallel, its scene ticks are not" : "");
     }
     if (!h->d_scene) {
@@ -827,18 +828,27 @@ static int strict_costs(mppi_handle_t h, const double *x0, const float *d_eps, f
     return MPPI_OK;
 }
 
-static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
-    const bool scene = a.scene_mask != 0;                // only the fleet entry points get here with a scene installed
-    const int stash = scene ? h->scene_stash : (!inj && !(a.flags & F_FROM_S)) ? (h->tpar ? 2 : h->stash ? 1 : 0) : 0;
-    dim3 grid(stash == 2 ? h->grid_x_tpar : stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
+// A tick launch on the handle's plan.  Its rollout path: a per-robot scene (installed only on fleet entry points) takes the one
+// prepare_scene chose; a Philox tick that updates the nominal from its own rollouts takes time-parallel (unless `tpar` is
+// false: mppi_step_batched), else the noise stash, else regenerate; injected noise, costs read from S and cost-only launches
+// regenerate.  The grid is that path's width per robot, one CTA for the learned-dynamics index update (F_IDX_ONLY).
+static cudaError_t launch_tick(mppi_handle_t h, const TickArgs &a, bool inj, bool tpar = true) {
+    const bool scene = a.scene_mask != 0;
+    int stash = 0;
+    if (scene) stash = h->scene_stash;
+    else if ((a.flags & F_UPDATE) && !(a.flags & F_FROM_S) && !inj) stash = tpar && h->tpar ? 2 : h->stash ? 1 : 0;
+    const dim3 grid((a.flags & F_IDX_ONLY) ? 1 : h->grid_x[stash], h->cfg.n_robots);
     if (a.trace) h->trace_grid = (int)grid.x;
-    const int model = (h->cfg.model == MPPI_MODEL_DIFFDRIVE_MLP) ? MPPI_MODEL_DIFFDRIVE : h->cfg.model;
+    return mppi_launch_tick(a, tick_key(h->cfg, h->tick_model, inj, stash, scene), grid, h->stream);
+}
+
+static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
     if (h->world > 1 && h->p2p && (a.flags & F_UPDATE)) {
         TickArgs b = a;                      // exchange fused into the tick kernel: ONE launch, no NCCL call
         b.flags |= F_P2P;
         for (int p = 0; p < h->world; ++p) b.peer_buf[p] = h->peer_buf[p];
         b.p2p_rank = h->rank; b.p2p_world = h->world; b.p2p_seq = ++h->p2p_seq; b.p2p_timeout_ms = h->p2p_timeout_ms;
-        CK(h, mppi_launch_tick(b, model, h->cfg.collision, h->cfg.cost_kind, h->sum, inj, stash, grid, h->stream));
+        CK(h, launch_tick(h, b, inj));
         h->tm.launches++;
         return MPPI_OK;
     }
@@ -846,7 +856,7 @@ static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
         TickArgs b = a;
         b.flags |= F_TRIPLE_OUT;
         b.triple_out = h->d_send;
-        CK(h, mppi_launch_tick(b, model, h->cfg.collision, h->cfg.cost_kind, h->sum, inj, stash, grid, h->stream));
+        CK(h, launch_tick(h, b, inj));
         const size_t nf = MPPI_NF(h->cfg.T);
         ncclResult_t r = g_nccl.AllGather(h->d_send, h->d_recv, nf, ncclFloat, h->comm, h->stream);
         if (r != ncclSuccess) { h->err = g_nccl.GetErrorString(r); return MPPI_E_NCCL; }
@@ -854,7 +864,7 @@ static int launch_update(mppi_handle_t h, const TickArgs &a, bool inj) {
         h->tm.launches += 2;
         return MPPI_OK;
     }
-    CK(h, mppi_launch_tick(a, model, h->cfg.collision, h->cfg.cost_kind, h->sum, inj, stash, grid, h->stream, scene));
+    CK(h, launch_tick(h, a, inj));
     h->tm.launches++;
     return MPPI_OK;
 }
@@ -873,7 +883,7 @@ static int step_common(mppi_handle_t h, const double *x0, const float *d_eps, ui
     if (h->mlp) {
         int rc = mlp_rollout_costs(h->mlp, h->args, h->sum, d_eps, h->d_S, h->stream);
         if (rc != 0) return fail(h, rc == -2 ? MPPI_E_STATE : MPPI_E_CUDA, rc == -2 ? "mppi_set_mlp has not been called" : "MLP rollout launch failed");
-        h->tm.launches += mlp_launches_per_tick(h->mlp);
+        h->tm.launches++;
         if (h->timing) CK(h, cudaEventRecord(h->ev[1], h->stream));
         TickArgs a = h->args;
         a.S = h->d_S; a.eps = d_eps;
@@ -934,12 +944,10 @@ int mppi_rollout_costs(mppi_handle_t h, const double *x0, const float *d_eps, ui
     set_seed(h, seed, tick);
     if (h->mlp) {
         if (mlp_rollout_costs(h->mlp, h->args, h->sum, d_eps, d_S, h->stream) != 0) return fail(h, MPPI_E_CUDA, "MLP rollout failed");
-        h->tm.launches += mlp_launches_per_tick(h->mlp);
+        h->tm.launches++;
         TickArgs a = h->args;
         a.flags = F_IDX_ONLY;
-        dim3 grid(1, 1);
-        if (a.trace) h->trace_grid = 1;
-        CK(h, mppi_launch_tick(a, MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE, MPPI_COSTKIND_PATH, h->sum, false, false, grid, h->stream));
+        CK(h, launch_tick(h, a, false));
         h->tm.launches++;
     } else if (h->strict) {
         int idx_after = 0;
@@ -951,9 +959,7 @@ int mppi_rollout_costs(mppi_handle_t h, const double *x0, const float *d_eps, ui
     } else {
         TickArgs a = h->args;
         a.eps = d_eps; a.S = d_S; a.flags = F_WRITE_S;
-        dim3 grid(h->grid_x, 1);
-        if (a.trace) h->trace_grid = (int)grid.x;
-        CK(h, mppi_launch_tick(a, h->cfg.model, h->cfg.collision, h->cfg.cost_kind, h->sum, d_eps != nullptr, false, grid, h->stream));
+        CK(h, launch_tick(h, a, d_eps != nullptr));
         h->tm.launches++;
     }
     CK(h, cudaStreamSynchronize(h->stream));
@@ -1091,18 +1097,16 @@ int mppi_run_closed_loop(mppi_handle_t h, const double *x0, int32_t n_ticks, uin
 
     // The n ticks as ONE CUDA graph of n identical kernel nodes: every launch carries the same arguments (the running tick
     // and the log row come from d_loop, advanced by each launch's last CTA), so the instantiated graph is reused by every
-    // later call with the same (n_ticks, plant, seed, sample-cost flag, obstacle set); MPPI_CLOSED_LOOP_GRAPH=0 falls back
-    // to n stream launches (A/B measurements).  Per-robot goals / obstacles are read from the handle's table, whose pointer
-    // never changes: re-installing them between calls does not re-instantiate the graph.
+    // later call with the same (n_ticks, plant, seed, sample-cost flag, obstacle set).  Per-robot goals / obstacles are read
+    // from the handle's table, whose pointer never changes: re-installing them between calls does not re-instantiate the graph.
     set_seed(h, seed, 0);
     TickArgs a = h->args;
     a.x0_dev = h->d_x0; a.eps = nullptr; a.S = nullptr; a.flags = F_UPDATE;
     if (R > 1) a.out_host = nullptr;
     a.plant_state = h->d_x0; a.plant_log = h->d_plant_log; a.plant_mode = plant; a.plant_tick = 0; a.plant_n = n_ticks;
     a.loop_state = h->d_loop; a.loop_ticket = h->d_loop + 2;
-    static const bool use_graph = [] { const char *e = std::getenv("MPPI_CLOSED_LOOP_GRAPH"); return !(e && e[0] == '0'); }();
     const bool same = h->loop_graph && h->loop_graph_n == n_ticks && std::memcmp(&h->loop_graph_args, &a, sizeof(TickArgs)) == 0;
-    if (use_graph && !same) {
+    if (!same) {
         if (h->loop_graph) { cudaGraphExecDestroy(h->loop_graph); h->loop_graph = nullptr; }
         cudaGraph_t g = nullptr;
         const int launches_before = h->tm.launches;
@@ -1126,15 +1130,8 @@ int mppi_run_closed_loop(mppi_handle_t h, const double *x0, int32_t n_ticks, uin
         if (ce != cudaSuccess) { h->loop_graph = nullptr; return fail(h, MPPI_E_CUDA, "closed loop: graph instantiation failed"); }
         h->loop_graph_n = n_ticks; h->loop_graph_args = a;
     }
-    if (use_graph) {
-        CK(h, cudaGraphLaunch(h->loop_graph, h->stream));
-        h->tm.launches += n_ticks;
-    } else {
-        for (int i = 0; i < n_ticks; ++i) {
-            int rc = launch_update(h, a, false);
-            if (rc != MPPI_OK) return rc;
-        }
-    }
+    CK(h, cudaGraphLaunch(h->loop_graph, h->stream));
+    h->tm.launches += n_ticks;
     std::vector<float> log(log_floats);
     CK(h, cudaMemcpyAsync(log.data(), h->d_plant_log, sizeof(float) * log_floats, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
@@ -1157,11 +1154,7 @@ int mppi_step_batched(mppi_handle_t h, const float *d_x0, uint64_t seed, uint64_
                             h->cfg.n_robots, cudaMemcpyDeviceToDevice, h->stream));
     a.x0_dev = h->d_x0; a.eps = nullptr; a.S = nullptr; a.flags = F_UPDATE; a.u0_out = d_u0_out;
     a.out_host = nullptr;
-    const bool scene = a.scene_mask != 0;
-    const int stash = scene ? h->scene_stash : h->stash ? 1 : 0;
-    dim3 grid(stash ? h->grid_x_stash : h->grid_x, h->cfg.n_robots);
-    if (a.trace) h->trace_grid = (int)grid.x;
-    CK(h, mppi_launch_tick(a, h->cfg.model, h->cfg.collision, h->cfg.cost_kind, h->sum, false, stash, grid, h->stream, scene));
+    CK(h, launch_tick(h, a, false, false));
     h->tm.launches++;
     return MPPI_OK;
 }
@@ -1236,7 +1229,7 @@ int mppi_set_trace(mppi_handle_t h, int32_t on) {
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaStreamSynchronize(h->stream));
     if (on && !h->d_trace) {
-        h->trace_n = 2 * (std::max(std::max(h->grid_x, h->grid_x_stash), h->grid_x_tpar) + 1);
+        h->trace_n = 2 * (*std::max_element(h->grid_x, h->grid_x + 3) + 1);
         CK(h, gmalloc(h, &h->d_trace, sizeof(unsigned long long) * h->trace_n));
         CK(h, cudaMemset(h->d_trace, 0, sizeof(unsigned long long) * h->trace_n));
     }

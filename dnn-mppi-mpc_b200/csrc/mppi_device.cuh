@@ -518,6 +518,37 @@ __device__ __forceinline__ float tracking_cost(const float4 ref, const float z[4
 #define MPPI_WIN_GOAL (-1)
 #define MPPI_WIN_TARGET (-2)
 
+// One tick-kernel variant: model (MPPI_MODEL_DIFFDRIVE / _BICYCLE), collision, window (20, 0 = dynamic, MPPI_WIN_GOAL,
+// MPPI_WIN_TARGET), cost mode sum, injected noise, rollout path (0 regenerate, 1 noise stash, 2 stash + time-parallel) and
+// per-robot scene.
+struct TickKey {
+    int model, coll, win;
+    bool sum, inj;
+    int stash;
+    bool scene;
+};
+
+// The variants this library builds -- the one statement of that set (111 kernels):
+//  - path tracking, static or dynamic window: diff-drive without obstacles or with circles, bicycle with every collision
+//    model; cost mode last or sum; injected noise on the regenerate path, Philox noise on the regenerate or noise-stash
+//    path, and time-parallel for Philox noise, sum mode and the dynamic window;
+//  - the path-free cost kinds, diff-drive only: GOAL without obstacles or with circles, TARGET_SOFT without obstacles,
+//    with the same noise / path choices except time-parallel;
+//  - per-robot scenes (fleets): Philox noise, regenerate or noise stash, for diff-drive + circles and bicycle + footprint
+//    on a path and for the path-free kinds.
+__host__ __device__ constexpr bool mppi_tick_built(const TickKey &k) {
+    const bool dd = k.model == MPPI_MODEL_DIFFDRIVE, bic = k.model == MPPI_MODEL_BICYCLE;
+    const bool circle = k.coll == MPPI_COLLISION_CIRCLE, footprint = k.coll == MPPI_COLLISION_FOOTPRINT;
+    const bool coll_ok = k.coll == MPPI_COLLISION_NONE || circle || footprint;
+    if (k.win == MPPI_WIN_GOAL) { if (!dd || !coll_ok || footprint) return false; }
+    else if (k.win == MPPI_WIN_TARGET) { if (!dd || k.coll != MPPI_COLLISION_NONE) return false; }
+    else if (k.win == 20 || k.win == 0) { if (!(dd || bic) || !coll_ok || (dd && footprint)) return false; }
+    else return false;
+    if (k.stash < 0 || k.stash > 2 || (k.inj && k.stash != 0)) return false;
+    if (k.stash == 2) return k.sum && k.win == 0 && !k.scene;
+    return !k.scene || (!k.inj && (k.win < 0 || (dd && circle) || (bic && footprint)));
+}
+
 // Goal-point cost of test/mppi_differential_drive_obs.py:202-232: w0 * |xy - goal|^2 + w1 * wrap(atan2(dy, dx) - yaw)^2
 // with (dx, dy) = xy - goal (the bearing FROM the goal, as the reference writes it) and wrap(a) =
 // atan2(sin a, cos a) in (-pi, pi], evaluated as the FMA remainder a - 2pi*rint(a / 2pi) (only its square is used).

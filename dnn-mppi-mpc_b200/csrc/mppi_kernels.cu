@@ -9,8 +9,10 @@
 #include "mppi_launch.h"
 
 #include <algorithm>
+#include <array>
+#include <atomic>
 #include <mutex>
-#include <vector>
+#include <utility>
 
 namespace {
 
@@ -324,6 +326,7 @@ __device__ __forceinline__ auto &scene_src(const TickArgs &a) {
 // STASH: 0 regenerate, 1 noise stash, 2 stash + time-parallel rollout.  SCENE: per-robot goal / obstacles (fleets).
 template <int MODEL, int COLL, bool SUM, bool INJ, int WIN, int STASH, bool SCENE>
 __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick_add) {
+    static_assert(mppi_tick_built(TickKey{MODEL, COLL, WIN, SUM, INJ, STASH, SCENE}), "a variant mppi_tick_built does not list");
     __shared__ TickSmem sm;
     __shared__ RunSmem run;
     __shared__ MergeSmem ms;
@@ -340,7 +343,6 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
     if constexpr (SCENE) {
         // this robot's scene, each component from its per-robot record or from the shared fields; the obstacle count is
         // per CTA, so the obstacle loops stay warp-uniform
-        static_assert(STASH != 2, "scene ticks take the noise-stash or regenerate path");
         const SceneRec &row = a.scene[robot];
         const bool pg = a.scene_mask & MPPI_SCENE_GOAL, po = a.scene_mask & MPPI_SCENE_OBS;
         if (tid < 4) sc.goal[tid] = pg ? row.goal[tid] : a.goal[tid];
@@ -430,7 +432,6 @@ __device__ __forceinline__ void tick_body(const TickArgs &a, const uint32_t tick
     MPPI_DCHECK(k_begin >= 0 && k_end <= K && (!STASH || (size_t)T * MPPI_BLOCK * sizeof(float2) <= 232448));
     float *Srow = a.S ? a.S + (size_t)robot * K : nullptr;
     // (time-parallel rollout: chunks of MPPI_TPAR_SLOTS samples on chunk slots 0 .. MPPI_TPAR_SLOTS - 1, the other slots idle)
-    static_assert(STASH != 2 || (SUM && !INJ), "time-parallel rollout: sum mode, Philox noise");
     constexpr int CHUNK_STRIDE = STASH == 2 ? MPPI_TPAR_SLOTS : MPPI_BLOCK;
     for (int base = k_begin; base < k_end; base += CHUNK_STRIDE) {
         int k[SPT], ksafe[SPT], ncoll[SPT];
@@ -916,95 +917,73 @@ __global__ void __launch_bounds__(MPPI_BLOCK) mppi_strict_kernel(const __grid_co
 }  // namespace
 
 // ------------------------------------------------------------------------------------------
-// dispatch
+// dispatch: a table of every built tick kernel, indexed by its packed key
 // ------------------------------------------------------------------------------------------
-// Calls f(kernel pointer) for the instantiation selected by the runtime mode flags.
-// The path-free cost kinds (diff-drive only) have a handful of instantiations of their own.
-template <int COLL, int WIN, typename F>
-static cudaError_t with_tick_kernel_nopath(bool sum, bool inj, int stash, F &&f) {
-#define MPPI_PICK(S, I, ST) return f(mppi_tick_kernel<MPPI_MODEL_DIFFDRIVE, COLL, S, I, WIN, ST>)
-    if (sum) {
-        if (inj) MPPI_PICK(true, true, false);
-        if (stash) MPPI_PICK(true, false, true);
-        MPPI_PICK(true, false, false);
-    }
-    if (inj) MPPI_PICK(false, true, false);
-    if (stash) MPPI_PICK(false, false, true);
-    MPPI_PICK(false, false, false);
-#undef MPPI_PICK
+namespace {
+constexpr int kTickSlots = 2 * 3 * 4 * 2 * 2 * 3 * 2;      // model, collision, window, sum, inj, stash, scene
+constexpr int kMaxDevices = 64;
+
+// the table slot of a key whose fields are in range (built or not)
+constexpr int tick_slot(const TickKey &k) {
+    const int w = k.win == 20 ? 0 : k.win == 0 ? 1 : k.win == MPPI_WIN_GOAL ? 2 : 3;
+    return (((((k.model * 3 + k.coll) * 4 + w) * 2 + k.sum) * 2 + k.inj) * 3 + k.stash) * 2 + k.scene;
 }
 
-template <int MODEL, int COLL, typename F>
-static cudaError_t with_tick_kernel_mc(bool sum, bool inj, bool win20, int stash, F &&f) {
-#define MPPI_PICK(S, I, W, ST) return f(mppi_tick_kernel<MODEL, COLL, S, I, W, ST>)
-    if (sum) {
-        if (inj) { if (win20) MPPI_PICK(true, true, 20, false); else MPPI_PICK(true, true, 0, false); }
-        if (stash == 2 && !win20) MPPI_PICK(true, false, 0, 2);       // time-parallel rollout: dynamic-window kernels only (see mppi_api.cu)
-        if (stash) { if (win20) MPPI_PICK(true, false, 20, 1); else MPPI_PICK(true, false, 0, 1); }
-        if (win20) MPPI_PICK(true, false, 20, 0); else MPPI_PICK(true, false, 0, 0);
-    } else {
-        if (inj) { if (win20) MPPI_PICK(false, true, 20, false); else MPPI_PICK(false, true, 0, false); }
-        if (stash) { if (win20) MPPI_PICK(false, false, 20, true); else MPPI_PICK(false, false, 0, true); }
-        if (win20) MPPI_PICK(false, false, 20, false); else MPPI_PICK(false, false, 0, false);
-    }
-#undef MPPI_PICK
+// The i-th key in the order the table names the kernels, which is the order the device compiler meets them in.  Its inlining
+// and scheduling of helpers several kernels share depend on that order, so it is the order the earlier if-chain dispatchers
+// named them in: scene variants first, then goal, target and path kinds, model, collision; flags descending and window 20
+// before the dynamic one, the window above sum and stash for scene variants and below them for the others.
+constexpr int kTickOrder = 2 * 3 * 2 * 3 * 24;
+constexpr TickKey ordered_key(int i) {
+    TickKey k{};
+    k.scene = i < kTickOrder / 2;
+    const int kind = i / 144 % 3, w = k.scene ? i / 12 % 2 : i % 2;
+    k.model = i / 72 % 2;
+    k.coll = i / 24 % 3;
+    k.win = kind == 0 ? MPPI_WIN_GOAL : kind == 1 ? MPPI_WIN_TARGET : w ? 0 : 20;
+    k.sum = (k.scene ? i / 6 : i / 12) % 2 == 0;
+    k.inj = (k.scene ? i / 3 : i / 6) % 2 == 0;
+    k.stash = 2 - (k.scene ? i : i / 2) % 3;
+    return k;
 }
 
-// Per-robot-scene instantiations: only what fleets launch (Philox noise, noise stash or regenerate, cost mode last / sum)
-// for diff-drive + circles and bicycle + footprint on a path (static and dynamic window), and the path-free kinds.
-template <int MODEL, int COLL, int WIN, typename F>
-static cudaError_t with_scene_kernel_w(bool sum, int stash, F &&f) {
-#define MPPI_PICK(S, ST) return f(mppi_tick_kernel<MODEL, COLL, S, false, WIN, ST, true>)
-    if (sum) { if (stash) MPPI_PICK(true, 1); MPPI_PICK(true, 0); }
-    if (stash) MPPI_PICK(false, 1);
-    MPPI_PICK(false, 0);
-#undef MPPI_PICK
-}
+using TickKernel = void (*)(TickArgs);
 
-template <typename F>
-static cudaError_t with_scene_kernel(int model, int coll, int cost_kind, bool sum, bool inj, bool win20, int stash, F &&f) {
-    if (inj || stash == 2 || model == MPPI_MODEL_DIFFDRIVE_MLP) return cudaErrorInvalidValue;
-    if (cost_kind == MPPI_COSTKIND_GOAL) {
-        if (coll == MPPI_COLLISION_NONE) return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE, MPPI_WIN_GOAL>(sum, stash, f);
-        if (coll == MPPI_COLLISION_CIRCLE) return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE, MPPI_WIN_GOAL>(sum, stash, f);
-        return cudaErrorInvalidValue;
-    }
-    if (cost_kind == MPPI_COSTKIND_TARGET_SOFT)
-        return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE, MPPI_WIN_TARGET>(sum, stash, f);
-    if (model == MPPI_MODEL_DIFFDRIVE && coll == MPPI_COLLISION_CIRCLE) {
-        if (win20) return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE, 20>(sum, stash, f);
-        return with_scene_kernel_w<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE, 0>(sum, stash, f);
-    }
-    if (model == MPPI_MODEL_BICYCLE && coll == MPPI_COLLISION_FOOTPRINT) {
-        if (win20) return with_scene_kernel_w<MPPI_MODEL_BICYCLE, MPPI_COLLISION_FOOTPRINT, 20>(sum, stash, f);
-        return with_scene_kernel_w<MPPI_MODEL_BICYCLE, MPPI_COLLISION_FOOTPRINT, 0>(sum, stash, f);
-    }
-    return cudaErrorInvalidValue;
+template <int I>
+constexpr TickKernel tick_kernel_at() {
+    constexpr TickKey k = ordered_key(I);
+    if constexpr (mppi_tick_built(k)) return mppi_tick_kernel<k.model, k.coll, k.sum, k.inj, k.win, k.stash, k.scene>;
+    else return nullptr;
 }
+template <int... I>
+constexpr std::array<TickKernel, kTickSlots> tick_table(std::integer_sequence<int, I...>) {
+    std::array<TickKernel, kTickSlots> t{};
+    ((t[tick_slot(ordered_key(I))] = tick_kernel_at<I>()), ...);
+    return t;
+}
+constexpr std::array<TickKernel, kTickSlots> kTickKernels = tick_table(std::make_integer_sequence<int, kTickOrder>{});
 
-template <typename F>
-static cudaError_t with_tick_kernel(int model, int coll, int cost_kind, bool sum, bool inj, bool win20, int stash, bool scene, F &&f) {
-    if (scene) return with_scene_kernel(model, coll, cost_kind, sum, inj, win20, stash, f);
-    if (cost_kind == MPPI_COSTKIND_GOAL) {              // test/mppi_differential_drive_obs.py: unicycle, circle obstacles
-        if (model != MPPI_MODEL_DIFFDRIVE) return cudaErrorInvalidValue;
-        if (coll == MPPI_COLLISION_NONE) return with_tick_kernel_nopath<MPPI_COLLISION_NONE, MPPI_WIN_GOAL>(sum, inj, stash, f);
-        if (coll == MPPI_COLLISION_CIRCLE) return with_tick_kernel_nopath<MPPI_COLLISION_CIRCLE, MPPI_WIN_GOAL>(sum, inj, stash, f);
-        return cudaErrorInvalidValue;
-    }
-    if (cost_kind == MPPI_COSTKIND_TARGET_SOFT) {       // test/test_mppi_diff_obs.py: unicycle, soft moving obstacles
-        if (model != MPPI_MODEL_DIFFDRIVE || coll != MPPI_COLLISION_NONE) return cudaErrorInvalidValue;
-        return with_tick_kernel_nopath<MPPI_COLLISION_NONE, MPPI_WIN_TARGET>(sum, inj, stash, f);
-    }
-    if (model == MPPI_MODEL_DIFFDRIVE) {
-        if (coll == MPPI_COLLISION_NONE) return with_tick_kernel_mc<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_NONE>(sum, inj, win20, stash, f);
-        if (coll == MPPI_COLLISION_CIRCLE) return with_tick_kernel_mc<MPPI_MODEL_DIFFDRIVE, MPPI_COLLISION_CIRCLE>(sum, inj, win20, stash, f);
-    } else if (model == MPPI_MODEL_BICYCLE) {
-        if (coll == MPPI_COLLISION_NONE) return with_tick_kernel_mc<MPPI_MODEL_BICYCLE, MPPI_COLLISION_NONE>(sum, inj, win20, stash, f);
-        if (coll == MPPI_COLLISION_CIRCLE) return with_tick_kernel_mc<MPPI_MODEL_BICYCLE, MPPI_COLLISION_CIRCLE>(sum, inj, win20, stash, f);
-        if (coll == MPPI_COLLISION_FOOTPRINT) return with_tick_kernel_mc<MPPI_MODEL_BICYCLE, MPPI_COLLISION_FOOTPRINT>(sum, inj, win20, stash, f);
-    }
-    return cudaErrorInvalidValue;
+// Opt-in of kTickKernels[s] to `dyn` bytes of dynamic shared memory on the current device.  The attribute belongs to the
+// function, so every handle of a variant shares it: it is only ever RAISED, under one lock, and the slot's record keeps the
+// largest size set per device.  Setting it to each new handle's own size would cut it below what a live handle with a longer
+// horizon launches with, and that handle's next tick would fail with cudaErrorInvalidValue.  A size the record already
+// covers is read without the lock: the record only grows.
+cudaError_t opt_in_dyn_smem(int s, size_t dyn) {
+    if (dyn <= 32 * 1024) return cudaSuccess;       // static shared memory (12 KB) counts against the 48 KB default limit too
+    static std::atomic<unsigned> raised[kTickSlots][kMaxDevices];
+    static std::mutex mu;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= kMaxDevices) return cudaErrorInvalidDevice;
+    std::atomic<unsigned> &rec = raised[s][dev];
+    if (rec.load(std::memory_order_acquire) >= dyn) return cudaSuccess;
+    std::lock_guard<std::mutex> lock(mu);
+    if (rec.load(std::memory_order_relaxed) >= dyn) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute((const void *)kTickKernels[s], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
+    if (e == cudaSuccess) rec.store((unsigned)dyn, std::memory_order_release);
+    return e;
 }
+}  // namespace
 
 size_t mppi_tick_dyn_smem(int T, int stash) {
     // regenerate path: per-warp column sums (8 KB), also large enough for the exchange's gathered triples
@@ -1013,65 +992,26 @@ size_t mppi_tick_dyn_smem(int T, int stash) {
     return stash ? std::max(sizeof(float2) * (size_t)T * MPPI_BLOCK, small) : small;
 }
 
-// Opt-in of a tick kernel to `dyn` bytes of dynamic shared memory on the current device.  The attribute belongs to the
-// function, so every handle of an instantiation shares it: it is only ever RAISED, under one process-wide record of the
-// largest opt-in per (kernel, device).  Setting it to each new handle's own size would cut it below what a live handle with a
-// longer horizon launches with, and that handle's next tick would fail with cudaErrorInvalidValue.
-static cudaError_t raise_dyn_smem_limit(const void *kern, int dev, size_t dyn) {
-    struct OptIn { const void *kern; int dev; size_t dyn; };
-    static std::mutex mu;
-    static std::vector<OptIn> done;
-    std::lock_guard<std::mutex> lock(mu);
-    OptIn *rec = nullptr;
-    for (OptIn &o : done)
-        if (o.kern == kern && o.dev == dev) { rec = &o; break; }
-    if (rec && rec->dyn >= dyn) return cudaSuccess;
-    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
-    if (e != cudaSuccess) return e;
-    if (rec) rec->dyn = dyn;
-    else done.push_back({kern, dev, dyn});
-    return cudaSuccess;
+cudaError_t mppi_launch_tick(const TickArgs &a, const TickKey &k, dim3 grid, cudaStream_t st) {
+    if (!mppi_tick_built(k)) return cudaErrorInvalidValue;
+    const int s = tick_slot(k);
+    const size_t dyn = mppi_tick_dyn_smem(a.T, k.stash);
+    if (const cudaError_t e = opt_in_dyn_smem(s, dyn)) return e;
+    kTickKernels[s]<<<grid, MPPI_BLOCK, dyn, st>>>(a);
+    return cudaGetLastError();
 }
 
-cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_kind, bool sum, bool inj, int stash, dim3 grid,
-                             cudaStream_t st, bool scene) {
-    const size_t dyn = mppi_tick_dyn_smem(a.T, stash);
-    return with_tick_kernel(model, coll, cost_kind, sum, inj, a.window == 20, stash, scene, [&](auto kern) {
-        if (dyn > 32 * 1024) {          // static shared memory (12 KB) counts against the 48 KB default limit too
-            // lock-free fast path: a limit this thread has seen at >= dyn is still >= dyn (it only rises)
-            static thread_local const void *done_kern[64];
-            static thread_local size_t done_dyn[64];
-            static thread_local int done_dev[64], n_done = 0;
-            int dev = 0;
-            cudaGetDevice(&dev);
-            bool found = false;
-            for (int i = 0; i < n_done; ++i)
-                if (done_kern[i] == (const void *)kern && done_dev[i] == dev && done_dyn[i] >= dyn) { found = true; break; }
-            if (!found) {
-                cudaError_t e = raise_dyn_smem_limit((const void *)kern, dev, dyn);
-                if (e != cudaSuccess) return e;
-                if (n_done < 64) { done_kern[n_done] = (const void *)kern; done_dyn[n_done] = dyn; done_dev[n_done] = dev; ++n_done; }
-            }
-        }
-        kern<<<grid, MPPI_BLOCK, dyn, st>>>(a);
-        return cudaGetLastError();
-    });
-}
-
-// Resident CTAs per SM of the instantiation the given modes select (0 if it cannot launch).
-int mppi_tick_occupancy(int model, int coll, int cost_kind, bool sum, bool inj, int window, int T, int stash, bool scene) {
+// Resident CTAs per SM of a variant (0 if it is not built or cannot launch).
+int mppi_tick_occupancy(const TickKey &k, int T) {
+    if (!mppi_tick_built(k)) return 0;
+    const int s = tick_slot(k);
+    const size_t dyn = mppi_tick_dyn_smem(T, k.stash);
     int nb = 0;
-    const size_t dyn = mppi_tick_dyn_smem(T, stash);
-    cudaError_t e = with_tick_kernel(model, coll, cost_kind, sum, inj, window == 20, stash, scene, [&](auto kern) {
-        if (dyn > 32 * 1024) {          // static shared memory (12 KB) counts against the 48 KB default limit too
-            int dev = 0;
-            cudaGetDevice(&dev);
-            cudaError_t e2 = raise_dyn_smem_limit((const void *)kern, dev, dyn);
-            if (e2 != cudaSuccess) return e2;
-        }
-        return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, MPPI_BLOCK, dyn);
-    });
-    if (e != cudaSuccess) { cudaGetLastError(); return 0; }
+    if (opt_in_dyn_smem(s, dyn) != cudaSuccess ||
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kTickKernels[s], MPPI_BLOCK, dyn) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
     return nb;
 }
 

@@ -3,10 +3,9 @@
 #include <cuda_runtime.h>
 struct TickArgs;
 struct SceneRec;
-// stash: 0 regenerate, 1 noise stash, 2 stash + time-parallel rollout; scene: the per-robot-scene instantiation (a.scene /
-// a.scene_mask; Philox noise, stash 0 or 1, the combinations mppi_set_robot_* accept -- cudaErrorInvalidValue otherwise)
-cudaError_t mppi_launch_tick(const TickArgs &a, int model, int coll, int cost_kind, bool sum, bool inj, int stash, dim3 grid,
-                             cudaStream_t st, bool scene = false);
+struct TickKey;
+// the tick kernel of variant k (mppi_device.cuh: mppi_tick_built); cudaErrorInvalidValue for a variant that is not built
+cudaError_t mppi_launch_tick(const TickArgs &a, const TickKey &k, dim3 grid, cudaStream_t st);
 size_t mppi_tick_dyn_smem(int T, int stash);
 cudaError_t mppi_launch_strict(const TickArgs &a, int model, int coll, bool sum, bool inj, const unsigned *bp_n,
                                const int *bp_s, int nbp, int k_first, unsigned check_from,
@@ -24,7 +23,7 @@ size_t mppi_sort_costs_temp_bytes(int K);
 cudaError_t mppi_sort_costs(const float *d_S, int K, float *d_S_sorted, int *d_idx_sorted, int *d_iota, void *d_temp,
                             size_t temp_bytes, cudaStream_t st);
 cudaError_t mppi_launch_noise(const TickArgs &a, float *d_out, int robot, cudaStream_t st);
-int mppi_tick_occupancy(int model, int coll, int cost_kind, bool sum, bool inj, int window, int T, int stash, bool scene = false);
+int mppi_tick_occupancy(const TickKey &k, int T);
 // Installs per-robot scene components into d_scene[R] (in stream order; FP64 conversions of refresh_obstacle_args).
 //   obstacles: d_obs (R, m, ncol) float32, ncol 3 [x, y, r] (circle: r2 = (rr_base + r)^2 with rr_base = robot radius * margin;
 //   footprint: r2 = r^2; far2 = ((diag + r) * 1.001 + 1e-3)^2) or 4 [x, y, vx, vy]; d_count (R) int32 or null

@@ -1320,18 +1320,17 @@ int mlp_rollout_costs(MlpState *m, const TickArgs &args, bool sum, const float *
     a.flags = sum ? F_COST_SUM : 0;
     const int n_tiles = (a.K + TILE_M - 1) / TILE_M;
     int grid = std::min(((n_tiles + 1) / 2) * 2, m->n_sm & ~1);       // whole clusters of 2
-    // two tiles per CTA in flight (ping-pong) whenever a CTA owns more than one tile; MPPI_MLP_PINGPONG=0 forces the
-    // one-tile schedule (A/B measurements)
-    static const bool allow_pp = [] { const char *e = std::getenv("MPPI_MLP_PINGPONG"); return !(e && e[0] == '0'); }();
-    const bool pp = allow_pp && n_tiles > grid && m->n_gemm == 1;
+    // two tiles per CTA in flight (ping-pong) whenever a CTA owns more than one tile
+    const bool pp = n_tiles > grid && m->n_gemm == 1;
+    // the instantiation: (n_in, ping-pong, GEMMs per step) = variant (n_in 3 / 5 alternate)
+    static const decltype(&mppi_mlp_rollout_kernel<3, false, 1>) kernels[6] = {
+        mppi_mlp_rollout_kernel<3, false, 1>, mppi_mlp_rollout_kernel<5, false, 1>, mppi_mlp_rollout_kernel<3, true, 1>,
+        mppi_mlp_rollout_kernel<5, true, 1>,  mppi_mlp_rollout_kernel<3, false, 2>, mppi_mlp_rollout_kernel<5, false, 2>};
+    const int variant = (m->n_gemm == 2 ? 4 : (pp ? 2 : 0)) + (m->n_in == 5 ? 1 : 0);
     // never launch more clusters than the device keeps resident at once (fused-off SMs, MPS partitions): the grid is
     // persistent, so a smaller one only means more tiles per cluster
-    const int variant = (m->n_gemm == 2 ? 4 : (pp ? 2 : 0)) + (m->n_in == 5 ? 1 : 0);
     if (m->max_clusters[variant] == 0) {
-        int n = 0;
-        if (m->n_gemm == 2) n = m->n_in == 5 ? mlp_max_active_clusters(mppi_mlp_rollout_kernel<5, false, 2>, m->n_sm) : mlp_max_active_clusters(mppi_mlp_rollout_kernel<3, false, 2>, m->n_sm);
-        else if (pp) n = m->n_in == 5 ? mlp_max_active_clusters(mppi_mlp_rollout_kernel<5, true, 1>, m->n_sm) : mlp_max_active_clusters(mppi_mlp_rollout_kernel<3, true, 1>, m->n_sm);
-        else n = m->n_in == 5 ? mlp_max_active_clusters(mppi_mlp_rollout_kernel<5, false, 1>, m->n_sm) : mlp_max_active_clusters(mppi_mlp_rollout_kernel<3, false, 1>, m->n_sm);
+        const int n = mlp_max_active_clusters(kernels[variant], m->n_sm);
         m->max_clusters[variant] = n > 0 ? n : -1;                    // -1: the query failed, keep the SM-count grid
     }
     if (m->max_clusters[variant] > 0) grid = std::min(grid, 2 * m->max_clusters[variant]);
@@ -1345,15 +1344,11 @@ int mlp_rollout_costs(MlpState *m, const TickArgs &args, bool sum, const float *
                           (long long)n_quads * a.T / n_clusters >= a.T + 2) ? 1 : 0;
     const unsigned int epoch = ++m->epoch;
     unsigned int *fault = m->d_hand_flag + (size_t)(m->n_sm / 2 + 1) * 2;
-#define MPPI_MLP_LAUNCH(N, P, G) mppi_mlp_rollout_kernel<N, P, G><<<grid, MLP_THREADS, MLP_DYN_SMEM, st>>>(a, mlp_use_cg2(N, P, G) ? m->w2_map_half : m->w2_map, m->d_w01, m->d_w01u, m->d_w3, m->d_b3, m->d_bh, d_S, n_tiles, m->d_hand, m->d_hand_flag, fault, epoch, balanced, m->d_b1)
-    if (m->n_gemm == 2) { if (m->n_in == 5) MPPI_MLP_LAUNCH(5, false, 2); else MPPI_MLP_LAUNCH(3, false, 2); }
-    else if (m->n_in == 5) { if (pp) MPPI_MLP_LAUNCH(5, true, 1); else MPPI_MLP_LAUNCH(5, false, 1); }
-    else { if (pp) MPPI_MLP_LAUNCH(3, true, 1); else MPPI_MLP_LAUNCH(3, false, 1); }
-#undef MPPI_MLP_LAUNCH
+    kernels[variant]<<<grid, MLP_THREADS, MLP_DYN_SMEM, st>>>(a, mlp_use_cg2(m->n_in, pp, m->n_gemm) ? m->w2_map_half : m->w2_map,
+                                                              m->d_w01, m->d_w01u, m->d_w3, m->d_b3, m->d_bh, d_S, n_tiles, m->d_hand,
+                                                              m->d_hand_flag, fault, epoch, balanced, m->d_b1);
     return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
-
-int mlp_launches_per_tick(const MlpState *) { return 1; }
 
 int mlp_check_guards(MlpState *m) {
     if (!m || !m->d_hand) return 0;

@@ -23,7 +23,6 @@ cudaError_t mlp_set_weights(MlpState *m, int n_in, int n_hidden, const float *co
                             const double *in_scale, const double *out_mean, const double *out_scale, cudaStream_t st);
 // index update + K x T rollout through the MLP + costs -> d_S; returns 0 on success
 int mlp_rollout_costs(MlpState *m, const TickArgs &a, bool sum, const float *d_eps, float *d_S, cudaStream_t st);
-int mlp_launches_per_tick(const MlpState *m);
 // true (and cleared) if a cluster hand-off of the balanced schedule was missed since the last call
 bool mlp_take_fault(MlpState *m, cudaStream_t st);
 // number of hand-off buffers whose guard zone was overwritten (0 = clean)

@@ -13,7 +13,6 @@ def timeit(eng, x0, n=200):
     b.record(st); torch.cuda.synchronize()
     eng.set_stream(0)
     return a.elapsed_time(b)/n
-print("MIN_CTA", os.environ.get("MPPI_MIN_CTA_SAMPLES"))
 for K in (1024, 4096, 16384, 65536, 262144):
     rc = MPPIRacecarController(horizon_step_T=50, number_of_samples_K=K, visualize_optimal_traj=False, visualze_sampled_trajs=False, seed=3)
     lp = rc.generate_lemniscate_trajectory(100, 10.0).astype(np.float32); rc.ref_path = lp

@@ -51,6 +51,52 @@ def test_errors_are_status_codes_not_exceptions_across_the_abi():
     assert lib.mppi_create(C.byref(c), C.byref(h)) == -1 and not h.value
 
 
+def test_create_refuses_exactly_the_unbuilt_mode_combinations():
+    """mppi_create over model x collision x cost kind x waypoint mode x robot count: MPPI_E_UNSUPPORTED exactly where the
+    rules below (the library's supported set, written out) refuse; every other combination is created (or, without a
+    device, fails with MPPI_E_CUDA after the combination checks)."""
+    import itertools
+    from mppi_b200 import _lib
+    lib = _lib.load()
+    DD, BIC, MLP = 0, 1, 2
+    NONE, CIRCLE, FOOTPRINT = 0, 1, 2
+    PATH, GOAL, TARGET = 0, 1, 2
+    STRICT, FROZEN = 0, 1
+    OK, E_CUDA, E_UNSUPPORTED = 0, -2, -5
+
+    def refused(model, coll, kind, wp, R):
+        pathless = kind != PATH
+        return ((coll == FOOTPRINT and model != BIC)
+                or (model == MLP and (wp != FROZEN or R != 1 or coll != NONE))
+                or (pathless and model != DD)
+                or (kind == GOAL and coll == FOOTPRINT)
+                or (kind == TARGET and coll != NONE)
+                or (wp == STRICT and R != 1 and not pathless))
+
+    accepted = set()
+    for model, coll, kind, wp, R in itertools.product((DD, BIC, MLP), (NONE, CIRCLE, FOOTPRINT), (PATH, GOAL, TARGET),
+                                                      (STRICT, FROZEN), (1, 2)):
+        c = _lib.MppiConfig()
+        lib.mppi_default_config(C.byref(c))
+        c.model, c.collision, c.cost_kind, c.waypoint_mode, c.n_robots = model, coll, kind, wp, R
+        h = C.c_void_p()
+        rc = lib.mppi_create(C.byref(c), C.byref(h))
+        case = (model, coll, kind, wp, R)
+        if refused(*case):
+            assert rc == E_UNSUPPORTED and not h.value, (case, rc)
+            continue
+        assert rc in (OK, E_CUDA), (case, rc)
+        accepted.add(rc)
+        if rc == OK:
+            assert h.value
+            assert lib.mppi_destroy(h) == OK
+        else:
+            assert not h.value
+    if E_CUDA in accepted:
+        import torch
+        assert accepted == {E_CUDA} and not torch.cuda.is_available()
+
+
 def test_no_cpu_fallback():
     """Without a CUDA device the drop-in class refuses to construct.  Checked in a child process that sees no device, so
     the check also runs on a machine that has one."""
