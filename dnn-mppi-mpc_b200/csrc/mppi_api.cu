@@ -104,6 +104,11 @@ struct mppi_handle_s {
     int *d_sorted_idx = nullptr, *d_iota = nullptr;
     void *d_sort_temp = nullptr;
     size_t sort_temp_bytes = 0;
+    // learned-dynamics viewers: control table (rows, T, 2), the replay's costs (rows) and states (rows, T, 3), its hand-off fault word,
+    // allocated at the first viewer call for the rows it replays (n_top + 1 or K + 1) and grown when a call needs more
+    float *d_rep_ctl = nullptr, *d_rep_X = nullptr;
+    unsigned *d_rep_fault = nullptr;
+    int rep_rows = 0;
     // per-robot scenes (fleets): one SceneRec per robot, installed by mppi_set_robot_goals / mppi_set_robot_obstacles; the
     // components in use are args.scene_mask.  scene_stash: the rollout path of the scene instantiation (1 noise stash, 0
     // regenerate), chosen at the first install; -1 before.
@@ -442,6 +447,7 @@ int mppi_destroy(mppi_handle_t h) {
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
     gfree(h, h->d_paths); gfree(h, h->d_path_len); gfree(h, h->d_scene);
     gfree(h, h->d_Sc); gfree(h, h->d_Ssorted); gfree(h, h->d_sorted_idx); gfree(h, h->d_iota); gfree(h, h->d_sort_temp);
+    gfree(h, h->d_rep_ctl); gfree(h, h->d_rep_X); gfree(h, h->d_rep_fault);
     if (h->mlp) mlp_destroy(h->mlp);
     gfree(h, h->d_path); gfree(h, h->d_U); gfree(h, h->d_M); gfree(h, h->d_S); gfree(h, h->d_part);
     gfree(h, h->d_out); gfree(h, h->d_idx); gfree(h, h->d_NC); gfree(h, h->d_ticket); gfree(h, h->d_first);
@@ -881,12 +887,13 @@ static int step_common(mppi_handle_t h, const double *x0, const float *d_eps, ui
     if (h->timing) CK(h, cudaEventRecord(h->ev[0], h->stream));
     int strict_idx_after = -1;
     if (h->mlp) {
-        int rc = mlp_rollout_costs(h->mlp, h->args, h->sum, d_eps, h->d_S, h->stream);
+        float *S = h->keep_costs ? h->d_Sc : h->d_S;          // kept for mppi_get_top_trajectories
+        int rc = mlp_rollout_costs(h->mlp, h->args, h->sum, d_eps, S, h->stream);
         if (rc != 0) return fail(h, rc == -2 ? MPPI_E_STATE : MPPI_E_CUDA, rc == -2 ? "mppi_set_mlp has not been called" : "MLP rollout launch failed");
         h->tm.launches++;
         if (h->timing) CK(h, cudaEventRecord(h->ev[1], h->stream));
         TickArgs a = h->args;
-        a.S = h->d_S; a.eps = d_eps;
+        a.S = S; a.eps = d_eps;
         a.flags = F_UPDATE | F_FROM_S;      // K2 repeats step 1 (same result as in the MLP kernel) and persists the index
         int rc2 = launch_update(h, a, d_eps != nullptr);
         if (rc2 != MPPI_OK) return rc2;
@@ -1002,16 +1009,54 @@ int mppi_generate_noise_robot(mppi_handle_t h, uint64_t seed, uint64_t tick, int
     return MPPI_OK;
 }
 
+// Learned-dynamics viewers: the controls mppi_traj_kernel would apply (n_rows selected samples, or all K without a selection,
+// then the updated nominal) are written to a table and replayed through the tick's own MLP rollout, so a replayed state is the
+// state the tick scored.  Sampled rows -> d_samp (n_rows, T, 3) when given, the nominal's row -> optimal_out (host) when given.
+// Only scratch is written: the nominal, the waypoint index and the tick's fault word stay as the tick left them.
+static int mlp_replay(mppi_handle_t h, const TickArgs &a, const int *d_sel, int n_rows, int shift, float *optimal_out, float *d_samp) {
+    const int T = h->cfg.T, rows = n_rows + 1;
+    if (rows > h->rep_rows) {
+        gfree(h, h->d_rep_ctl); gfree(h, h->d_rep_X); gfree(h, h->d_rep_fault);
+        h->d_rep_ctl = h->d_rep_X = nullptr; h->d_rep_fault = nullptr; h->rep_rows = 0;
+        CK(h, gmalloc(h, &h->d_rep_ctl, sizeof(float) * (size_t)rows * T * 2));
+        CK(h, gmalloc(h, &h->d_rep_X, sizeof(float) * (size_t)rows * (1 + T * 3)));
+        CK(h, gmalloc(h, &h->d_rep_fault, sizeof(unsigned)));
+        CK(h, cudaMemset(h->d_rep_fault, 0, sizeof(unsigned)));
+        h->rep_rows = rows;
+    }
+    CK(h, mppi_launch_traj_controls(a, h->d_out, h->d_rep_ctl, d_sel, n_rows, shift, h->stream));
+    TickArgs r = a;
+    r.K = rows;
+    if (int rc = mlp_rollout_states(h->mlp, r, h->d_rep_ctl, h->d_rep_X, h->d_rep_fault, h->stream))
+        return fail(h, rc == -2 ? MPPI_E_STATE : MPPI_E_CUDA, rc == -2 ? "mppi_set_mlp has not been called" : "MLP replay launch failed");
+    h->tm.launches += 2;
+    const size_t row_floats = (size_t)T * 3;
+    const float *X = h->d_rep_X + rows;                      // behind the replay's costs
+    if (d_samp && n_rows > 0)
+        CK(h, cudaMemcpyAsync(d_samp, X, sizeof(float) * row_floats * n_rows, cudaMemcpyDeviceToDevice, h->stream));
+    if (optimal_out)
+        CK(h, cudaMemcpyAsync(optimal_out, X + row_floats * n_rows, sizeof(float) * row_floats, cudaMemcpyDeviceToHost, h->stream));
+    unsigned fault = 0;
+    CK(h, cudaMemcpyAsync(&fault, h->d_rep_fault, sizeof(fault), cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaStreamSynchronize(h->stream));
+    if (fault) {
+        CK(h, cudaMemset(h->d_rep_fault, 0, sizeof(unsigned)));
+        return fail(h, MPPI_E_NUMERIC, "learned-dynamics replay: a cluster hand-off was missed (producer cluster not co-resident)");
+    }
+    return MPPI_OK;
+}
+
 int mppi_get_trajectories(mppi_handle_t h, const double *x0, const float *d_eps, uint64_t seed, uint64_t tick,
                           float *optimal_out, float *d_sampled_out) {
     if (!h || !x0) return MPPI_E_BADARG;
-    if (h->cfg.n_robots != 1 || h->mlp) return fail(h, MPPI_E_UNSUPPORTED, "trajectories: single-robot analytic models only");
+    if (h->cfg.n_robots != 1) return fail(h, MPPI_E_UNSUPPORTED, "trajectories: single-robot handles only");
     if (int rc = scene_refused(h, "mppi_get_trajectories")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
     set_x0(h, x0);
     set_seed(h, seed, tick);
     TickArgs a = h->args;
     a.eps = d_eps;
+    if (h->mlp) return mlp_replay(h, a, nullptr, d_sampled_out ? h->cfg.K : 0, 1, optimal_out, d_sampled_out);
     const int nx = h->nx, T = h->cfg.T;
     if (optimal_out && !h->d_opt) CK(h, gmalloc(h, &h->d_opt, sizeof(float) * MPPI_MAX_T * 4));
     CK(h, mppi_launch_traj(a, h->cfg.model, h->d_out, optimal_out ? h->d_opt : nullptr, d_sampled_out, nullptr, 0, 1, h->stream));
@@ -1042,7 +1087,7 @@ int mppi_get_top_trajectories(mppi_handle_t h, const double *x0, const float *d_
                               int32_t n_top, int32_t index_shift, float *optimal_out, float *d_traj_out,
                               int32_t *d_idx_out, float *d_cost_out) {
     if (!h || !x0 || n_top < 1 || n_top > h->cfg.K || !d_traj_out || index_shift < 0 || index_shift > 1) return MPPI_E_BADARG;
-    if (h->cfg.n_robots != 1 || h->mlp) return fail(h, MPPI_E_UNSUPPORTED, "trajectories: single-robot analytic models only");
+    if (h->cfg.n_robots != 1) return fail(h, MPPI_E_UNSUPPORTED, "trajectories: single-robot handles only");
     if (!h->keep_costs || !h->d_Sc) return fail(h, MPPI_E_STATE, "call mppi_set_keep_costs(h, 1) before the tick");
     if (int rc = scene_refused(h, "mppi_get_top_trajectories")) return rc;
     CK(h, cudaSetDevice(h->cfg.device));
@@ -1052,6 +1097,12 @@ int mppi_get_top_trajectories(mppi_handle_t h, const double *x0, const float *d_
     a.eps = d_eps;
     const int nx = h->nx, T = h->cfg.T;
     CK(h, mppi_sort_costs(h->d_Sc, h->cfg.K, h->d_Ssorted, h->d_sorted_idx, h->d_iota, h->d_sort_temp, h->sort_temp_bytes, h->stream));
+    if (h->mlp) {
+        h->tm.launches += 2;
+        if (d_idx_out) CK(h, cudaMemcpyAsync(d_idx_out, h->d_sorted_idx, sizeof(int) * n_top, cudaMemcpyDeviceToDevice, h->stream));
+        if (d_cost_out) CK(h, cudaMemcpyAsync(d_cost_out, h->d_Ssorted, sizeof(float) * n_top, cudaMemcpyDeviceToDevice, h->stream));
+        return mlp_replay(h, a, h->d_sorted_idx, n_top, index_shift, optimal_out, d_traj_out);
+    }
     if (optimal_out && !h->d_opt) CK(h, gmalloc(h, &h->d_opt, sizeof(float) * MPPI_MAX_T * 4));
     CK(h, mppi_launch_traj(a, h->cfg.model, h->d_out, optimal_out ? h->d_opt : nullptr, d_traj_out, h->d_sorted_idx, n_top,
                            index_shift, h->stream));

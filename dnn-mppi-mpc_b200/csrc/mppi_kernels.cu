@@ -837,6 +837,40 @@ __global__ void mppi_traj_kernel(const __grid_constant__ TickArgs a, const float
     }
 }
 
+// The controls of those replays as a table, for the learned-dynamics viewers (mppi_mlp.cu replays it through the tick's own
+// rollout): row i < n_rows = sample sel[i] (sample i without a selection), row n_rows = the updated nominal; same rule as above.
+__global__ void mppi_traj_controls_kernel(const __grid_constant__ TickArgs a, const float *__restrict__ rec, float2 *__restrict__ ctl,
+                                          const int *__restrict__ sel, int n_rows, int shift) {
+    const int row = blockIdx.x * blockDim.x + threadIdx.x;
+    if (row > n_rows) return;
+    const bool nominal = row == n_rows;
+    const int k = nominal ? a.K : (sel ? sel[row] : row);
+    const int T = a.T;
+    const float *upre = rec + MPPI_OUT_UPRE, *uold = rec + MPPI_OUT_UOLD;
+    const uint32_t kg = (uint32_t)(a.k_offset + k);
+    const bool exploit = (int)kg < a.n_exploit;
+    for (int t = 0; t < T; ++t) {
+        const int tc = shift ? (t + T - 1) % T : t;
+        float v0, v1;
+        if (nominal) {
+            v0 = clampf(upre[2 * tc], a.umax0); v1 = clampf(upre[2 * tc + 1], a.umax1);
+        } else {
+            float e0, e1;
+            if (a.eps) {
+                const float2 ee = reinterpret_cast<const float2 *>(a.eps)[(size_t)k * T + tc];
+                e0 = ee.x; e1 = ee.y;
+            } else {
+                float e[4];
+                philox_eps_pair(a, kg, (uint32_t)(tc >> 1), 0u, e);
+                e0 = e[2 * (tc & 1)]; e1 = e[2 * (tc & 1) + 1];
+            }
+            v0 = clampf(exploit ? __fadd_rn(uold[2 * tc], e0) : e0, a.umax0);
+            v1 = clampf(exploit ? __fadd_rn(uold[2 * tc + 1], e1) : e1, a.umax1);
+        }
+        ctl[(size_t)row * T + t] = make_float2(v0, v1);
+    }
+}
+
 // (K,T,2) export of the Philox noise the tick kernel consumes
 __global__ void mppi_noise_kernel(const __grid_constant__ TickArgs a, float *out, int robot) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1058,6 +1092,12 @@ cudaError_t mppi_launch_traj(const TickArgs &a, int model, const float *rec, flo
     const int n = (d_sel ? n_sel : a.K) + 1;
     if (model == MPPI_MODEL_BICYCLE) mppi_traj_kernel<MPPI_MODEL_BICYCLE><<<(n + 127) / 128, 128, 0, st>>>(a, rec, d_opt, d_samp, d_sel, n_sel, shift);
     else mppi_traj_kernel<MPPI_MODEL_DIFFDRIVE><<<(n + 127) / 128, 128, 0, st>>>(a, rec, d_opt, d_samp, d_sel, n_sel, shift);
+    return cudaGetLastError();
+}
+
+cudaError_t mppi_launch_traj_controls(const TickArgs &a, const float *rec, float *d_ctl, const int *d_sel, int n_rows, int shift,
+                                      cudaStream_t st) {
+    mppi_traj_controls_kernel<<<(n_rows + 1 + 127) / 128, 128, 0, st>>>(a, rec, reinterpret_cast<float2 *>(d_ctl), d_sel, n_rows, shift);
     return cudaGetLastError();
 }
 

@@ -14,6 +14,9 @@ cudaError_t mppi_launch_merge(const TickArgs &a, const float *triples, int G, cu
 cudaError_t mppi_launch_p2p_barrier(const TickArgs &a, unsigned long long count, cudaStream_t st);
 cudaError_t mppi_launch_traj(const TickArgs &a, int model, const float *rec, float *d_opt, float *d_samp,
                              const int *d_sel, int n_sel, int shift, cudaStream_t st);
+// the controls mppi_traj_kernel applies, as a (n_rows + 1, T, 2) table: rows sel[i] (i without a selection), then the nominal
+cudaError_t mppi_launch_traj_controls(const TickArgs &a, const float *rec, float *d_ctl, const int *d_sel, int n_rows, int shift,
+                                      cudaStream_t st);
 // mppi_spline.cu: per-robot courses from waypoints (calc_spline_course on the device)
 #define MPPI_SPLINE_MAX_WAYPOINTS 32
 cudaError_t mppi_launch_spline(const float *d_wx, const float *d_wy, int n_robots, int n_wp, double ds, int max_pts,

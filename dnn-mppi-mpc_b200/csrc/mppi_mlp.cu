@@ -35,6 +35,11 @@
 // activations and of every accumulator quarter, so MMA start and epilogue tail are both short).
 // Variants that were built, measured and rejected (mma.sync layer 1, register-tiled 16x256b layer 1 / epilogue, early layer 1,
 // K-interleaved last quarters, output-layer records through the constant bank) are described in DESIGN.md 3.4 with the commits that hold them.
+//
+// THIS FILE IS COMPILED TWICE.  mppi_mlp_traj.cu includes it with MPPI_MLP_TRAJ_UNIT defined to instantiate the replay (TRAJ)
+// kernels apart from the tick's (see mlp_traj_kernels below).  In that unit only the TRAJ table is emitted: everything that
+// must exist once -- host functions, the tick's kernel table, any __device__ / __constant__ variable or other kernel -- belongs
+// in the `#else` branch of the `#ifdef MPPI_MLP_TRAJ_UNIT` at the end, or behind a guard of its own.
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -398,7 +403,14 @@ __device__ __forceinline__ void handoff_take(const float *hand, unsigned int *ha
     }
 }
 
-template <int NIN, bool PP, int NG>
+// TRAJ (replays for the trajectory viewers): behind the K costs, S_out also receives the state after every Euler step, (K, T, 3),
+// stored by the owner thread of each row from whichever cluster runs the step.
+__device__ __forceinline__ void store_state(float *S_out, int K, int T, int k, int t, const float (&z)[4]) {
+    float *xo = S_out + K + ((size_t)k * T + t) * 3;
+    xo[0] = z[0]; xo[1] = z[1]; xo[2] = z[2];
+}
+
+template <int NIN, bool PP, int NG, bool TRAJ = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MLP_THREADS, 1)
 mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constant__ CUtensorMap w2_map,
                         const float4 *__restrict__ g_w01, const float2 *__restrict__ g_w01u, const float4 *__restrict__ g_w3,
@@ -922,6 +934,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                 if (t > t0) {
                     epilogue(3, s0, s1, s2);                         // Y(t-1), last quarter
                     finish(1, s0, s1, s2);
+                    if constexpr (TRAJ) { if (grp == 1 && active) store_state(S_out, a.K, T, k, t - 1, z); }
                     if (grp == 1) prep(t);
                 }
                 if constexpr (L1TC) l1_publish(1);                   // inputs of L1(Y, t): the evaluation before it is long done
@@ -931,6 +944,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                 // ---- slot Y(t): the tensor core runs GEMM Y(t)
                 epilogue(3, r0, r1, r2);                             // X(t), last quarter
                 finish(0, r0, r1, r2);
+                if constexpr (TRAJ) { if (grp == 0 && active) store_state(S_out, a.K, T, k, t, z); }
                 if (grp == 0 && t + 1 < t1) prep(t + 1);
                 if constexpr (L1TC) { if (t + 1 < t1) l1_publish(0); }
                 s0 = s1 = s2 = 0.f;
@@ -939,6 +953,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
             }
             epilogue(3, s0, s1, s2);                                 // Y(t1-1), last quarter
             finish(1, s0, s1, s2);
+            if constexpr (TRAJ) { if (grp == 1 && active) store_state(S_out, a.K, T, k, t1 - 1, z); }
             if (warp == 2 && pr == n_nat - 1) MLP_PROBE_PRINT("compute warp 0: wait d_full q0-3 | a_free p0-3 | L1 work p0-3 | tmem ld, L1 bar, finish bar, epilogue math", my_tile_steps / 2);
             if (t1 < T) {
                 // head of a split quad: publish the state after step t1-1 for the next cluster's tail
@@ -1106,6 +1121,7 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
                     z[1] = fmaf(fmaf(vc0, sn, r1), a.dt, z[1]);
                     z[2] = fmaf(vc1 + r2, a.dt, z[2]);
                     vp0 = vc0; vp1 = vc1; vc0 = vn0; vc1 = vn1;
+                    if constexpr (TRAJ) { if (active) store_state(S_out, a.K, T, k, t, z); }
                 }
             }
             if (t1 < T) {
@@ -1134,11 +1150,32 @@ mppi_mlp_rollout_kernel(const __grid_constant__ TickArgs a, const __grid_constan
     }
 }
 
+#ifdef MPPI_MLP_TRAJ_UNIT
+typedef decltype(&mppi_mlp_rollout_kernel<3, false, 1, true>) MlpKernel;
+#else
+typedef decltype(&mppi_mlp_rollout_kernel<3, false, 1>) MlpKernel;
+#endif
+
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                     const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 }  // namespace
+
+// The instantiations, indexed by the (n_in, ping-pong, GEMMs per step) variant (n_in 3 / 5 alternate): the tick's here, the
+// replays' (TRAJ) in mppi_mlp_traj.cu, which compiles this file with MPPI_MLP_TRAJ_UNIT.  Instantiated in this translation unit,
+// the TRAJ kernels change how the device compiler numbers the shared code of <5, true, 1> and with it that kernel's machine
+// code; apart, the tick's six compile exactly as they did without them.
+extern const MlpKernel mlp_traj_kernels[6];
+#ifdef MPPI_MLP_TRAJ_UNIT
+const MlpKernel mlp_traj_kernels[6] = {
+    mppi_mlp_rollout_kernel<3, false, 1, true>, mppi_mlp_rollout_kernel<5, false, 1, true>, mppi_mlp_rollout_kernel<3, true, 1, true>,
+    mppi_mlp_rollout_kernel<5, true, 1, true>,  mppi_mlp_rollout_kernel<3, false, 2, true>, mppi_mlp_rollout_kernel<5, false, 2, true>};
+#else
+static const MlpKernel mlp_kernels[6] = {
+    mppi_mlp_rollout_kernel<3, false, 1>, mppi_mlp_rollout_kernel<5, false, 1>, mppi_mlp_rollout_kernel<3, true, 1>,
+    mppi_mlp_rollout_kernel<5, true, 1>,  mppi_mlp_rollout_kernel<3, false, 2>, mppi_mlp_rollout_kernel<5, false, 2>};
+static MlpKernel mlp_kernel(int variant, bool traj) { return traj ? mlp_traj_kernels[variant] : mlp_kernels[variant]; }
 
 struct MlpState {
     int K = 0, T = 0, n_sm = 148;
@@ -1150,7 +1187,7 @@ struct MlpState {
     float *d_bh = nullptr;                // n_hidden = 3: bias of the layer the first GEMM evaluates
     float *d_hand = nullptr;              // balanced schedule: state records of split quads [cluster][rank][slot][6][128]
     unsigned int *d_hand_flag = nullptr;  // [cluster][rank]: epoch of the launch that published the record; then one fault word
-    int max_clusters[6] = {0, 0, 0, 0, 0, 0};   // co-resident 2-CTA clusters per instantiation (cudaOccupancyMaxActiveClusters)
+    int max_clusters[12] = {};            // co-resident 2-CTA clusters per instantiation (cudaOccupancyMaxActiveClusters), TRAJ at 6..11
     unsigned int epoch = 0;
     int n_in = 3, n_gemm = 1;
     CUtensorMap w2_map;
@@ -1176,14 +1213,10 @@ MlpState *mlp_create(int K, int T) {
         cudaMalloc(&m->d_w01u, sizeof(float2) * HID) != cudaSuccess ||
         cudaMalloc(&m->d_b3, sizeof(float) * 4) != cudaSuccess ||
         cudaMalloc(&m->d_b1, (size_t)B1TC_BYTES) != cudaSuccess) { mlp_destroy(m); return nullptr; }
-    if (cudaFuncSetAttribute(mppi_mlp_rollout_kernel<3, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess ||
-        cudaFuncSetAttribute(mppi_mlp_rollout_kernel<5, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess ||
-        cudaFuncSetAttribute(mppi_mlp_rollout_kernel<3, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess ||
-        cudaFuncSetAttribute(mppi_mlp_rollout_kernel<5, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess ||
-        cudaFuncSetAttribute(mppi_mlp_rollout_kernel<3, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess ||
-        cudaFuncSetAttribute(mppi_mlp_rollout_kernel<5, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess) {
-        mlp_destroy(m); return nullptr;
-    }
+    for (int v = 0; v < 12; ++v)
+        if (cudaFuncSetAttribute(mlp_kernel(v % 6, v >= 6), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_DYN_SMEM) != cudaSuccess) {
+            mlp_destroy(m); return nullptr;
+        }
     return m;
 }
 
@@ -1313,27 +1346,20 @@ static int mlp_max_active_clusters(Kern kern, int n_sm) {
     return n;
 }
 
-int mlp_rollout_costs(MlpState *m, const TickArgs &args, bool sum, const float *d_eps, float *d_S, cudaStream_t st) {
-    if (!m || !m->ready) return -2;
-    TickArgs a = args;
-    a.eps = d_eps;
-    a.flags = sum ? F_COST_SUM : 0;
+// One rollout launch over a.K rows: costs into `out` (K), with `traj` followed by the states after every step (K, T, 3).
+static int mlp_launch(MlpState *m, const TickArgs &a, bool traj, float *out, unsigned int *fault, cudaStream_t st) {
     const int n_tiles = (a.K + TILE_M - 1) / TILE_M;
     int grid = std::min(((n_tiles + 1) / 2) * 2, m->n_sm & ~1);       // whole clusters of 2
     // two tiles per CTA in flight (ping-pong) whenever a CTA owns more than one tile
     const bool pp = n_tiles > grid && m->n_gemm == 1;
-    // the instantiation: (n_in, ping-pong, GEMMs per step) = variant (n_in 3 / 5 alternate)
-    static const decltype(&mppi_mlp_rollout_kernel<3, false, 1>) kernels[6] = {
-        mppi_mlp_rollout_kernel<3, false, 1>, mppi_mlp_rollout_kernel<5, false, 1>, mppi_mlp_rollout_kernel<3, true, 1>,
-        mppi_mlp_rollout_kernel<5, true, 1>,  mppi_mlp_rollout_kernel<3, false, 2>, mppi_mlp_rollout_kernel<5, false, 2>};
-    const int variant = (m->n_gemm == 2 ? 4 : (pp ? 2 : 0)) + (m->n_in == 5 ? 1 : 0);
+    const int variant = (m->n_gemm == 2 ? 4 : (pp ? 2 : 0)) + (m->n_in == 5 ? 1 : 0), slot = (traj ? 6 : 0) + variant;
     // never launch more clusters than the device keeps resident at once (fused-off SMs, MPS partitions): the grid is
     // persistent, so a smaller one only means more tiles per cluster
-    if (m->max_clusters[variant] == 0) {
-        const int n = mlp_max_active_clusters(kernels[variant], m->n_sm);
-        m->max_clusters[variant] = n > 0 ? n : -1;                    // -1: the query failed, keep the SM-count grid
+    if (m->max_clusters[slot] == 0) {
+        const int n = mlp_max_active_clusters(mlp_kernel(variant, traj), m->n_sm);
+        m->max_clusters[slot] = n > 0 ? n : -1;                       // -1: the query failed, keep the SM-count grid
     }
-    if (m->max_clusters[variant] > 0) grid = std::min(grid, 2 * m->max_clusters[variant]);
+    if (m->max_clusters[slot] > 0) grid = std::min(grid, 2 * m->max_clusters[slot]);
     // balanced (horizon-split) walk when whole quads do not divide over the clusters and every cluster still gets more
     // than one horizon of steps; MPPI_MLP_BALANCED=0 forces whole quads (A/B measurements)
     const char *bal_env = std::getenv("MPPI_MLP_BALANCED");               // read per launch: tests flip it in-process
@@ -1343,11 +1369,27 @@ int mlp_rollout_costs(MlpState *m, const TickArgs &args, bool sum, const float *
     const int balanced = ((pp || one_tile_bal) && allow_bal && n_clusters > 0 && (n_quads % n_clusters) != 0 &&
                           (long long)n_quads * a.T / n_clusters >= a.T + 2) ? 1 : 0;
     const unsigned int epoch = ++m->epoch;
-    unsigned int *fault = m->d_hand_flag + (size_t)(m->n_sm / 2 + 1) * 2;
-    kernels[variant]<<<grid, MLP_THREADS, MLP_DYN_SMEM, st>>>(a, mlp_use_cg2(m->n_in, pp, m->n_gemm) ? m->w2_map_half : m->w2_map,
-                                                              m->d_w01, m->d_w01u, m->d_w3, m->d_b3, m->d_bh, d_S, n_tiles, m->d_hand,
-                                                              m->d_hand_flag, fault, epoch, balanced, m->d_b1);
+    mlp_kernel(variant, traj)<<<grid, MLP_THREADS, MLP_DYN_SMEM, st>>>(a, mlp_use_cg2(m->n_in, pp, m->n_gemm) ? m->w2_map_half : m->w2_map,
+                                                                       m->d_w01, m->d_w01u, m->d_w3, m->d_b3, m->d_bh, out, n_tiles, m->d_hand,
+                                                                       m->d_hand_flag, fault, epoch, balanced, m->d_b1);
     return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
+int mlp_rollout_costs(MlpState *m, const TickArgs &args, bool sum, const float *d_eps, float *d_S, cudaStream_t st) {
+    if (!m || !m->ready) return -2;
+    TickArgs a = args;
+    a.eps = d_eps;
+    a.flags = sum ? F_COST_SUM : 0;
+    return mlp_launch(m, a, false, d_S, m->d_hand_flag + (size_t)(m->n_sm / 2 + 1) * 2, st);
+}
+
+int mlp_rollout_states(MlpState *m, const TickArgs &args, const float *d_ctl, float *d_out, unsigned int *d_fault, cudaStream_t st) {
+    if (!m || !m->ready) return -2;
+    TickArgs a = args;
+    a.eps = d_ctl;
+    a.n_exploit = 0; a.k_offset = 0;
+    a.flags = 0;
+    return mlp_launch(m, a, true, d_out, d_fault, st);
 }
 
 int mlp_check_guards(MlpState *m) {
@@ -1365,3 +1407,4 @@ bool mlp_take_fault(MlpState *m, cudaStream_t st) {
     if (v) cudaMemsetAsync(fault, 0, sizeof(v), st);
     return v != 0;
 }
+#endif  // MPPI_MLP_TRAJ_UNIT

@@ -23,6 +23,11 @@ cudaError_t mlp_set_weights(MlpState *m, int n_in, int n_hidden, const float *co
                             const double *in_scale, const double *out_mean, const double *out_scale, cudaStream_t st);
 // index update + K x T rollout through the MLP + costs -> d_S; returns 0 on success
 int mlp_rollout_costs(MlpState *m, const TickArgs &a, bool sum, const float *d_eps, float *d_S, cudaStream_t st);
+// Replay (trajectory viewers): a.K rows, row k applies the controls d_ctl (K, T, 2) -- already clamped, so the rollout's own
+// clamp leaves them exact -- through the same learned step as the tick.  d_out receives K costs (scratch: they are scored against
+// whatever nominal `a` holds) followed by the state after every step, (K, T, 3).  A missed cluster hand-off raises *d_fault
+// instead of the handle's fault word.  Returns 0 on success
+int mlp_rollout_states(MlpState *m, const TickArgs &a, const float *d_ctl, float *d_out, unsigned int *d_fault, cudaStream_t st);
 // true (and cleared) if a cluster hand-off of the balanced schedule was missed since the last call
 bool mlp_take_fault(MlpState *m, cudaStream_t st);
 // number of hand-off buffers whose guard zone was overwritten (0 = clean)

@@ -97,7 +97,7 @@ class ControllerBase:
         u = self._u_cache
         optimal_traj = np.zeros((self.T, self.dim_x), dtype=self._out_dtype)
         want_opt, want_samp = self._viz_gates()
-        if (want_opt or want_samp) and self._top_n and self._engine.model != "diffdrive_mlp":
+        if (want_opt or want_samp) and self._top_n:
             import torch
             dev = "cuda:%d" % self._engine.device
             d_samp = torch.empty(self._top_n, self.T, self.dim_x, dtype=torch.float32, device=dev)
@@ -110,7 +110,7 @@ class ControllerBase:
             sampled = d_samp.cpu().numpy().astype(self._out_dtype)
             self.last_top_idx = d_idx.cpu().numpy() + self._rank * self._K_local
             self.last_top_cost = d_cost.cpu().numpy()
-        elif (want_opt or want_samp) and self._world == 1 and self._engine.model != "diffdrive_mlp":
+        elif (want_opt or want_samp) and self._world == 1:
             import torch
             d_samp = torch.empty(self.K, self.T, self.dim_x, dtype=torch.float32,
                                  device="cuda:%d" % self._engine.device) if want_samp else None
@@ -123,7 +123,7 @@ class ControllerBase:
             # (K,T,nx) zeros like the reference returns when the flag is off, without allocating K*T*nx
             sampled = np.broadcast_to(np.zeros((), dtype=self._out_dtype), (self.K, self.T, self.dim_x))
             if (want_opt or want_samp) and not self._viz_warned:
-                warnings.warn("visualisation trajectories are not produced for sharded / learned-dynamics controllers")
+                warnings.warn("visualisation trajectories are not produced for sharded controllers")
                 self._viz_warned = True
         return u[0], u, optimal_traj, sampled
 

@@ -226,6 +226,10 @@ int mppi_get_stats(mppi_handle_t h, mppi_stats_t *out);   /* robot 0 */
 /* Visualisation outputs of the LAST tick (A16: mppi_differential_drive.py:144-159, mppi_race_car_obstacle.py:111-125):
  * the replay of the updated (pre-shift) nominal and of every sample's clamped controls, both with the reference's
  * `t-1` indexing.  Call right after mppi_step with the same x0 / d_eps / seed / tick.
+ * Learned dynamics (MPPI_MODEL_DIFFDRIVE_MLP): the same controls are replayed through the tick's own tensor-core MLP
+ * rollout, so a replayed state is the state the tick scored (fp16 hidden layers, hardware tanh; DESIGN.md 3.4).  The
+ * nominal, the waypoint index and the tick's fault word are not touched; a missed cluster hand-off of the replay
+ * returns MPPI_E_NUMERIC.  Fleets (n_robots > 1) return MPPI_E_UNSUPPORTED.
  *   optimal_out  host, T*nx floats, or NULL;   d_sampled_out  device, K*T*nx floats, or NULL */
 int mppi_get_trajectories(mppi_handle_t h, const double *x0, const float *d_eps, uint64_t seed, uint64_t tick,
                           float *optimal_out, float *d_sampled_out);
@@ -235,7 +239,8 @@ int mppi_get_trajectories(mppi_handle_t h, const double *x0, const float *d_eps,
  * [:num_top_samples]` with num_top_samples = max(10, K/10), test/test_mppi_diff_obs.py:102-104) replayed from x0,
  * instead of all K trajectories (600 MB at K = 1M, H = 50).  mppi_set_keep_costs(h, 1) makes every following tick
  * keep its per-sample costs (4 bytes per sample); call mppi_get_top_trajectories right after mppi_step with the same
- * x0 / d_eps / seed / tick.
+ * x0 / d_eps / seed / tick.  Learned dynamics: as mppi_get_trajectories (the n_top rows and the nominal are replayed
+ * through the tick's MLP rollout); the tick keeps its costs in the same buffer the sort reads.
  *   index_shift   1: controls indexed t-1, last row first, like the reference classes (A16);
  *                 0: controls indexed t (test/test_mppi_diff_obs.py:94,108)
  *   optimal_out   host T*nx floats, replay of the updated pre-shift nominal, or NULL
